@@ -16,7 +16,7 @@ compared bit for bit with tables recomputed on every rank: `setup`).  After the 
 its own output against the CPU oracle (`ranks_verified`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--method bilinear|nearestneighbor|bicubic]
-                    [--variant plain|fill|short] [--scaling strong|weak] [--no-extra]
+                    [--variant plain|fill|short] [--scaling strong|weak] [--no-extra] [--dump-outputs DIR]
 
 --variant (default plain = CachedInterpolation::interpolateValues, the BASELINE workload) selects the whole slice body of
 CDMInterpolator::getDataSlice instead, with its two adapter passes fused into the gather kernel: `fill` = float32 field
@@ -405,6 +405,8 @@ def main_b200(args):
         ev[k + 1].record()
     barrier()
     launches = fb.kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:  # before the e2e and extra legs reuse d_out
+        dump_outputs(args.dump_outputs, d_out.view(nlev, -1), torch)
     own_ms = ev[0].elapsed_time(ev[-1])
     per_launch_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
     clocks = sampler.stop() if rank == 0 else None
@@ -567,6 +569,24 @@ def main_b200(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_LEVELS, DUMP_POINTS, DUMP_SEED = 3, 2_000_000, 20261021
+
+
+def dump_outputs(path, out, torch):
+    """What the last timed step returned, as float32 .npy (int16 outputs convert exactly): `levels.npy` = DUMP_LEVELS whole
+    output levels [k][OUT_N][OUT_N] and `sample.npy` = DUMP_POINTS values at seeded positions of the whole [levels][points]
+    stack, 56 MB in all.  The positions depend only on the stack's shape, so two builds can be compared value for value."""
+    nlev, npts = out.shape
+    rng = np.random.default_rng(DUMP_SEED)
+    lv = np.sort(rng.choice(nlev, min(DUMP_LEVELS, nlev), replace=False))
+    flat = rng.integers(0, nlev * npts, DUMP_POINTS)
+    os.makedirs(path, exist_ok=True)
+    levels = out[torch.from_numpy(lv).to(out.device)].to(torch.float32).cpu().numpy().reshape(-1, OUT_N, OUT_N)
+    sample = out.reshape(-1)[torch.from_numpy(flat).to(out.device)].to(torch.float32).cpu().numpy()
+    np.save(os.path.join(path, "levels.npy"), levels)
+    np.save(os.path.join(path, "sample.npy"), sample)
 
 
 def bicubic_note():
@@ -736,7 +756,13 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the extra block (the other BASELINE configs, N = 1 only)")
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="strong (default): ONE stack of 24 x 137 levels split across the GPUs (SURVEY.md 8e); weak: a whole stack per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded float32 sample of rank 0's output of the last timed step "
+                                                          "to DIR/levels.npy and DIR/sample.npy (56 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the GPU path (--impl b200)")
     if args.impl == "reference":
         return main_reference(args)
     return main_b200(args)

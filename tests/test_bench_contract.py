@@ -1,5 +1,5 @@
 """bench.py's output contract, as far as it can be checked without a GPU: the reference arm's JSON line (driver keys, the
-`config` object both arms share), the slab split, and the bookkeeping of profiles/traffic.json."""
+`config` object both arms share), the slab split, the --dump-outputs sample, and the bookkeeping of profiles/traffic.json."""
 import json
 import os
 import subprocess
@@ -49,6 +49,25 @@ def test_strong_scaling_slabs_cover_the_stack_once():
         assert parts[0][0] == 0 and parts[-1][1] == total
         assert all(parts[i][1] == parts[i + 1][0] for i in range(world - 1))
     assert slab_range(total, 0, 8) == (0, 411)
+
+
+def test_dump_outputs_is_a_fixed_float32_sample_of_the_output(tmp_path):
+    import numpy as np
+    import torch
+    nlev, npts = 4, bench.OUT_N * bench.OUT_N
+    out = torch.arange(nlev * npts, dtype=torch.float32).view(nlev, npts)  # every value names its own position (< 2**24)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), out, torch)
+    assert sorted(os.listdir(tmp_path / "a")) == ["levels.npy", "sample.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in ("levels.npy", "sample.npy")) <= 64 << 20
+    levels, sample = np.load(tmp_path / "a" / "levels.npy"), np.load(tmp_path / "a" / "sample.npy")
+    assert np.array_equal(levels, np.load(tmp_path / "b" / "levels.npy")) and np.array_equal(sample, np.load(tmp_path / "b" / "sample.npy"))
+    assert levels.dtype == sample.dtype == np.float32
+    assert levels.shape == (bench.DUMP_LEVELS, bench.OUT_N, bench.OUT_N) and sample.shape == (bench.DUMP_POINTS,)
+    first = levels[:, 0, 0]
+    assert np.all(first % npts == 0) and np.all(np.diff(first) > 0)  # whole levels, in order
+    assert all(np.array_equal(levels[i].ravel(), first[i] + np.arange(npts, dtype=np.float32)) for i in range(bench.DUMP_LEVELS))
+    assert sample.min() >= 0 and sample.max() < nlev * npts and np.unique(sample).size > 0.9 * sample.size
 
 
 def test_traffic_json_names_the_sources_it_was_measured_on():

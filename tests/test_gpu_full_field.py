@@ -6,6 +6,9 @@ with the CPU pipeline (project_axes -> points2position -> createReducedDomain) o
 index flips bounded by the number of positions within 4e-9 cells (1e-9 degree on the 0.25-degree axes) of a cell or half-cell
 boundary.
 
+Where oracle/_ref is not built (it needs the reference's sources, which the repository does not hold), the same comparison
+runs against the restatement (oracle/liboracle.so), which tests/test_oracle_golden.py pins to vectors the reference computed.
+
 Levels are compared in chunks so the host never holds more than one chunk of the reference's output.
 """
 import os
@@ -31,6 +34,13 @@ AX2 = (np.arange(2000) - 999.5) * 0.0225
 NZ = 137
 
 
+@pytest.fixture(scope="module")
+def cpu_kernels(oracle):
+    """the reference's own kernels where oracle/_ref is built, else the restatement: the same Python surface"""
+    from oracle import oracle as orc
+    return orc.Reference() if orc.Reference.available() else oracle
+
+
 def _cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -45,7 +55,7 @@ def _bilinear_ub_count(oracle, px, py, inX, inY):
     return sum(1 for i in cand if oracle.bilinear_is_ub(px[i], py[i], inX, inY))
 
 
-def _compare_levels(reference, method, gx, gy, inX, inY, outX, outY, d_in, d_out, nan_payload, chunk=16, post=None):
+def _compare_levels(cpu_kernels, method, gx, gy, inX, inY, outX, outY, d_in, d_out, nan_payload, chunk=16, post=None):
     """d_in: list of device tensors [nz][inY][inX] (one per field), d_out: matching list [nz][outY][outX].  Returns the number
     of differing values over the whole stack.  post(list of host arrays) -> list of host arrays (e.g. the rotation)."""
     import torch
@@ -53,7 +63,7 @@ def _compare_levels(reference, method, gx, gy, inX, inY, outX, outY, d_in, d_out
     differing, compared = 0, 0
     for z0 in range(0, nz, chunk):
         z1 = min(nz, z0 + chunk)
-        want = [reference.cached_interpolate(int(method), gx, gy, inX, inY, outX, outY, f[z0:z1].cpu().numpy(), nthreads=_cores()) for f in d_in]
+        want = [cpu_kernels.cached_interpolate(int(method), gx, gy, inX, inY, outX, outY, f[z0:z1].cpu().numpy(), nthreads=_cores()) for f in d_in]
         if post is not None:
             want = post(want, z1 - z0)
         for w, out in zip(want, d_out):
@@ -88,7 +98,7 @@ def _field(inX, inY, seed, nan_frac=0.01):
 
 
 @pytest.mark.parametrize("method", [Method.BILINEAR, Method.NEAREST_NEIGHBOR], ids=["config2-bilinear", "config3i-nearestneighbor"])
-def test_full_field_rotated_pole(oracle, reference, method):
+def test_full_field_rotated_pole(oracle, cpu_kernels, method):
     """configs 2 and 3(i): every one of the 137 x 2000 x 2000 output values equals the reference's, bit for bit (NaN payload
     included for nearest neighbour); the index tables equal the CPU pipeline's except at positions within 1e-9 degree of a
     (half-)cell boundary"""
@@ -114,14 +124,14 @@ def test_full_field_rotated_pole(oracle, reference, method):
     # ---- values, whole field ----
     field = _field(inX, inY, 20261018)
     out = ci.interpolateValues(field)
-    differing, compared = _compare_levels(reference, method, gx, gy, inX, inY, 2000, 2000, [field], [out],
+    differing, compared = _compare_levels(cpu_kernels, method, gx, gy, inX, inY, 2000, 2000, [field], [out],
                                           nan_payload=(method == Method.NEAREST_NEIGHBOR))
     assert compared == NZ * 4_000_000
     assert differing == 0, f"{differing} of {compared} values differ from the reference"
     print(f"full field {method.name}: {compared} values identical, {flips} index flips / {near} near a boundary, {time.perf_counter() - t0:.1f} s")
 
 
-def test_full_field_coord_nearestneighbor(oracle, reference):
+def test_full_field_coord_nearestneighbor(oracle, cpu_kernels):
     """config 3(ii): coord_nearestneighbor over the uncropped 1440 x 721 source: whole field memcmp-equal to the reference's
     mifi_get_values_f on the GPU's index table; the table itself against the CPU search on 20000 sampled targets"""
     lon2d, lat2d = oracle.lonlat_to_matrix(np.radians(LON), np.radians(LAT))
@@ -135,11 +145,11 @@ def test_full_field_coord_nearestneighbor(oracle, reference):
     assert differ <= max(3, ties), (differ, ties)
     field = _field(1440, 721, 33)
     out = ci.interpolateValues(field)
-    differing, compared = _compare_levels(reference, Method.COORD_NN, gx, gy, 1440, 721, 2000, 2000, [field], [out], nan_payload=True)
+    differing, compared = _compare_levels(cpu_kernels, Method.COORD_NN, gx, gy, 1440, 721, 2000, 2000, [field], [out], nan_payload=True)
     assert compared == NZ * 4_000_000 and differing == 0, f"{differing} of {compared} values differ from the reference"
 
 
-def test_full_field_bicubic_vector_polar_stereographic(oracle, reference):
+def test_full_field_bicubic_vector_polar_stereographic(oracle, cpu_kernels):
     """config 4: bicubic x_wind / y_wind, 137 levels, to the 3000 x 3000 polar-stereographic grid, rotated by
     CachedVectorReprojection: both whole output fields (2 x 1.23e9 values) equal the reference's mifi_get_values_bicubic_f +
     mifi_vector_reproject_values_by_matrix_f, bit for bit, NaN wedges included"""
@@ -161,15 +171,15 @@ def test_full_field_bicubic_vector_polar_stereographic(oracle, reference):
     uo, vo = ci.interpolateVector(u, v, cvr)
 
     def rotate(want, nz):
-        wu, wv = reference.vector_reproject_by_matrix(matrix, want[0], want[1], 3000, 3000, nz)
+        wu, wv = cpu_kernels.vector_reproject_by_matrix(matrix, want[0], want[1], 3000, 3000, nz)
         return [wu, wv]
 
-    differing, compared = _compare_levels(reference, Method.BICUBIC, gx, gy, inX, inY, 3000, 3000, [u, v], [uo, vo], nan_payload=False,
+    differing, compared = _compare_levels(cpu_kernels, Method.BICUBIC, gx, gy, inX, inY, 3000, 3000, [u, v], [uo, vo], nan_payload=False,
                                           chunk=8, post=rotate)
     assert compared == 2 * NZ * 9_000_000 and differing == 0, f"{differing} of {compared} values differ from the reference"
 
 
-def test_full_field_bicubic_fp32_mode_error(reference, monkeypatch):
+def test_full_field_bicubic_fp32_mode_error(cpu_kernels, monkeypatch):
     """config 4 in the opt-in fp32 arithmetic (FIMEX_B200_BICUBIC_FP32=1): the whole 137 x 3000 x 3000 field of each component
     against the reference: identical NaN masks, and max |error| <= 1e-5 x D, D = the largest |tap| of the point's own 4 x 4
     stencil (for the rotated pair: of both components) -- the denominator of north_star's "<= 1e-5 relative"."""
@@ -198,9 +208,9 @@ def test_full_field_bicubic_fp32_mode_error(reference, monkeypatch):
         z1 = min(NZ, z0 + chunk)
         nz = z1 - z0
         hu, hv = u[z0:z1].cpu().numpy(), v[z0:z1].cpu().numpy()
-        wu = reference.cached_interpolate(2, gx, gy, inX, inY, 3000, 3000, hu, nthreads=_cores())
-        wv = reference.cached_interpolate(2, gx, gy, inX, inY, 3000, 3000, hv, nthreads=_cores())
-        wu, wv = reference.vector_reproject_by_matrix(matrix, wu, wv, 3000, 3000, nz)
+        wu = cpu_kernels.cached_interpolate(2, gx, gy, inX, inY, 3000, 3000, hu, nthreads=_cores())
+        wv = cpu_kernels.cached_interpolate(2, gx, gy, inX, inY, 3000, 3000, hv, nthreads=_cores())
+        wu, wv = cpu_kernels.vector_reproject_by_matrix(matrix, wu, wv, 3000, 3000, nz)
         amax = torch.maximum(u[z0:z1].abs(), v[z0:z1].abs())
         win = F.max_pool2d(amax[None], kernel_size=4, stride=1)[0].reshape(nz, -1)  # [nz][(inY-3)*(inX-3)]
         D = win[:, flat]  # [nz][9e6]
