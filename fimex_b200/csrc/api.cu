@@ -11,6 +11,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <limits>
 #include <map>
 #include <unordered_map>
@@ -665,18 +666,26 @@ void parallel_memcpy(void* dst, const void* src, size_t bytes)
         w.join();
 }
 
-// Host-buffer execution: levels are cut into chunks that rotate through three (stream, scratch) slots, so that
-// the H2D copy of chunk k+1, the kernel of chunk k and the D2H copy of chunk k-1 overlap.  `nfields` is 1
-// (scalar) or 2 (u/v).  Every call owns its streams and scratch => re-entrant on a shared handle.
-int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, const void* const* in, void* const* out, size_t nz,
-                   const SliceIO& io)
+// Host arrays of a call that the device works through in chunks of `units` (levels, time steps): up to two inputs and two
+// outputs, each `bytes per unit` long per unit (0: that array is absent and its device pointer is null).
+struct HostArrays {
+    int device = 0;
+    const void* in[2] = {nullptr, nullptr};
+    size_t in_unit[2] = {0, 0};
+    void* out[2] = {nullptr, nullptr};
+    size_t out_unit[2] = {0, 0};
+};
+// the device work of one chunk: `n` units of every array, already on the device
+using ChunkRun = std::function<int(const void* const* d_in, size_t n, void* const* d_out, cudaStream_t st)>;
+
+// Host-buffer execution: units are cut into chunks that rotate through three (stream, scratch) slots, so that
+// the H2D copy of chunk k+1, the kernel of chunk k and the D2H copy of chunk k-1 overlap.  Every call owns its
+// streams and scratch => re-entrant on a shared handle.
+int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
 {
-    const size_t in_level = h->inX * h->inY, out_level = h->outX * h->outY;
-    if (nz == 0 || out_level == 0)
-        return FB_OK;
-    const size_t in_elem = io.typed ? type_size(io.in_type) : sizeof(float), out_elem = io.typed ? type_size(io.out_type) : sizeof(float);
-    FB_REQUIRE(in_elem > 0 && out_elem > 0, "unsupported data type");
-    const size_t bytes_per_level = (in_level * in_elem + out_level * out_elem) * (size_t)nfields;
+    size_t bytes_per_level = 0;
+    for (int f = 0; f < 2; ++f)
+        bytes_per_level += io.in_unit[f] + io.out_unit[f];
     size_t chunk_bytes = 192ull << 20;
     if (const char* env = std::getenv("FIMEX_B200_HOST_CHUNK_MB")) // experiments: bytes of (input + output) per pipeline chunk
         if (std::atoll(env) > 0)
@@ -694,9 +703,9 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
     bool bounce_in = false, bounce_out = false; // pageable host arrays: staged through page-locked bounce buffers, see above
     // (with fewer than 4 host threads the driver's own staging, one thread at ~15 GB/s, is as fast; small calls are latency-bound)
     if (copy_threads() >= 4 && nz * bytes_per_level >= (size_t)(8u << 20)) {
-        for (int f = 0; f < nfields; ++f) {
-            bounce_in = bounce_in || (in_level && host_pageable(in[f]));
-            bounce_out = bounce_out || host_pageable(out[f]);
+        for (int f = 0; f < 2; ++f) {
+            bounce_in = bounce_in || (io.in_unit[f] && host_pageable(io.in[f]));
+            bounce_out = bounce_out || (io.out_unit[f] && host_pageable(io.out[f]));
         }
     }
     if ((bounce_in || bounce_out) && zc * bytes_per_level > (64ull << 20)) { // smaller chunks: the host copy of chunk k runs while k+1, k+2 are in flight
@@ -712,7 +721,7 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
         void* h_out[2] = {nullptr, nullptr};
         cudaEvent_t uploaded = nullptr, computed = nullptr, downloaded = nullptr;
     } slots[3];
-    HostPipe* pipe = host_pipe(h->device);
+    HostPipe* pipe = host_pipe(io.device);
     FB_REQUIRE(pipe != nullptr, std::string("cannot create the copy / compute streams: ") + cudaGetErrorString(cudaGetLastError()));
     const cudaStream_t s_up = pipe->up, s_run = pipe->run, s_down = pipe->down;
     for (int s = 0; s < nslots; ++s) {
@@ -726,9 +735,11 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
     double t0 = now(), t1 = 0, t2 = 0, t3 = 0;
     auto body = [&]() -> int {
         for (int s = 0; s < nslots; ++s) {
-            for (int f = 0; f < nfields; ++f) {
-                FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_in[f], in_elem * ((zc * in_level) > 0 ? zc * in_level : 1), s_run));
-                FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_out[f], out_elem * zc * out_level, s_run));
+            for (int f = 0; f < 2; ++f) {
+                if (io.in_unit[f])
+                    FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_in[f], zc * io.in_unit[f], s_run));
+                if (io.out_unit[f])
+                    FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_out[f], zc * io.out_unit[f], s_run));
             }
         }
         // the buffers were allocated in s_run's order: the copy streams must not touch them earlier
@@ -738,13 +749,13 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
         FB_CUDA_CHECK(cudaStreamWaitEvent(s_down, ready, 0));
         if (bounce_in || bounce_out) {
             for (int s = 0; s < nslots; ++s) {
-                for (int f = 0; f < nfields; ++f) {
-                    if (bounce_in) {
-                        slots[s].h_in[f] = fb200_host_alloc(in_elem * zc * in_level);
+                for (int f = 0; f < 2; ++f) {
+                    if (bounce_in && io.in_unit[f]) {
+                        slots[s].h_in[f] = fb200_host_alloc(zc * io.in_unit[f]);
                         FB_REQUIRE(slots[s].h_in[f] != nullptr, "cannot allocate a page-locked staging buffer");
                     }
-                    if (bounce_out) {
-                        slots[s].h_out[f] = fb200_host_alloc(out_elem * zc * out_level);
+                    if (bounce_out && io.out_unit[f]) {
+                        slots[s].h_out[f] = fb200_host_alloc(zc * io.out_unit[f]);
                         FB_REQUIRE(slots[s].h_out[f] != nullptr, "cannot allocate a page-locked staging buffer");
                     }
                 }
@@ -759,27 +770,29 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
             const size_t zn = (z0 + zc <= nz) ? zc : nz - z0;
             if (reused) // the kernel that read this slot's input three chunks ago is done
                 FB_CUDA_CHECK(cudaStreamWaitEvent(s_up, sl.computed, 0));
-            for (int f = 0; f < nfields; ++f) {
-                if (!in_level)
+            for (int f = 0; f < 2; ++f) {
+                if (!io.in_unit[f])
                     continue;
-                const char* src = static_cast<const char*>(in[f]) + z0 * in_level * in_elem;
+                const char* src = static_cast<const char*>(io.in[f]) + z0 * io.in_unit[f];
                 if (bounce_in) { // the upload that last read this bounce buffer finished before its chunk's download was waited for
-                    parallel_memcpy(sl.h_in[f], src, in_elem * zn * in_level);
+                    parallel_memcpy(sl.h_in[f], src, zn * io.in_unit[f]);
                     src = static_cast<const char*>(sl.h_in[f]);
                 }
-                FB_CUDA_CHECK(cudaMemcpyAsync(sl.d_in[f], src, in_elem * zn * in_level, cudaMemcpyHostToDevice, s_up));
+                FB_CUDA_CHECK(cudaMemcpyAsync(sl.d_in[f], src, zn * io.in_unit[f], cudaMemcpyHostToDevice, s_up));
             }
             FB_CUDA_CHECK(cudaEventRecord(sl.uploaded, s_up));
             FB_CUDA_CHECK(cudaStreamWaitEvent(s_run, sl.uploaded, 0));
             if (reused) // ... and the download of its previous output
                 FB_CUDA_CHECK(cudaStreamWaitEvent(s_run, sl.downloaded, 0));
-            if (run_slice_device(h, v, nfields, sl.d_in, zn, sl.d_out, io, s_run) != FB_OK)
+            if (run(sl.d_in, zn, sl.d_out, s_run) != FB_OK)
                 return FB_ERROR;
             FB_CUDA_CHECK(cudaEventRecord(sl.computed, s_run));
             FB_CUDA_CHECK(cudaStreamWaitEvent(s_down, sl.computed, 0));
-            for (int f = 0; f < nfields; ++f) {
-                char* dst = bounce_out ? static_cast<char*>(sl.h_out[f]) : static_cast<char*>(out[f]) + z0 * out_level * out_elem;
-                FB_CUDA_CHECK(cudaMemcpyAsync(dst, sl.d_out[f], out_elem * zn * out_level, cudaMemcpyDeviceToHost, s_down));
+            for (int f = 0; f < 2; ++f) {
+                if (!io.out_unit[f])
+                    continue;
+                char* dst = bounce_out ? static_cast<char*>(sl.h_out[f]) : static_cast<char*>(io.out[f]) + z0 * io.out_unit[f];
+                FB_CUDA_CHECK(cudaMemcpyAsync(dst, sl.d_out[f], zn * io.out_unit[f], cudaMemcpyDeviceToHost, s_down));
             }
             FB_CUDA_CHECK(cudaEventRecord(sl.downloaded, s_down));
             return FB_OK;
@@ -803,8 +816,9 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
             const size_t zn = (z0 + zc <= nz) ? zc : nz - z0;
             FB_CUDA_CHECK(cudaEventSynchronize(sl.downloaded));
             if (bounce_out)
-                for (int f = 0; f < nfields; ++f)
-                    parallel_memcpy(static_cast<char*>(out[f]) + z0 * out_level * out_elem, sl.h_out[f], out_elem * zn * out_level);
+                for (int f = 0; f < 2; ++f)
+                    if (io.out_unit[f])
+                        parallel_memcpy(static_cast<char*>(io.out[f]) + z0 * io.out_unit[f], sl.h_out[f], zn * io.out_unit[f]);
             if (chunk + nslots < nchunks && enqueue(chunk + nslots) != FB_OK)
                 return FB_ERROR;
         }
@@ -821,7 +835,7 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
     }
     // all work that touches the buffers is complete: hand them back in s_run's order (no further synchronisation needed)
     for (int s = 0; s < nslots; ++s) {
-        for (int f = 0; f < nfields; ++f) {
+        for (int f = 0; f < 2; ++f) {
             if (slots[s].d_in[f])
                 cudaFreeAsync(slots[s].d_in[f], s_run);
             if (slots[s].d_out[f])
@@ -836,6 +850,28 @@ int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, co
         fprintf(stderr, "[fb200 trace] host slice: setup %.3f ms, enqueue %.3f ms, wait %.3f ms, cleanup %.3f ms\n", t1 - t0, t2 - t1, t3 - t2,
                 now() - t3);
     return rc;
+}
+
+// `nfields` is 1 (scalar) or 2 (u/v); the levels are the units of the pipeline
+int run_slice_host(const fb200_interp* h, const fb200_vector* v, int nfields, const void* const* in, void* const* out, size_t nz,
+                   const SliceIO& io)
+{
+    const size_t in_level = h->inX * h->inY, out_level = h->outX * h->outY;
+    if (nz == 0 || out_level == 0)
+        return FB_OK;
+    const size_t in_elem = io.typed ? type_size(io.in_type) : sizeof(float), out_elem = io.typed ? type_size(io.out_type) : sizeof(float);
+    FB_REQUIRE(in_elem > 0 && out_elem > 0, "unsupported data type");
+    HostArrays arrays;
+    arrays.device = h->device;
+    for (int f = 0; f < nfields; ++f) {
+        arrays.in[f] = in[f];
+        arrays.in_unit[f] = in_level * in_elem;
+        arrays.out[f] = out[f];
+        arrays.out_unit[f] = out_level * out_elem;
+    }
+    return stage_host(arrays, nz, [&](const void* const* d_in, size_t zn, void* const* d_out, cudaStream_t st) {
+        return run_slice_device(h, v, nfields, d_in, zn, d_out, io, st);
+    });
 }
 
 // plain interpolateValues forms of the above
@@ -2022,6 +2058,194 @@ int fb200_vector_get_slice(const fb200_vector* v, int inType, const void* uIn, c
     FB_CUDA_CHECK(cudaMemcpyAsync(vOut, d_vo, ob, cudaMemcpyDeviceToHost, st));
     FB_CUDA_CHECK(cudaStreamSynchronize(st));
     return MIFI_OK;
+}
+
+} // extern "C"
+
+// ======================================================================================================
+// vertical interpolation to pressure levels (the pressure branch of CDMVerticalInterpolator)
+// ======================================================================================================
+struct fb200_vinterp {
+    int device = 0;
+    bool has_ps = false; // hybrid or sigma levels: the column pressures depend on the surface pressure
+    fb::VertTable vt;
+    ~fb200_vinterp()
+    {
+        fb::DeviceGuard on(device);
+        if (vt.d_tab)
+            cudaFree(vt.d_tab);
+    }
+};
+
+namespace {
+
+constexpr int kMaxVertLevels = 1024; // the coefficient table of one handle stays below 48 KB of shared memory
+
+bool all_finite(const double* v, int n)
+{
+    for (int i = 0; i < n; ++i)
+        if (!std::isfinite(v[i]))
+            return false;
+    return true;
+}
+
+// p_k = a_k + b_k * (ps * ps_scale - shift): hybrid a = ap, shift 0; sigma a = ptop, b = sigma, shift = ptop; pressure levels b = 0
+int vinterp_create(int method, const double* a, const double* b, int nk, bool sigma, double ptop, double ps_scale, const double* levels, int np,
+                   int extrapolate, fb200_vinterp** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(method >= FB_VINT_LIN && method <= FB_VINT_NN, "unknown vertical interpolation method " + std::to_string(method));
+    FB_REQUIRE(nk >= 2 && nk <= kMaxVertLevels, "number of source levels must be in [2, 1024], got " + std::to_string(nk));
+    FB_REQUIRE(np >= 1 && np <= kMaxVertLevels, "number of target levels must be in [1, 1024], got " + std::to_string(np));
+    FB_REQUIRE(levels != nullptr, "null target levels");
+    FB_REQUIRE(all_finite(levels, np), "target levels must be finite");
+    FB_REQUIRE(a != nullptr, sigma ? "null sigma" : "null ap (or pressure levels)");
+    FB_REQUIRE(all_finite(a, nk) && (b == nullptr || all_finite(b, nk)), "vertical coordinate values must be finite");
+    FB_REQUIRE(std::isfinite(ps_scale) && std::isfinite(ptop), "ps_scale and ptop must be finite");
+    if (use_device(default_device()) != FB_OK)
+        return FB_ERROR;
+    std::unique_ptr<fb200_vinterp> h(new fb200_vinterp());
+    h->device = default_device();
+    h->has_ps = sigma || b != nullptr;
+    VertTable& vt = h->vt;
+    vt.method = method;
+    vt.nk = nk;
+    vt.np = np;
+    vt.extrapolate = extrapolate != 0;
+    vt.ps_scale = ps_scale;
+    vt.shift = sigma ? ptop : 0.0;
+    std::vector<double> tab(2 * (size_t)nk + 3 * (size_t)np, 0.0);
+    for (int k = 0; k < nk; ++k) {
+        tab[k] = sigma ? ptop : a[k];
+        tab[nk + k] = sigma ? a[k] : (b ? b[k] : 0.0);
+    }
+    std::vector<int> order(np);
+    for (int i = 0; i < np; ++i)
+        order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return levels[x] < levels[y]; });
+    double* lev = tab.data() + 2 * nk;
+    for (int i = 0; i < np; ++i) {
+        lev[i] = levels[order[i]];
+        lev[2 * np + i] = order[i]; // the output row of the i-th smallest target
+    }
+    cudaStream_t st = cudaStreamPerThread;
+    if (dev_alloc(&vt.d_tab, tab.size()) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaMemcpyAsync(vt.d_tab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, st));
+    if (launch_vert_coords(method, vt.d_tab + 2 * nk, vt.d_tab + 2 * nk + np, np, st) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    *handle = h.release();
+    return FB_OK;
+}
+
+int check_vinterp_call(const fb200_vinterp* h, const void* in, const float* ps, size_t nxy, size_t nt, const void* out)
+{
+    FB_REQUIRE(h != nullptr, "null vertical interpolation handle");
+    FB_REQUIRE(nxy * nt == 0 || (in && out), "null data pointer");
+    FB_REQUIRE(!h->has_ps || nxy * nt == 0 || ps, "this vertical coordinate needs the surface pressure ps");
+    return use_device(h->device);
+}
+
+// typed: data2InterpolationArray (any CDM type, fill -> NaN) before and interpolationArray2Data (NaN -> fill, cast) after, both as
+// separate passes; untyped: float in, float out
+int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* d_in, const float* d_ps, size_t nxy, size_t nt, double bad,
+                   int out_type, void* d_out, cudaStream_t st)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    const size_t in_n = nxy * nt * (size_t)h->vt.nk, out_n = nxy * nt * (size_t)h->vt.np;
+    Scratch tmp(st);
+    const float* fin = static_cast<const float*>(d_in);
+    const bool has_bad = typed && !std::isnan((float)bad); // mifi_bad2nanf takes a float
+    if (typed && (in_type != FB_T_FLOAT || has_bad)) {
+        float* conv = nullptr;
+        if (tmp.get(&conv, in_n) != FB_OK || launch_as_float(in_type, d_in, (long long)in_n, has_bad, (float)bad, conv, st) != FB_OK)
+            return FB_ERROR;
+        fin = conv;
+    }
+    float* fout = static_cast<float*>(d_out);
+    if (typed && out_type != FB_T_FLOAT && tmp.get(&fout, out_n) != FB_OK)
+        return FB_ERROR;
+    if (launch_vertical(h->vt, fin, h->has_ps ? d_ps : nullptr, (long long)nxy, (long long)nt, fout, st) != FB_OK)
+        return FB_ERROR;
+    if (typed)
+        return launch_from_float(fout, (long long)out_n, out_type, bad, d_out, st);
+    return FB_OK;
+}
+
+// host arrays: time steps are the units of the staging pipeline of the horizontal calls
+int vinterp_host(const fb200_vinterp* h, bool typed, int in_type, const void* in, const float* ps, size_t nxy, size_t nt, double bad, int out_type,
+                 void* out)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    HostArrays arrays;
+    arrays.device = h->device;
+    arrays.in[0] = in;
+    arrays.in_unit[0] = nxy * (size_t)h->vt.nk * type_size(in_type);
+    if (h->has_ps) {
+        arrays.in[1] = ps;
+        arrays.in_unit[1] = nxy * sizeof(float);
+    }
+    arrays.out[0] = out;
+    arrays.out_unit[0] = nxy * (size_t)h->vt.np * type_size(out_type);
+    return stage_host(arrays, nt, [&](const void* const* d_in, size_t n, void* const* d_out, cudaStream_t st) {
+        return vinterp_device(h, typed, in_type, d_in[0], static_cast<const float*>(d_in[1]), nxy, n, bad, out_type, d_out[0], st);
+    });
+}
+
+} // namespace
+
+extern "C" {
+
+int fb200_vinterp_create_hybrid(int method, const double* ap, const double* b, int nk, double ps_scale, const double* levels, int np,
+                                int extrapolate, fb200_vinterp** handle)
+{
+    return vinterp_create(method, ap, b, nk, false, 0.0, ps_scale, levels, np, extrapolate, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_create_sigma(int method, const double* sigma, int nk, double ptop, double ps_scale, const double* levels, int np, int extrapolate,
+                               fb200_vinterp** handle)
+{
+    return vinterp_create(method, sigma, nullptr, nk, true, ptop, ps_scale, levels, np, extrapolate, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+void fb200_vinterp_destroy(fb200_vinterp* h)
+{
+    delete h;
+}
+
+int fb200_vinterp_interpolate_values(const fb200_vinterp* h, const float* in, const float* ps, size_t nxy, size_t nt, float* out)
+{
+    if (check_vinterp_call(h, in, ps, nxy, nt, out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_host(h, false, FB_T_FLOAT, in, ps, nxy, nt, 0.0, FB_T_FLOAT, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_interpolate_values_device(const fb200_vinterp* h, const float* d_in, const float* d_ps, size_t nxy, size_t nt, float* d_out,
+                                            void* stream)
+{
+    if (check_vinterp_call(h, d_in, d_ps, nxy, nt, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_device(h, false, FB_T_FLOAT, d_in, d_ps, nxy, nt, 0.0, FB_T_FLOAT, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_get_data_slice(const fb200_vinterp* h, int inType, const void* in, const float* ps, size_t nxy, size_t nt, double badValue,
+                                 int outType, void* out)
+{
+    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, in, ps, nxy, nt, out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_host(h, true, inType, in, ps, nxy, nt, badValue, outType, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_get_data_slice_device(const fb200_vinterp* h, int inType, const void* d_in, const float* d_ps, size_t nxy, size_t nt,
+                                        double badValue, int outType, void* d_out, void* stream)
+{
+    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, d_in, d_ps, nxy, nt, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_device(h, true, inType, d_in, d_ps, nxy, nt, badValue, outType, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
 }
 
 // ---------------------------------------------------------------------------------------- mifi_* drop-ins

@@ -136,4 +136,18 @@ int forward_build_plan(const int* d_cell, long long n_in, long long n_cells, For
 void forward_free_plan(ForwardPlan* plan);
 int launch_forward(int method, const ForwardPlan& plan, const float* d_in, float* d_out, long long nz, cudaStream_t st);
 
+// ---- vertical_kernels.cu (vertical interpolation to pressure levels) --------------------------------------------------
+// methods, numbered as the reference's MIFI_VINT_METHOD_* (include/fimex/mifi_constants.h)
+enum { FB_VINT_LIN = 0, FB_VINT_LOG = 1, FB_VINT_LOGLOG = 2, FB_VINT_NN = 3 };
+struct VertTable {
+    int method = 0, nk = 0, np = 0;
+    bool extrapolate = true;
+    double ps_scale = 1.0, shift = 0.0; // p_k = a_k + b_k * (ps * ps_scale - shift)
+    double* d_tab = nullptr;            // a[nk] | b[nk] | sorted targets[np] | their coordinates[np] | output row of each[np]
+};
+// the coordinate of each target the weights are linear in (p, ln p or ln ln p), computed with the kernel's own ln()
+int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st);
+// in [nt][nk][nxy], ps [nt][nxy] (null for pressure levels), out [nt][np][nxy]
+int launch_vertical(const VertTable& vt, const float* d_in, const float* d_ps, long long nxy, long long nt, float* d_out, cudaStream_t st);
+
 } // namespace fb

@@ -1,0 +1,209 @@
+// fimex_b200/csrc/vertical_kernels.cu -- vertical interpolation to pressure levels: the pressure branch of the reference's
+// CDMVerticalInterpolator (linear / log / loglog / nearest neighbour between the two model levels that bracket each target
+// pressure; the per-column step of mifi_get_values_linear_f / _log_f / _log_log_f, src/interpolation.c:1030-1156).
+//
+// One thread per column, consecutive lanes on consecutive columns, so every load of a level row and every store of a
+// target row coalesces.  The column's pressures are never materialised: p_k = a_k + b_k * q is evaluated from the
+// coefficients in shared memory where the walk needs it (q = ps * ps_scale for hybrid levels, ps * ps_scale - ptop for
+// sigma levels, 0 for pressure levels).  The targets are sorted once on the host, so one forward walk over k finds every
+// bracket; a bracket shared with the previous target (or shifted by one level) reuses the values held in registers, and
+// only the levels a column actually brackets are read.
+//
+// Arithmetic (DESIGN.md section 2): fp64, every product through __dmul_rn so that nothing is contracted into an FMA, and
+// ln() by vlog() below, the same sequence of IEEE operations as the oracle's orc_vlog (tests/vertical_oracle.c) -- results are bit-identical.
+#include "kernels.h"
+
+namespace fb {
+namespace {
+
+constexpr int kThreads = 256;
+
+// ln(x): fdlibm's __ieee754_log (e_log.c) -- argument reduction to [sqrt(2)/2, sqrt(2)) and a degree-14 odd polynomial in
+// s = f / (2 + f); < 1 ulp.  Only +, -, *, / and bit operations, so it rounds identically on the GPU and in plain C.
+__device__ double vlog(double x)
+{
+    const double ln2_hi = 6.93147180369123816490e-01, ln2_lo = 1.90821492927058770002e-10, two54 = 1.80143985094819840000e+16;
+    const double Lg1 = 6.666666666666735130e-01, Lg2 = 3.999999999940941908e-01, Lg3 = 2.857142874366239149e-01,
+                 Lg4 = 2.222219843214978396e-01, Lg5 = 1.818357216161805012e-01, Lg6 = 1.531383769920937332e-01,
+                 Lg7 = 1.479819860511658591e-01;
+    int hx = __double2hiint(x);
+    const unsigned lx = (unsigned)__double2loint(x);
+    int k = 0;
+    if (hx < 0x00100000) { // x < 2^-1022
+        if (((hx & 0x7fffffff) | lx) == 0)
+            return -__longlong_as_double(0x7ff0000000000000ll); // log(+-0) = -inf
+        if (hx < 0)
+            return __longlong_as_double(0x7ff8000000000000ll); // log(negative) = NaN
+        k -= 54;
+        x = __dmul_rn(x, two54); // subnormal: scale up
+        hx = __double2hiint(x);
+    }
+    if (hx >= 0x7ff00000)
+        return x + x; // inf, NaN
+    k += (hx >> 20) - 1023;
+    hx &= 0x000fffff;
+    const int i0 = (hx + 0x95f64) & 0x100000;
+    x = __hiloint2double(hx | (i0 ^ 0x3ff00000), __double2loint(x)); // normalise x or x / 2
+    k += (i0 >> 20);
+    const double f = x - 1.0;
+    const double dk = (double)k;
+    if ((0x000fffff & (2 + hx)) < 3) { // |f| < 2^-20
+        if (f == 0.0)
+            return k == 0 ? 0.0 : __dmul_rn(dk, ln2_hi) + __dmul_rn(dk, ln2_lo);
+        const double R = __dmul_rn(__dmul_rn(f, f), 0.5 - __dmul_rn(0.33333333333333333, f));
+        return k == 0 ? f - R : __dmul_rn(dk, ln2_hi) - ((R - __dmul_rn(dk, ln2_lo)) - f);
+    }
+    const double s = f / (2.0 + f);
+    const double z = __dmul_rn(s, s);
+    int i = hx - 0x6147a;
+    const double w = __dmul_rn(z, z);
+    const int j = 0x6b851 - hx;
+    const double t1 = __dmul_rn(w, Lg2 + __dmul_rn(w, Lg4 + __dmul_rn(w, Lg6)));
+    const double t2 = __dmul_rn(z, Lg1 + __dmul_rn(w, Lg3 + __dmul_rn(w, Lg5 + __dmul_rn(w, Lg7))));
+    i |= j;
+    const double R = t2 + t1;
+    if (i > 0) {
+        const double hfsq = __dmul_rn(__dmul_rn(0.5, f), f);
+        if (k == 0)
+            return f - (hfsq - __dmul_rn(s, hfsq + R));
+        return __dmul_rn(dk, ln2_hi) - ((hfsq - (__dmul_rn(s, hfsq + R) + __dmul_rn(dk, ln2_lo))) - f);
+    }
+    if (k == 0)
+        return f - __dmul_rn(s, f - R);
+    return __dmul_rn(dk, ln2_hi) - ((__dmul_rn(s, f - R) - __dmul_rn(dk, ln2_lo)) - f);
+}
+
+// the coordinate the weights are linear in: p (linear, nearest neighbour), ln p (log), ln ln p (loglog)
+template <int M>
+__device__ __forceinline__ double vcoord(double p)
+{
+    if (M == FB_VINT_LOG)
+        return vlog(p);
+    if (M == FB_VINT_LOGLOG)
+        return vlog(vlog(p));
+    return p;
+}
+
+__global__ void k_vert_coords(int method, const double* __restrict__ lev, double* __restrict__ x, int np)
+{
+    for (int i = threadIdx.x; i < np; i += blockDim.x) {
+        const double p = lev[i];
+        x[i] = method == FB_VINT_LOG ? vcoord<FB_VINT_LOG>(p) : method == FB_VINT_LOGLOG ? vcoord<FB_VINT_LOGLOG>(p) : p;
+    }
+}
+
+// in [nt][nk][nxy], ps [nt][nxy] (null for pressure levels), out [nt][np][nxy]; blockIdx.y = time step.
+// tab: a[nk] | b[nk] | sorted target pressures[np] | their coordinates[np] | output row of each sorted target[np]
+// (4 blocks per SM: 40-56 registers, no spills; without the minimum ptxas holds the kernel at 32 registers and spills)
+template <int M>
+__global__ void __launch_bounds__(kThreads, 4) k_vertical(const float* __restrict__ in, const float* __restrict__ ps, float* __restrict__ out,
+                                                       const double* __restrict__ tab, int nk, int np, int extrapolate, double ps_scale,
+                                                       double shift, long long nxy, long long t0)
+{
+    extern __shared__ double s_tab[];
+    const int ntab = 2 * nk + 3 * np;
+    for (int i = threadIdx.x; i < ntab; i += blockDim.x)
+        s_tab[i] = tab[i];
+    __syncthreads();
+    const double* s_a = s_tab;
+    const double* s_b = s_tab + nk;
+    const double* s_lev = s_tab + 2 * nk;
+    const double* s_x = s_lev + np;
+    const double* s_row = s_x + np;
+
+    const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (c >= nxy)
+        return;
+    const long long t = t0 + blockIdx.y;
+    const float* col = in + t * nk * nxy + c;
+    float* ocol = out + t * np * nxy + c;
+    const double q = ps ? __dmul_rn((double)__ldg(ps + t * nxy + c), ps_scale) - shift : 0.0;
+    auto pres = [&](int k) { return s_a[k] + __dmul_rn(s_b[k], q); };
+
+    const double p0 = pres(0), pl = pres(nk - 1);
+    const bool incr = p0 < pl;
+    const bool flat = !(p0 < pl) && !(p0 > pl); // equal ends or NaN
+    const double lo = incr ? p0 : pl, hi = incr ? pl : p0;
+    // Targets in the column's direction: the bracket index j (first level at or beyond P) never moves back.
+    int j = 1, kc = -2;
+    double pa = 0., pb = 0., xa = 0., xb = 0.;
+    float va = 0.f, vb = 0.f;
+    for (int ii = 0; ii < np; ++ii) {
+        const int i = incr ? ii : np - 1 - ii;
+        const double P = s_lev[i];
+        float r = undef_f();
+        if (!flat && (extrapolate || (P >= lo && P <= hi))) {
+            if (incr) {
+                while (j < nk - 1 && pres(j) < P)
+                    ++j;
+            } else {
+                while (j < nk - 1 && pres(j) > P)
+                    ++j;
+            }
+            const int k = j - 1;
+            if (k != kc) {
+                if (k == kc + 1) { // the lower level of this bracket is the upper one of the last
+                    pa = pb;
+                    xa = xb;
+                    va = vb;
+                } else {
+                    pa = pres(k);
+                    xa = vcoord<M>(pa);
+                    va = __ldg(col + (long long)k * nxy);
+                }
+                pb = pres(k + 1);
+                xb = vcoord<M>(pb);
+                vb = __ldg(col + (long long)(k + 1) * nxy);
+                kc = k;
+            }
+            if (M == FB_VINT_NN) {
+                r = fabs(P - pb) < fabs(P - pa) ? vb : va;
+            } else {
+                const double w = xa == xb ? 0.0 : (s_x[i] - xa) / (xb - xa);
+                r = (float)((double)va + __dmul_rn(w, (double)vb - (double)va));
+            }
+        }
+        __stcs(ocol + (long long)s_row[i] * nxy, r);
+    }
+}
+
+} // namespace
+
+int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st)
+{
+    k_vert_coords<<<1, kThreads, 0, st>>>(method, d_lev, d_x, np);
+    count_launch();
+    FB_CUDA_CHECK(cudaGetLastError());
+    return FB_OK;
+}
+
+int launch_vertical(const VertTable& vt, const float* d_in, const float* d_ps, long long nxy, long long nt, float* d_out, cudaStream_t st)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    const size_t smem = sizeof(double) * (size_t)(2 * vt.nk + 3 * vt.np);
+    const long long bx = (nxy + kThreads - 1) / kThreads;
+    FB_REQUIRE(bx < 2147483647LL, "too many columns for one call");
+    for (long long t0 = 0; t0 < nt; t0 += 65535) {
+        const dim3 grid((unsigned)bx, (unsigned)std::min<long long>(nt - t0, 65535));
+        switch (vt.method) {
+#define FB_CASE(M)                                                                                                                         \
+    case M:                                                                                                                                \
+        k_vertical<M><<<grid, kThreads, smem, st>>>(d_in, d_ps, d_out, vt.d_tab, vt.nk, vt.np, vt.extrapolate ? 1 : 0, vt.ps_scale,       \
+                                                    vt.shift, nxy, t0);                                                                    \
+        break;
+            FB_CASE(FB_VINT_LIN)
+            FB_CASE(FB_VINT_LOG)
+            FB_CASE(FB_VINT_LOGLOG)
+            FB_CASE(FB_VINT_NN)
+#undef FB_CASE
+        default:
+            FB_REQUIRE(false, "unknown vertical interpolation method " + std::to_string(vt.method));
+        }
+        count_launch();
+        FB_CUDA_CHECK(cudaGetLastError());
+    }
+    return FB_OK;
+}
+
+} // namespace fb

@@ -1,0 +1,146 @@
+"""Host-side mirror of the pressure branch of the reference's CDMVerticalInterpolator
+(``--verticalInterpolate.type=pressure --verticalInterpolate.method=... --verticalInterpolate.level1=...``).
+
+The source vertical coordinate is given by its CF standard name and formula terms, as the reference reads them from the CDM:
+
+* ``air_pressure``: pressure levels, terms ``{"p": levels}``;
+* ``atmosphere_hybrid_sigma_pressure_coordinate``: terms ``{"ap": ap, "b": b}`` or ``{"a": a, "p0": p0, "b": b}``;
+* ``atmosphere_sigma_coordinate``: terms ``{"sigma": sigma, "ptop": ptop}``.
+
+The surface pressure ``ps`` is not a term here: it is a field, passed with every slice.  All pressures are in the unit of the
+target levels (hPa, as the reference's level1 option); ``ps_scale`` converts the ``ps`` field to it (0.01 for Pa).  The
+arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md section 2 states it).
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import numpy as np
+
+from . import capi
+from .cached import _is_torch, _stream_ptr
+from .capi import FimexB200Error, check, f64, load, ptr
+
+#: --verticalInterpolate.method values -> MIFI_VINT_METHOD_* (include/fimex/mifi_constants.h)
+METHODS = {"linear": 0, "log": 1, "loglog": 2, "nearestneighbor": 3}
+
+PRESSURE = "air_pressure"
+HYBRID = "atmosphere_hybrid_sigma_pressure_coordinate"
+SIGMA = "atmosphere_sigma_coordinate"
+
+
+def vertical_method(name: str) -> int:
+    """--verticalInterpolate.method string -> MIFI_VINT_METHOD_*; an unknown name raises"""
+    try:
+        return METHODS[name]
+    except KeyError:
+        raise FimexB200Error(f"unknown vertical interpolation method: '{name}' (one of {', '.join(METHODS)})") from None
+
+
+class VerticalInterpolator:
+    """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on the target pressure levels."""
+
+    def __init__(self, standard_name: str, terms: dict, method: str, levels, ps_scale: float = 1.0, extrapolate: bool = True):
+        self.method = vertical_method(method)
+        self.levels = f64(levels).ravel()
+        self._h = C.c_void_p()
+        lib = load()
+        t = {k: v for k, v in terms.items() if k != "ps"}
+        if standard_name == PRESSURE:
+            p = f64(t["p"]).ravel()
+            self.nk, self.needs_ps = p.size, False
+            rc = lib.fb200_vinterp_create_hybrid(self.method, ptr(p), None, p.size, float(ps_scale), ptr(self.levels), self.levels.size,
+                                                 int(bool(extrapolate)), C.byref(self._h))
+        elif standard_name == HYBRID:
+            if "ap" in t:
+                ap = f64(t["ap"]).ravel()
+            elif "a" in t and "p0" in t:
+                ap = f64(t["a"]).ravel() * float(np.asarray(t["p0"], dtype=np.float64).reshape(-1)[0])  # ap_k = a_k * p0, fp64
+            else:
+                raise FimexB200Error(f"{HYBRID} needs the terms ap, b or a, p0, b; got {sorted(terms)}")
+            b = f64(t["b"]).ravel()
+            if b.size != ap.size:
+                raise FimexB200Error(f"{HYBRID}: {ap.size} values of ap but {b.size} of b")
+            self.nk, self.needs_ps = ap.size, True
+            rc = lib.fb200_vinterp_create_hybrid(self.method, ptr(ap), ptr(b), ap.size, float(ps_scale), ptr(self.levels), self.levels.size,
+                                                 int(bool(extrapolate)), C.byref(self._h))
+        elif standard_name == SIGMA:
+            sigma = f64(t["sigma"]).ravel()
+            ptop = float(np.asarray(t["ptop"], dtype=np.float64).reshape(-1)[0])
+            self.nk, self.needs_ps = sigma.size, True
+            rc = lib.fb200_vinterp_create_sigma(self.method, ptr(sigma), sigma.size, ptop, float(ps_scale), ptr(self.levels), self.levels.size,
+                                                int(bool(extrapolate)), C.byref(self._h))
+        else:
+            raise FimexB200Error(f"vertical coordinate '{standard_name}' is not supported (one of {PRESSURE}, {HYBRID}, {SIGMA})")
+        check(rc, "VerticalInterpolator")
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h:
+            load().fb200_vinterp_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _shape(self, field, ps):
+        if field.ndim < 2 or field.shape[1] != self.nk:
+            raise FimexB200Error(f"field must be [nt][{self.nk}][...], got shape {tuple(field.shape)}")
+        nt = int(field.shape[0])
+        nxy = int(np.prod(field.shape[2:], dtype=np.int64))
+        if self.needs_ps and (ps is None or int(np.prod(ps.shape, dtype=np.int64)) != nt * nxy):
+            raise FimexB200Error(f"ps must hold nt * nxy = {nt * nxy} values")
+        return nt, nxy, (nt, self.levels.size) + tuple(field.shape[2:])
+
+    def interpolateValues(self, field, ps=None, stream=None):
+        """float32 [nt][nk][...] with NaN for undefined values -> float32 [nt][np][...] (numpy or CUDA tensors)"""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
+            nt, nxy, shape = self._shape(field, ps)
+            psd = ps.contiguous() if ps is not None and self.needs_ps else None
+            out = torch.empty(shape, dtype=torch.float32, device=field.device)
+            check(lib.fb200_vinterp_interpolate_values_device(self._h, ptr(field), ptr(psd), nxy, nt, ptr(out), _stream_ptr(stream)),
+                  "interpolateValues")
+            return out
+        a = capi.f32(field)
+        nt, nxy, shape = self._shape(a, ps)
+        p = capi.f32(ps) if ps is not None and self.needs_ps else None
+        out = np.empty(shape, dtype=np.float32)
+        check(lib.fb200_vinterp_interpolate_values(self._h, ptr(a), ptr(p), nxy, nt, ptr(out)), "interpolateValues")
+        return out
+
+    def getDataSlice(self, field, ps=None, bad_value=None, out_dtype=None, stream=None):
+        """The per-slice body of the vertical getDataSlice: `field` [nt][nk][...] of any CDM numeric type (numpy array, or CUDA tensor
+        for the device-resident path), fill -> NaN, interpolate, NaN -> fill and cast to `out_dtype` (default: the input's type).
+        `bad_value` = CDM::getFillValue of the variable (default: the type's default fill value); `ps` [nt][...] float32."""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous CUDA tensor")
+            odt = out_dtype if out_dtype is not None else field.dtype
+            bad = capi.default_fill_value(field.dtype) if bad_value is None else float(bad_value)
+            nt, nxy, shape = self._shape(field, ps)
+            psd = None
+            if ps is not None and self.needs_ps:
+                if not ps.is_cuda or ps.dtype != torch.float32:
+                    raise FimexB200Error("ps must be a float32 CUDA tensor on the device path")
+                psd = ps.contiguous()
+            out = torch.empty(shape, dtype=odt, device=field.device)
+            check(lib.fb200_vinterp_get_data_slice_device(self._h, int(capi.cdm_type(field.dtype)), ptr(field), ptr(psd), nxy, nt, bad,
+                                                          int(capi.cdm_type(odt)), ptr(out), _stream_ptr(stream)), "getDataSlice")
+            return out
+        a = np.ascontiguousarray(field)
+        odt = np.dtype(out_dtype) if out_dtype is not None else a.dtype
+        bad = capi.default_fill_value(a.dtype) if bad_value is None else float(bad_value)
+        nt, nxy, shape = self._shape(a, ps)
+        p = capi.f32(ps) if ps is not None and self.needs_ps else None
+        out = np.empty(shape, dtype=odt)
+        check(lib.fb200_vinterp_get_data_slice(self._h, int(capi.cdm_type(a.dtype)), ptr(a), ptr(p), nxy, nt, bad, int(capi.cdm_type(odt)),
+                                               ptr(out)), "getDataSlice")
+        return out

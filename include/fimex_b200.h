@@ -285,6 +285,45 @@ int fb200_interp_get_vector_slice_device(const fb200_interp* handle, const fb200
                                          void* d_vOut, size_t* newSize, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * (1d) vertical interpolation to pressure levels: the pressure branch of CDMVerticalInterpolator
+ *      (--verticalInterpolate.type=pressure; DESIGN.md section 2 states the arithmetic)
+ *
+ * Source vertical coordinates, all pressures in ONE unit, that of the target levels (hPa, as the reference's level1 option):
+ *   pressure levels                          p_k = ap_k                                  (create_hybrid with b == NULL)
+ *   atmosphere_hybrid_sigma_pressure_coordinate  p_k = ap_k + b_k * (ps * ps_scale)      (a, p0 form: pass ap_k = a_k * p0)
+ *   atmosphere_sigma_coordinate              p_k = ptop + sigma_k * (ps * ps_scale - ptop)
+ * ps_scale converts the surface pressure field to that unit (0.01 for a Pa field against hPa levels).
+ * method: MIFI_VINT_METHOD_LIN 0, _LOG 1, _LOGLOG 2, _NN 3 (the reference's numbering).  extrapolate != 0: targets outside a
+ * column's pressure range use the end pair of levels on that side; 0: they give NaN.  2 <= nk, np <= 1024, all values finite.
+ * The handle is immutable and every call re-entrant, as for the horizontal handles.
+ * ---------------------------------------------------------------------------------------------- */
+#ifndef MIFI_VINT_METHOD_LIN
+#define MIFI_VINT_METHOD_LIN 0
+#define MIFI_VINT_METHOD_LOG 1
+#define MIFI_VINT_METHOD_LOGLOG 2
+#define MIFI_VINT_METHOD_NN 3
+#endif
+typedef struct fb200_vinterp fb200_vinterp; /* opaque */
+
+int fb200_vinterp_create_hybrid(int method, const double* ap, const double* b, int nk, double ps_scale, const double* levels, int np,
+                                int extrapolate, fb200_vinterp** handle);
+int fb200_vinterp_create_sigma(int method, const double* sigma, int nk, double ptop, double ps_scale, const double* levels, int np, int extrapolate,
+                               fb200_vinterp** handle);
+void fb200_vinterp_destroy(fb200_vinterp* handle);
+/* in: [nt][nk][nxy] floats (NaN = undefined), ps: [nt][nxy] floats (may be NULL for pressure levels), out: [nt][np][nxy] floats,
+ * the target levels in the order they were given.  Host buffers (copies pipelined over the time steps) or, for _device, device
+ * pointers on `cuda_stream` without synchronisation. */
+int fb200_vinterp_interpolate_values(const fb200_vinterp* handle, const float* in, const float* ps, size_t nxy, size_t nt, float* out);
+int fb200_vinterp_interpolate_values_device(const fb200_vinterp* handle, const float* d_in, const float* d_ps, size_t nxy, size_t nt, float* d_out,
+                                            void* cuda_stream);
+/* the per-slice body of the vertical getDataSlice: inType / outType as in (1c), badValue -> NaN on the way in, NaN -> badValue and
+ * round + cast on the way out */
+int fb200_vinterp_get_data_slice(const fb200_vinterp* handle, int inType, const void* in, const float* ps, size_t nxy, size_t nt, double badValue,
+                                 int outType, void* out);
+int fb200_vinterp_get_data_slice_device(const fb200_vinterp* handle, int inType, const void* d_in, const float* d_ps, size_t nxy, size_t nt,
+                                        double badValue, int outType, void* d_out, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
  * ---------------------------------------------------------------------------------------------- */
 int mifi_string_to_interpolation_method(const char* stringMethod); /* :44 */
