@@ -666,14 +666,15 @@ void parallel_memcpy(void* dst, const void* src, size_t bytes)
         w.join();
 }
 
-// Host arrays of a call that the device works through in chunks of `units` (levels, time steps): up to two inputs and two
+// Host arrays of a call that the device works through in chunks of `units` (levels, time steps): up to four inputs and two
 // outputs, each `bytes per unit` long per unit (0: that array is absent and its device pointer is null).
+constexpr int kHostIn = 4, kHostOut = 2;
 struct HostArrays {
     int device = 0;
-    const void* in[2] = {nullptr, nullptr};
-    size_t in_unit[2] = {0, 0};
-    void* out[2] = {nullptr, nullptr};
-    size_t out_unit[2] = {0, 0};
+    const void* in[kHostIn] = {nullptr, nullptr, nullptr, nullptr};
+    size_t in_unit[kHostIn] = {0, 0, 0, 0};
+    void* out[kHostOut] = {nullptr, nullptr};
+    size_t out_unit[kHostOut] = {0, 0};
 };
 // the device work of one chunk: `n` units of every array, already on the device
 using ChunkRun = std::function<int(const void* const* d_in, size_t n, void* const* d_out, cudaStream_t st)>;
@@ -684,8 +685,10 @@ using ChunkRun = std::function<int(const void* const* d_in, size_t n, void* cons
 int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
 {
     size_t bytes_per_level = 0;
-    for (int f = 0; f < 2; ++f)
-        bytes_per_level += io.in_unit[f] + io.out_unit[f];
+    for (int f = 0; f < kHostIn; ++f)
+        bytes_per_level += io.in_unit[f];
+    for (int f = 0; f < kHostOut; ++f)
+        bytes_per_level += io.out_unit[f];
     size_t chunk_bytes = 192ull << 20;
     if (const char* env = std::getenv("FIMEX_B200_HOST_CHUNK_MB")) // experiments: bytes of (input + output) per pipeline chunk
         if (std::atoll(env) > 0)
@@ -703,10 +706,10 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
     bool bounce_in = false, bounce_out = false; // pageable host arrays: staged through page-locked bounce buffers, see above
     // (with fewer than 4 host threads the driver's own staging, one thread at ~15 GB/s, is as fast; small calls are latency-bound)
     if (copy_threads() >= 4 && nz * bytes_per_level >= (size_t)(8u << 20)) {
-        for (int f = 0; f < 2; ++f) {
+        for (int f = 0; f < kHostIn; ++f)
             bounce_in = bounce_in || (io.in_unit[f] && host_pageable(io.in[f]));
+        for (int f = 0; f < kHostOut; ++f)
             bounce_out = bounce_out || (io.out_unit[f] && host_pageable(io.out[f]));
-        }
     }
     if ((bounce_in || bounce_out) && zc * bytes_per_level > (64ull << 20)) { // smaller chunks: the host copy of chunk k runs while k+1, k+2 are in flight
         zc = (64ull << 20) / bytes_per_level;
@@ -715,10 +718,10 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
     }
     const int nslots = (nz > zc) ? 3 : 1;
     struct Slot {
-        void* d_in[2] = {nullptr, nullptr};
-        void* d_out[2] = {nullptr, nullptr};
-        void* h_in[2] = {nullptr, nullptr};  // bounce buffers (page-locked, from the pinned cache)
-        void* h_out[2] = {nullptr, nullptr};
+        void* d_in[kHostIn] = {nullptr, nullptr, nullptr, nullptr};
+        void* d_out[kHostOut] = {nullptr, nullptr};
+        void* h_in[kHostIn] = {nullptr, nullptr, nullptr, nullptr}; // bounce buffers (page-locked, from the pinned cache)
+        void* h_out[kHostOut] = {nullptr, nullptr};
         cudaEvent_t uploaded = nullptr, computed = nullptr, downloaded = nullptr;
     } slots[3];
     HostPipe* pipe = host_pipe(io.device);
@@ -735,12 +738,12 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
     double t0 = now(), t1 = 0, t2 = 0, t3 = 0;
     auto body = [&]() -> int {
         for (int s = 0; s < nslots; ++s) {
-            for (int f = 0; f < 2; ++f) {
+            for (int f = 0; f < kHostIn; ++f)
                 if (io.in_unit[f])
                     FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_in[f], zc * io.in_unit[f], s_run));
+            for (int f = 0; f < kHostOut; ++f)
                 if (io.out_unit[f])
                     FB_CUDA_CHECK(cudaMallocAsync(&slots[s].d_out[f], zc * io.out_unit[f], s_run));
-            }
         }
         // the buffers were allocated in s_run's order: the copy streams must not touch them earlier
         cudaEvent_t ready = pipe->ready;
@@ -749,11 +752,13 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
         FB_CUDA_CHECK(cudaStreamWaitEvent(s_down, ready, 0));
         if (bounce_in || bounce_out) {
             for (int s = 0; s < nslots; ++s) {
-                for (int f = 0; f < 2; ++f) {
+                for (int f = 0; f < kHostIn; ++f) {
                     if (bounce_in && io.in_unit[f]) {
                         slots[s].h_in[f] = fb200_host_alloc(zc * io.in_unit[f]);
                         FB_REQUIRE(slots[s].h_in[f] != nullptr, "cannot allocate a page-locked staging buffer");
                     }
+                }
+                for (int f = 0; f < kHostOut; ++f) {
                     if (bounce_out && io.out_unit[f]) {
                         slots[s].h_out[f] = fb200_host_alloc(zc * io.out_unit[f]);
                         FB_REQUIRE(slots[s].h_out[f] != nullptr, "cannot allocate a page-locked staging buffer");
@@ -770,7 +775,7 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
             const size_t zn = (z0 + zc <= nz) ? zc : nz - z0;
             if (reused) // the kernel that read this slot's input three chunks ago is done
                 FB_CUDA_CHECK(cudaStreamWaitEvent(s_up, sl.computed, 0));
-            for (int f = 0; f < 2; ++f) {
+            for (int f = 0; f < kHostIn; ++f) {
                 if (!io.in_unit[f])
                     continue;
                 const char* src = static_cast<const char*>(io.in[f]) + z0 * io.in_unit[f];
@@ -788,7 +793,7 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
                 return FB_ERROR;
             FB_CUDA_CHECK(cudaEventRecord(sl.computed, s_run));
             FB_CUDA_CHECK(cudaStreamWaitEvent(s_down, sl.computed, 0));
-            for (int f = 0; f < 2; ++f) {
+            for (int f = 0; f < kHostOut; ++f) {
                 if (!io.out_unit[f])
                     continue;
                 char* dst = bounce_out ? static_cast<char*>(sl.h_out[f]) : static_cast<char*>(io.out[f]) + z0 * io.out_unit[f];
@@ -816,7 +821,7 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
             const size_t zn = (z0 + zc <= nz) ? zc : nz - z0;
             FB_CUDA_CHECK(cudaEventSynchronize(sl.downloaded));
             if (bounce_out)
-                for (int f = 0; f < 2; ++f)
+                for (int f = 0; f < kHostOut; ++f)
                     if (io.out_unit[f])
                         parallel_memcpy(static_cast<char*>(io.out[f]) + z0 * io.out_unit[f], sl.h_out[f], zn * io.out_unit[f]);
             if (chunk + nslots < nchunks && enqueue(chunk + nslots) != FB_OK)
@@ -835,13 +840,15 @@ int stage_host(const HostArrays& io, size_t nz, const ChunkRun& run)
     }
     // all work that touches the buffers is complete: hand them back in s_run's order (no further synchronisation needed)
     for (int s = 0; s < nslots; ++s) {
-        for (int f = 0; f < 2; ++f) {
+        for (int f = 0; f < kHostIn; ++f) {
             if (slots[s].d_in[f])
                 cudaFreeAsync(slots[s].d_in[f], s_run);
-            if (slots[s].d_out[f])
-                cudaFreeAsync(slots[s].d_out[f], s_run);
             if (slots[s].h_in[f])
                 fb200_host_free(slots[s].h_in[f]);
+        }
+        for (int f = 0; f < kHostOut; ++f) {
+            if (slots[s].d_out[f])
+                cudaFreeAsync(slots[s].d_out[f], s_run);
             if (slots[s].h_out[f])
                 fb200_host_free(slots[s].h_out[f]);
         }
@@ -2063,11 +2070,15 @@ int fb200_vector_get_slice(const fb200_vector* v, int inType, const void* uIn, c
 } // extern "C"
 
 // ======================================================================================================
-// vertical interpolation to pressure levels (the pressure branch of CDMVerticalInterpolator)
+// vertical interpolation to pressure levels (the pressure branch of CDMVerticalInterpolator) and to height and altitude levels
+// (its height branch)
 // ======================================================================================================
 struct fb200_vinterp {
     int device = 0;
-    bool has_ps = false; // hybrid or sigma levels: the column pressures depend on the surface pressure
+    bool has_ps = false;   // the column pressures depend on the surface pressure (hybrid or sigma levels), and the converter uses them
+    bool needs_t = false;  // height handles: the hypsometric converter integrates the air temperature (and q, when given)
+    bool needs_z = false;  // the field converter reads the altitude field z
+    bool needs_zs = false; // the surface altitude: height targets of the standard and field converters, altitude targets of the hypsometric one
     fb::VertTable vt;
     ~fb200_vinterp()
     {
@@ -2087,6 +2098,27 @@ bool all_finite(const double* v, int n)
         if (!std::isfinite(v[i]))
             return false;
     return true;
+}
+
+// the targets in ascending order into lev[np], and the output row of each into row[np]
+void sort_targets(const double* levels, int np, double* lev, double* row)
+{
+    std::vector<int> order(np);
+    for (int i = 0; i < np; ++i)
+        order[i] = i;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return levels[x] < levels[y]; });
+    for (int i = 0; i < np; ++i) {
+        lev[i] = levels[order[i]];
+        row[i] = order[i];
+    }
+}
+
+int upload_table(VertTable& vt, const std::vector<double>& tab, cudaStream_t st)
+{
+    if (dev_alloc(&vt.d_tab, tab.size()) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaMemcpyAsync(vt.d_tab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, st));
+    return FB_OK;
 }
 
 // p_k = a_k + b_k * (ps * ps_scale - shift): hybrid a = ap, shift 0; sigma a = ptop, b = sigma, shift = ptop; pressure levels b = 0
@@ -2120,19 +2152,11 @@ int vinterp_create(int method, const double* a, const double* b, int nk, bool si
         tab[k] = sigma ? ptop : a[k];
         tab[nk + k] = sigma ? a[k] : (b ? b[k] : 0.0);
     }
-    std::vector<int> order(np);
-    for (int i = 0; i < np; ++i)
-        order[i] = i;
-    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return levels[x] < levels[y]; });
     double* lev = tab.data() + 2 * nk;
-    for (int i = 0; i < np; ++i) {
-        lev[i] = levels[order[i]];
-        lev[2 * np + i] = order[i]; // the output row of the i-th smallest target
-    }
+    sort_targets(levels, np, lev, lev + 2 * np);
     cudaStream_t st = cudaStreamPerThread;
-    if (dev_alloc(&vt.d_tab, tab.size()) != FB_OK)
+    if (upload_table(vt, tab, st) != FB_OK)
         return FB_ERROR;
-    FB_CUDA_CHECK(cudaMemcpyAsync(vt.d_tab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, st));
     if (launch_vert_coords(method, vt.d_tab + 2 * nk, vt.d_tab + 2 * nk + np, np, st) != FB_OK)
         return FB_ERROR;
     FB_CUDA_CHECK(cudaStreamSynchronize(st));
@@ -2140,18 +2164,107 @@ int vinterp_create(int method, const double* a, const double* b, int nk, bool si
     return FB_OK;
 }
 
-int check_vinterp_call(const fb200_vinterp* h, const void* in, const float* ps, size_t nxy, size_t nt, const void* out)
+// The standard atmosphere (US Standard Atmosphere 1976 / ICAO): geopotential layers with base altitude h_b [m], base temperature
+// T_b [K], lapse rate L_b [K/m] and the published base pressure p_b [hPa]; the gas constant R* [J/(mol K)], the molar masses of dry
+// air M and of water M_w [kg/mol], g0 [m/s2].  tests/vertical_height_oracle.c forms the same constants with the same expressions.
+constexpr double kStdH[kStdLayers] = {0.0, 11000.0, 20000.0, 32000.0, 47000.0, 51000.0, 71000.0};
+constexpr double kStdT[kStdLayers] = {288.15, 216.65, 216.65, 228.65, 270.65, 270.65, 214.65};
+constexpr double kStdL[kStdLayers] = {-6.5e-3, 0.0, 1e-3, 2.8e-3, 0.0, -2.8e-3, -2e-3};
+constexpr double kStdP[kStdLayers] = {1013.25, 226.3206, 54.74889, 8.680187, 1.109063, 0.6693887, 0.03956420};
+constexpr double kRstar = 8.31432, kMair = 0.0289644, kMwater = 0.01801528, kG0 = 9.80665;
+
+int vinterp_create_height(int method, int converter, int target, int vcoord, const double* a, const double* b, int nk, double ptop,
+                          double ps_scale, double z_scale, double zs_scale, const double* levels, int np, int extrapolate, fb200_vinterp** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(method == FB_VINT_LIN || method == FB_VINT_NN,
+               "height levels take the methods linear and nearestneighbor only (log and loglog are defined on ln p), got " + std::to_string(method));
+    FB_REQUIRE(converter >= FB_VZ_STANDARD && converter <= FB_VZ_FIELD, "unknown height converter " + std::to_string(converter));
+    FB_REQUIRE(target == FB_VZ_ALTITUDE || target == FB_VZ_HEIGHT, "unknown height target " + std::to_string(target));
+    const bool field = converter == FB_VZ_FIELD;
+    FB_REQUIRE(field || (vcoord >= FB200_VCOORD_PRESSURE && vcoord <= FB200_VCOORD_SIGMA), "unknown source vertical coordinate " + std::to_string(vcoord));
+    FB_REQUIRE(converter != FB_VZ_HYPSOMETRIC || vcoord != FB200_VCOORD_PRESSURE,
+               "the hypsometric converter needs a surface pressure: hybrid or sigma source levels, not pressure levels");
+    FB_REQUIRE(nk >= 2 && nk <= kMaxVertLevels, "number of source levels must be in [2, 1024], got " + std::to_string(nk));
+    FB_REQUIRE(np >= 1 && np <= kMaxVertLevels, "number of target levels must be in [1, 1024], got " + std::to_string(np));
+    FB_REQUIRE(levels != nullptr, "null target levels");
+    FB_REQUIRE(all_finite(levels, np), "target levels must be finite");
+    const bool sigma = vcoord == FB200_VCOORD_SIGMA, hybrid = vcoord == FB200_VCOORD_HYBRID;
+    if (!field) { // the field converter does not use the source's formula terms
+        FB_REQUIRE(sigma || a != nullptr, "null ap (or pressure levels)");
+        FB_REQUIRE(!(sigma || hybrid) || b != nullptr, sigma ? "null sigma" : "null b");
+        FB_REQUIRE((sigma || all_finite(a, nk)) && (!(sigma || hybrid) || all_finite(b, nk)), "vertical coordinate values must be finite");
+    }
+    FB_REQUIRE(std::isfinite(ps_scale) && std::isfinite(ptop) && std::isfinite(z_scale) && std::isfinite(zs_scale),
+               "ps_scale, ptop, z_scale and zs_scale must be finite");
+    if (use_device(default_device()) != FB_OK)
+        return FB_ERROR;
+    std::unique_ptr<fb200_vinterp> h(new fb200_vinterp());
+    h->device = default_device();
+    h->has_ps = converter == FB_VZ_HYPSOMETRIC || (converter == FB_VZ_STANDARD && vcoord != FB200_VCOORD_PRESSURE);
+    h->needs_t = converter == FB_VZ_HYPSOMETRIC;
+    h->needs_z = field;
+    h->needs_zs = (target == FB_VZ_HEIGHT) != (converter == FB_VZ_HYPSOMETRIC);
+    VertTable& vt = h->vt;
+    vt.method = method;
+    vt.nk = nk;
+    vt.np = np;
+    vt.extrapolate = extrapolate != 0;
+    vt.ps_scale = ps_scale;
+    vt.shift = sigma ? ptop : 0.0;
+    vt.converter = converter;
+    vt.target = target;
+    vt.z_scale = z_scale;
+    vt.zs_scale = zs_scale;
+    vt.H = kRstar / (kMair * kG0);
+    vt.cq = kMair / kMwater - 1.0;
+    std::vector<double> tab(2 * (size_t)nk + 4 * kStdLayers + 2 * (size_t)np, 0.0);
+    for (int k = 0; k < nk && !field; ++k) {
+        tab[k] = sigma ? ptop : a[k];
+        tab[nk + k] = (sigma || hybrid) ? b[k] : 0.0;
+    }
+    double* layers = tab.data() + 2 * nk; // h_b | p_b | c_b | e_b
+    for (int l = 0; l < kStdLayers; ++l) {
+        layers[l] = kStdH[l];
+        layers[kStdLayers + l] = kStdP[l];
+        layers[2 * kStdLayers + l] = kStdL[l] != 0.0 ? kStdT[l] / kStdL[l] : vt.H * kStdT[l];
+        layers[3 * kStdLayers + l] = kStdL[l] != 0.0 ? -(kRstar * kStdL[l]) / (kG0 * kMair) : 0.0;
+    }
+    double* lev = layers + 4 * kStdLayers;
+    sort_targets(levels, np, lev, lev + np);
+    cudaStream_t st = cudaStreamPerThread;
+    if (upload_table(vt, tab, st) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    *handle = h.release();
+    return FB_OK;
+}
+
+int check_vinterp_call(const fb200_vinterp* h, const void* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, const void* out)
 {
     FB_REQUIRE(h != nullptr, "null vertical interpolation handle");
     FB_REQUIRE(nxy * nt == 0 || (in && out), "null data pointer");
-    FB_REQUIRE(!h->has_ps || nxy * nt == 0 || ps, "this vertical coordinate needs the surface pressure ps");
+    if (nxy * nt != 0) {
+        FB_REQUIRE(!h->has_ps || cols.ps, "this vertical coordinate needs the surface pressure ps");
+        FB_REQUIRE(!h->needs_t || cols.t, "the hypsometric converter needs the air temperature t");
+        FB_REQUIRE(!h->needs_z || cols.z, "the field converter needs the altitude field z");
+        FB_REQUIRE(!h->needs_zs || cols.zs, "this converter and target need the surface altitude zs");
+    }
     return use_device(h->device);
 }
 
+fb200_vcolumns ps_only(const float* ps)
+{
+    fb200_vcolumns cols = {};
+    cols.ps = ps;
+    return cols;
+}
+
 // typed: data2InterpolationArray (any CDM type, fill -> NaN) before and interpolationArray2Data (NaN -> fill, cast) after, both as
-// separate passes; untyped: float in, float out
-int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* d_in, const float* d_ps, size_t nxy, size_t nt, double bad,
-                   int out_type, void* d_out, cudaStream_t st)
+// separate passes; untyped: float in, float out.  cols: device pointers.
+int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* d_in, const fb200_vcolumns& cols, size_t nxy, size_t nt,
+                   double bad, int out_type, void* d_out, cudaStream_t st)
 {
     if (nxy == 0 || nt == 0)
         return FB_OK;
@@ -2168,32 +2281,63 @@ int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* 
     float* fout = static_cast<float*>(d_out);
     if (typed && out_type != FB_T_FLOAT && tmp.get(&fout, out_n) != FB_OK)
         return FB_ERROR;
-    if (launch_vertical(h->vt, fin, h->has_ps ? d_ps : nullptr, (long long)nxy, (long long)nt, fout, st) != FB_OK)
+    const float* ps = h->has_ps ? cols.ps : nullptr;
+    const int rc = h->vt.converter == FB_VZ_NONE
+                       ? launch_vertical(h->vt, fin, ps, (long long)nxy, (long long)nt, fout, st)
+                       : launch_vertical_height(h->vt, fin, ps, h->needs_t ? cols.t : nullptr, h->needs_t ? cols.q : nullptr,
+                                                h->needs_z ? cols.z : nullptr, h->needs_zs ? cols.zs : nullptr, (long long)nxy, (long long)nt, fout, st);
+    if (rc != FB_OK)
         return FB_ERROR;
     if (typed)
         return launch_from_float(fout, (long long)out_n, out_type, bad, d_out, st);
     return FB_OK;
 }
 
-// host arrays: time steps are the units of the staging pipeline of the horizontal calls
-int vinterp_host(const fb200_vinterp* h, bool typed, int in_type, const void* in, const float* ps, size_t nxy, size_t nt, double bad, int out_type,
-                 void* out)
+// host arrays: time steps are the units of the staging pipeline of the horizontal calls; the field and up to three per-step inputs
+// (ps, t, q or z) go through it, zs (no time axis) is uploaded once per call
+int vinterp_host(const fb200_vinterp* h, bool typed, int in_type, const void* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, double bad,
+                 int out_type, void* out)
 {
     if (nxy == 0 || nt == 0)
         return FB_OK;
+    const size_t level = nxy * sizeof(float), column = level * (size_t)h->vt.nk;
     HostArrays arrays;
     arrays.device = h->device;
     arrays.in[0] = in;
     arrays.in_unit[0] = nxy * (size_t)h->vt.nk * type_size(in_type);
-    if (h->has_ps) {
-        arrays.in[1] = ps;
-        arrays.in_unit[1] = nxy * sizeof(float);
+    const float* steps[4] = {h->has_ps ? cols.ps : nullptr, h->needs_t ? cols.t : nullptr, h->needs_t ? cols.q : nullptr,
+                             h->needs_z ? cols.z : nullptr};
+    const size_t unit[4] = {level, column, column, column};
+    int slot[4] = {-1, -1, -1, -1};
+    for (int i = 0, n = 1; i < 4; ++i) {
+        if (!steps[i])
+            continue;
+        FB_REQUIRE(n < kHostIn, "too many per-step inputs");
+        slot[i] = n;
+        arrays.in[n] = steps[i];
+        arrays.in_unit[n++] = unit[i];
     }
     arrays.out[0] = out;
     arrays.out_unit[0] = nxy * (size_t)h->vt.np * type_size(out_type);
-    return stage_host(arrays, nt, [&](const void* const* d_in, size_t n, void* const* d_out, cudaStream_t st) {
-        return vinterp_device(h, typed, in_type, d_in[0], static_cast<const float*>(d_in[1]), nxy, n, bad, out_type, d_out[0], st);
+    cudaStream_t st = cudaStreamPerThread;
+    Scratch tmp(st); // freed after stage_host has returned, when every kernel that read it is complete
+    float* d_zs = nullptr;
+    if (h->needs_zs) {
+        if (tmp.upload(&d_zs, cols.zs, nxy) != FB_OK)
+            return FB_ERROR;
+        FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    }
+    return stage_host(arrays, nt, [&](const void* const* d_in, size_t n, void* const* d_out, cudaStream_t s) {
+        auto arg = [&](int i) { return slot[i] < 0 ? nullptr : static_cast<const float*>(d_in[slot[i]]); };
+        fb200_vcolumns dc = {arg(0), arg(1), arg(2), arg(3), d_zs};
+        return vinterp_device(h, typed, in_type, d_in[0], dc, nxy, n, bad, out_type, d_out[0], s);
     });
+}
+
+const fb200_vcolumns& or_none(const fb200_vcolumns* cols)
+{
+    static const fb200_vcolumns none = {};
+    return cols ? *cols : none;
 }
 
 } // namespace
@@ -2212,6 +2356,16 @@ int fb200_vinterp_create_sigma(int method, const double* sigma, int nk, double p
     return vinterp_create(method, sigma, nullptr, nk, true, ptop, ps_scale, levels, np, extrapolate, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
 }
 
+int fb200_vinterp_create_height(int method, int converter, int target, int vcoord, const double* a, const double* b, int nk, double ptop,
+                                double ps_scale, double z_scale, double zs_scale, const double* levels, int np, int extrapolate,
+                                fb200_vinterp** handle)
+{
+    return vinterp_create_height(method, converter, target, vcoord, a, b, nk, ptop, ps_scale, z_scale, zs_scale, levels, np, extrapolate, handle) ==
+                   FB_OK
+               ? MIFI_OK
+               : MIFI_ERROR;
+}
+
 void fb200_vinterp_destroy(fb200_vinterp* h)
 {
     delete h;
@@ -2219,33 +2373,62 @@ void fb200_vinterp_destroy(fb200_vinterp* h)
 
 int fb200_vinterp_interpolate_values(const fb200_vinterp* h, const float* in, const float* ps, size_t nxy, size_t nt, float* out)
 {
-    if (check_vinterp_call(h, in, ps, nxy, nt, out) != FB_OK)
-        return MIFI_ERROR;
-    return vinterp_host(h, false, FB_T_FLOAT, in, ps, nxy, nt, 0.0, FB_T_FLOAT, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+    const fb200_vcolumns cols = ps_only(ps);
+    return fb200_vinterp_interpolate_values_columns(h, in, &cols, nxy, nt, out);
 }
 
 int fb200_vinterp_interpolate_values_device(const fb200_vinterp* h, const float* d_in, const float* d_ps, size_t nxy, size_t nt, float* d_out,
                                             void* stream)
 {
-    if (check_vinterp_call(h, d_in, d_ps, nxy, nt, d_out) != FB_OK)
-        return MIFI_ERROR;
-    return vinterp_device(h, false, FB_T_FLOAT, d_in, d_ps, nxy, nt, 0.0, FB_T_FLOAT, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
+    const fb200_vcolumns cols = ps_only(d_ps);
+    return fb200_vinterp_interpolate_values_columns_device(h, d_in, &cols, nxy, nt, d_out, stream);
 }
 
 int fb200_vinterp_get_data_slice(const fb200_vinterp* h, int inType, const void* in, const float* ps, size_t nxy, size_t nt, double badValue,
                                  int outType, void* out)
 {
-    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, in, ps, nxy, nt, out) != FB_OK)
-        return MIFI_ERROR;
-    return vinterp_host(h, true, inType, in, ps, nxy, nt, badValue, outType, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+    const fb200_vcolumns cols = ps_only(ps);
+    return fb200_vinterp_get_data_slice_columns(h, inType, in, &cols, nxy, nt, badValue, outType, out);
 }
 
 int fb200_vinterp_get_data_slice_device(const fb200_vinterp* h, int inType, const void* d_in, const float* d_ps, size_t nxy, size_t nt,
                                         double badValue, int outType, void* d_out, void* stream)
 {
-    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, d_in, d_ps, nxy, nt, d_out) != FB_OK)
+    const fb200_vcolumns cols = ps_only(d_ps);
+    return fb200_vinterp_get_data_slice_columns_device(h, inType, d_in, &cols, nxy, nt, badValue, outType, d_out, stream);
+}
+
+int fb200_vinterp_interpolate_values_columns(const fb200_vinterp* h, const float* in, const fb200_vcolumns* cols, size_t nxy, size_t nt, float* out)
+{
+    if (check_vinterp_call(h, in, or_none(cols), nxy, nt, out) != FB_OK)
         return MIFI_ERROR;
-    return vinterp_device(h, true, inType, d_in, d_ps, nxy, nt, badValue, outType, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
+    return vinterp_host(h, false, FB_T_FLOAT, in, or_none(cols), nxy, nt, 0.0, FB_T_FLOAT, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_interpolate_values_columns_device(const fb200_vinterp* h, const float* d_in, const fb200_vcolumns* d_cols, size_t nxy, size_t nt,
+                                                    float* d_out, void* stream)
+{
+    if (check_vinterp_call(h, d_in, or_none(d_cols), nxy, nt, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_device(h, false, FB_T_FLOAT, d_in, or_none(d_cols), nxy, nt, 0.0, FB_T_FLOAT, d_out, as_stream(stream)) == FB_OK ? MIFI_OK
+                                                                                                                                     : MIFI_ERROR;
+}
+
+int fb200_vinterp_get_data_slice_columns(const fb200_vinterp* h, int inType, const void* in, const fb200_vcolumns* cols, size_t nxy, size_t nt,
+                                         double badValue, int outType, void* out)
+{
+    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, in, or_none(cols), nxy, nt, out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_host(h, true, inType, in, or_none(cols), nxy, nt, badValue, outType, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vinterp_get_data_slice_columns_device(const fb200_vinterp* h, int inType, const void* d_in, const fb200_vcolumns* d_cols, size_t nxy,
+                                                size_t nt, double badValue, int outType, void* d_out, void* stream)
+{
+    if (check_slice_types(inType, outType) != FB_OK || check_vinterp_call(h, d_in, or_none(d_cols), nxy, nt, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return vinterp_device(h, true, inType, d_in, or_none(d_cols), nxy, nt, badValue, outType, d_out, as_stream(stream)) == FB_OK ? MIFI_OK
+                                                                                                                                  : MIFI_ERROR;
 }
 
 // ---------------------------------------------------------------------------------------- mifi_* drop-ins

@@ -11,6 +11,11 @@
 //
 // Arithmetic (DESIGN.md section 2): fp64, every product through __dmul_rn so that nothing is contracted into an FMA, and
 // ln() by vlog() below, the same sequence of IEEE operations as the oracle's orc_vlog (tests/vertical_oracle.c) -- results are bit-identical.
+//
+// k_vertical_height is the height branch (targets in metres above sea level or above ground): the same walk, in the column's
+// altitude z_k, which it computes level by level as the walk goes up from the surface (standard atmosphere of p_k, the
+// hypsometric sum over T and q, or a z field) and never stores.  The walk ends at the bracket of the highest target, so a column
+// is read only up to there (DESIGN.md sections 2 and 4).
 #include "kernels.h"
 
 namespace fb {
@@ -167,6 +172,175 @@ __global__ void __launch_bounds__(kThreads, 4) k_vertical(const float* __restric
     }
 }
 
+// exp(x): fdlibm's __ieee754_exp (e_exp.c) -- x = k ln2 + r, |r| <= ln2 / 2, and a degree-5 rational approximation in r; < 1 ulp.
+// Only +, -, *, / and bit operations, as vlog; the oracle's orc_vexp (tests/vertical_height_oracle.c) is the same sequence.
+__device__ double vexp(double x)
+{
+    const double twom1000 = 9.33263618503218878990e-302, o_threshold = 7.09782712893383973096e+02,
+                 u_threshold = -7.45133219101941108420e+02, ln2_hi = 6.93147180369123816490e-01, ln2_lo = 1.90821492927058770002e-10,
+                 invln2 = 1.44269504088896338700e+00;
+    const double P1 = 1.66666666666666019037e-01, P2 = -2.77777777770155933842e-03, P3 = 6.61375632143793436117e-05,
+                 P4 = -1.65339022054652515390e-06, P5 = 4.13813679705723846039e-08;
+    const unsigned hw = (unsigned)__double2hiint(x), lx = (unsigned)__double2loint(x);
+    const int xsb = (int)(hw >> 31);
+    const unsigned hx = hw & 0x7fffffffu;
+    if (hx >= 0x40862E42u) { // |x| >= 709.78...
+        if (hx >= 0x7ff00000u) {
+            if (((hx & 0xfffffu) | lx) != 0)
+                return x + x; // NaN
+            return xsb == 0 ? x : 0.0;
+        }
+        if (x > o_threshold)
+            return __longlong_as_double(0x7ff0000000000000ll); // overflow: huge * huge
+        if (x < u_threshold)
+            return 0.0; // underflow: twom1000 * twom1000
+    }
+    double hi = 0.0, lo = 0.0;
+    int k = 0;
+    if (hx > 0x3fd62e42u) {     // |x| > 0.5 ln2
+        if (hx < 0x3FF0A2B2u) { // and |x| < 1.5 ln2
+            hi = xsb ? x + ln2_hi : x - ln2_hi;
+            lo = xsb ? -ln2_lo : ln2_lo;
+            k = 1 - xsb - xsb;
+        } else {
+            k = (int)(__dmul_rn(invln2, x) + (xsb ? -0.5 : 0.5));
+            const double t = (double)k;
+            hi = x - __dmul_rn(t, ln2_hi); // t * ln2_hi is exact here
+            lo = __dmul_rn(t, ln2_lo);
+        }
+        x = hi - lo;
+    } else if (hx < 0x3e300000u) { // |x| < 2^-28
+        return 1.0 + x;
+    }
+    const double t = __dmul_rn(x, x);
+    const double c = x - __dmul_rn(t, P1 + __dmul_rn(t, P2 + __dmul_rn(t, P3 + __dmul_rn(t, P4 + __dmul_rn(t, P5)))));
+    if (k == 0)
+        return 1.0 - (__dmul_rn(x, c) / (c - 2.0) - x);
+    const double y = 1.0 - ((lo - __dmul_rn(x, c) / (2.0 - c)) - hi);
+    if (k >= -1021)
+        return __hiloint2double(__double2hiint(y) + (k << 20), __double2loint(y)); // add k to y's exponent
+    return __dmul_rn(__hiloint2double(__double2hiint(y) + ((k + 1000) << 20), __double2loint(y)), twom1000);
+}
+
+// standard-atmosphere altitude of p: the last layer b with p <= p_b; layer constants [h_b | p_b | c_b | e_b] x kStdLayers (api.cu)
+__device__ __forceinline__ double zstd(const double* __restrict__ L, double p)
+{
+    int b = 0;
+#pragma unroll
+    for (int l = 1; l < kStdLayers; ++l)
+        if (p <= L[kStdLayers + l])
+            b = l;
+    const double h = L[b], pb = L[kStdLayers + b], c = L[2 * kStdLayers + b], e = L[3 * kStdLayers + b];
+    if (e != 0.0)
+        return h + __dmul_rn(c, vexp(__dmul_rn(e, vlog(p / pb))) - 1.0);
+    return h + __dmul_rn(c, vlog(pb / p));
+}
+
+// in, t, q, z [nt][nk][nxy]; ps [nt][nxy]; zs [nxy]; out [nt][np][nxy]; blockIdx.y = time step.  Inputs the converter does not use
+// are null (q: optional for the hypsometric converter).
+// tab: a[nk] | b[nk] | standard-atmosphere layers[4 * kStdLayers] | sorted target levels[np] | output row of each sorted target[np]
+template <int CONV, int M>
+__global__ void __launch_bounds__(kThreads, 3)
+    k_vertical_height(const float* __restrict__ in, const float* __restrict__ ps, const float* __restrict__ tt, const float* __restrict__ qq,
+                      const float* __restrict__ zf, const float* __restrict__ zs, float* __restrict__ out, const double* __restrict__ tab, int nk,
+                      int np, int extrapolate, int target, double ps_scale, double shift, double z_scale, double zs_scale, double H, double cq,
+                      long long nxy, long long t0)
+{
+    extern __shared__ double s_tab[];
+    const int ntab = 2 * nk + 4 * kStdLayers + 2 * np;
+    for (int i = threadIdx.x; i < ntab; i += blockDim.x)
+        s_tab[i] = tab[i];
+    __syncthreads();
+    const double* s_a = s_tab;
+    const double* s_b = s_tab + nk;
+    const double* s_std = s_tab + 2 * nk;
+    const double* s_lev = s_std + 4 * kStdLayers;
+    const double* s_row = s_lev + np;
+
+    const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (c >= nxy)
+        return;
+    const long long t = t0 + blockIdx.y;
+    const long long base = t * nk * nxy + c;
+    const float* col = in + base;
+    float* ocol = out + t * np * nxy + c;
+    const double psd = ps ? __dmul_rn((double)__ldg(ps + t * nxy + c), ps_scale) : 0.0;
+    const double qs = psd - shift;
+    const double zsd = zs ? __dmul_rn((double)__ldg(zs + c), zs_scale) : 0.0;
+    // the hypsometric sum starts at the surface altitude for altitude targets, at 0 for heights; the other converters subtract
+    // z_s from z for heights
+    const double zsub = (target == FB_VZ_HEIGHT && CONV != FB_VZ_HYPSOMETRIC) ? zsd : 0.0;
+    auto pres = [&](int k) { return s_a[k] + __dmul_rn(s_b[k], qs); };
+    auto zfield = [&](int k) { return __dmul_rn(z_scale, (double)__ldg(zf + base + (long long)k * nxy)); };
+
+    bool up, flat; // up: level 0 is the surface end
+    if (CONV == FB_VZ_FIELD) {
+        const double z0 = zfield(0), zl = zfield(nk - 1);
+        up = z0 < zl;
+        flat = !(z0 < zl) && !(z0 > zl);
+    } else {
+        const double p0 = pres(0), pl = pres(nk - 1);
+        up = p0 > pl;
+        flat = !(p0 < pl) && !(p0 > pl);
+    }
+    // The walk: level m counted from the surface; zj = the coordinate of level j, zjm = that of level j - 1.  The hypsometric
+    // converter carries Tv and p of level j in registers and returns the increment of its sum over the layer below level m.
+    double tvj = 0.0, pj = 0.0;
+    auto level_z = [&](int m) -> double {
+        const int k = up ? m : nk - 1 - m;
+        if (CONV == FB_VZ_FIELD)
+            return zfield(k) - zsub;
+        const double p = pres(k);
+        if (CONV == FB_VZ_STANDARD)
+            return zstd(s_std, p) - zsub;
+        const double T = (double)__ldg(tt + base + (long long)k * nxy);
+        const double tv = qq ? __dmul_rn(T, 1.0 + __dmul_rn(cq, (double)__ldg(qq + base + (long long)k * nxy))) : T;
+        const double hterm = m == 0 ? __dmul_rn(H, tv) : __dmul_rn(H, __dmul_rn(0.5, tv + tvj));
+        const double dz = __dmul_rn(hterm, vlog((m == 0 ? psd : pj) / p));
+        tvj = tv;
+        pj = p;
+        return dz;
+    };
+    double z0 = 0.0, zjm = 0.0, zj = 0.0;
+    if (!flat) {
+        z0 = CONV == FB_VZ_HYPSOMETRIC ? (target == FB_VZ_ALTITUDE ? zsd : 0.0) + level_z(0) : level_z(0);
+        zj = CONV == FB_VZ_HYPSOMETRIC ? z0 + level_z(1) : level_z(1);
+        zjm = z0;
+        flat = isnan(z0);
+    }
+    int j = 1, kc = -2;
+    float va = 0.f, vb = 0.f;
+    for (int i = 0; i < np; ++i) {
+        const double Z = s_lev[i];
+        float r = undef_f();
+        if (!flat) {
+            while (j < nk - 1 && zj < Z) { // NaN stops the walk: every target above it gets NaN
+                zjm = zj;
+                ++j;
+                zj = CONV == FB_VZ_HYPSOMETRIC ? zjm + level_z(j) : level_z(j);
+            }
+            if (extrapolate || (Z >= z0 && !(j == nk - 1 && zj < Z))) {
+                const int k = j - 1;
+                const int ka = up ? k : nk - 1 - k, kb = up ? k + 1 : nk - 2 - k;
+                if (k != kc) {
+                    va = k == kc + 1 ? vb : __ldg(col + (long long)ka * nxy); // the lower level of this bracket is the upper one of the last
+                    vb = __ldg(col + (long long)kb * nxy);
+                    kc = k;
+                }
+                if (isnan(zjm) || isnan(zj)) {
+                    r = undef_f();
+                } else if (M == FB_VINT_NN) {
+                    r = fabs(Z - zj) < fabs(Z - zjm) ? vb : va;
+                } else {
+                    const double w = zjm == zj ? 0.0 : (Z - zjm) / (zj - zjm);
+                    r = (float)((double)va + __dmul_rn(w, (double)vb - (double)va));
+                }
+            }
+        }
+        __stcs(ocol + (long long)s_row[i] * nxy, r);
+    }
+}
+
 } // namespace
 
 int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st)
@@ -199,6 +373,40 @@ int launch_vertical(const VertTable& vt, const float* d_in, const float* d_ps, l
 #undef FB_CASE
         default:
             FB_REQUIRE(false, "unknown vertical interpolation method " + std::to_string(vt.method));
+        }
+        count_launch();
+        FB_CUDA_CHECK(cudaGetLastError());
+    }
+    return FB_OK;
+}
+
+int launch_vertical_height(const VertTable& vt, const float* d_in, const float* d_ps, const float* d_t, const float* d_q, const float* d_z,
+                           const float* d_zs, long long nxy, long long nt, float* d_out, cudaStream_t st)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    const size_t smem = sizeof(double) * (size_t)(2 * vt.nk + 4 * kStdLayers + 2 * vt.np);
+    const long long bx = (nxy + kThreads - 1) / kThreads;
+    FB_REQUIRE(bx < 2147483647LL, "too many columns for one call");
+    const int key = vt.converter * 8 + vt.method;
+    for (long long t0 = 0; t0 < nt; t0 += 65535) {
+        const dim3 grid((unsigned)bx, (unsigned)std::min<long long>(nt - t0, 65535));
+        switch (key) {
+#define FB_CASE(C, M)                                                                                                                      \
+    case C * 8 + M:                                                                                                                        \
+        k_vertical_height<C, M><<<grid, kThreads, smem, st>>>(d_in, d_ps, d_t, d_q, d_z, d_zs, d_out,                 vt.d_tab, vt.nk, vt.np, \
+                                                              vt.extrapolate ? 1 : 0, vt.target, vt.ps_scale, vt.shift, vt.z_scale,        \
+                                                              vt.zs_scale, vt.H, vt.cq, nxy, t0);                                          \
+        break;
+            FB_CASE(FB_VZ_STANDARD, FB_VINT_LIN)
+            FB_CASE(FB_VZ_STANDARD, FB_VINT_NN)
+            FB_CASE(FB_VZ_HYPSOMETRIC, FB_VINT_LIN)
+            FB_CASE(FB_VZ_HYPSOMETRIC, FB_VINT_NN)
+            FB_CASE(FB_VZ_FIELD, FB_VINT_LIN)
+            FB_CASE(FB_VZ_FIELD, FB_VINT_NN)
+#undef FB_CASE
+        default:
+            FB_REQUIRE(false, "unknown height converter / method " + std::to_string(vt.converter) + " / " + std::to_string(vt.method));
         }
         count_launch();
         FB_CUDA_CHECK(cudaGetLastError());

@@ -1,5 +1,5 @@
-"""Host-side mirror of the pressure branch of the reference's CDMVerticalInterpolator
-(``--verticalInterpolate.type=pressure --verticalInterpolate.method=... --verticalInterpolate.level1=...``).
+"""Host-side mirror of the pressure and height branches of the reference's CDMVerticalInterpolator
+(``--verticalInterpolate.type=pressure|height|altitude --verticalInterpolate.method=... --verticalInterpolate.level1=...``).
 
 The source vertical coordinate is given by its CF standard name and formula terms, as the reference reads them from the CDM:
 
@@ -8,8 +8,9 @@ The source vertical coordinate is given by its CF standard name and formula term
 * ``atmosphere_sigma_coordinate``: terms ``{"sigma": sigma, "ptop": ptop}``.
 
 The surface pressure ``ps`` is not a term here: it is a field, passed with every slice.  All pressures are in the unit of the
-target levels (hPa, as the reference's level1 option); ``ps_scale`` converts the ``ps`` field to it (0.01 for Pa).  The
-arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md section 2 states it).
+target levels (hPa, as the reference's level1 option); ``ps_scale`` converts the ``ps`` field to it (0.01 for Pa).  Height and
+altitude levels are in metres (:class:`HeightInterpolator`).  The arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md
+section 2 states it).
 """
 from __future__ import annotations
 
@@ -27,6 +28,12 @@ METHODS = {"linear": 0, "log": 1, "loglog": 2, "nearestneighbor": 3}
 PRESSURE = "air_pressure"
 HYBRID = "atmosphere_hybrid_sigma_pressure_coordinate"
 SIGMA = "atmosphere_sigma_coordinate"
+VCOORD_PRESSURE, VCOORD_HYBRID, VCOORD_SIGMA = 0, 1, 2  # FB200_VCOORD_*
+
+#: --verticalInterpolate.type values of the height branch -> FB200_VZ_ALTITUDE / _HEIGHT
+TARGETS = {"altitude": 0, "height": 1}
+#: the ways to the altitude of every source level -> FB200_VZ_*
+CONVERTERS = {"standard": 0, "hypsometric": 1, "field": 2}
 
 
 def vertical_method(name: str) -> int:
@@ -37,42 +44,34 @@ def vertical_method(name: str) -> int:
         raise FimexB200Error(f"unknown vertical interpolation method: '{name}' (one of {', '.join(METHODS)})") from None
 
 
-class VerticalInterpolator:
-    """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on the target pressure levels."""
-
-    def __init__(self, standard_name: str, terms: dict, method: str, levels, ps_scale: float = 1.0, extrapolate: bool = True):
-        self.method = vertical_method(method)
-        self.levels = f64(levels).ravel()
-        self._h = C.c_void_p()
-        lib = load()
-        t = {k: v for k, v in terms.items() if k != "ps"}
-        if standard_name == PRESSURE:
-            p = f64(t["p"]).ravel()
-            self.nk, self.needs_ps = p.size, False
-            rc = lib.fb200_vinterp_create_hybrid(self.method, ptr(p), None, p.size, float(ps_scale), ptr(self.levels), self.levels.size,
-                                                 int(bool(extrapolate)), C.byref(self._h))
-        elif standard_name == HYBRID:
-            if "ap" in t:
-                ap = f64(t["ap"]).ravel()
-            elif "a" in t and "p0" in t:
-                ap = f64(t["a"]).ravel() * float(np.asarray(t["p0"], dtype=np.float64).reshape(-1)[0])  # ap_k = a_k * p0, fp64
-            else:
-                raise FimexB200Error(f"{HYBRID} needs the terms ap, b or a, p0, b; got {sorted(terms)}")
-            b = f64(t["b"]).ravel()
-            if b.size != ap.size:
-                raise FimexB200Error(f"{HYBRID}: {ap.size} values of ap but {b.size} of b")
-            self.nk, self.needs_ps = ap.size, True
-            rc = lib.fb200_vinterp_create_hybrid(self.method, ptr(ap), ptr(b), ap.size, float(ps_scale), ptr(self.levels), self.levels.size,
-                                                 int(bool(extrapolate)), C.byref(self._h))
-        elif standard_name == SIGMA:
-            sigma = f64(t["sigma"]).ravel()
-            ptop = float(np.asarray(t["ptop"], dtype=np.float64).reshape(-1)[0])
-            self.nk, self.needs_ps = sigma.size, True
-            rc = lib.fb200_vinterp_create_sigma(self.method, ptr(sigma), sigma.size, ptop, float(ps_scale), ptr(self.levels), self.levels.size,
-                                                int(bool(extrapolate)), C.byref(self._h))
+def _source_levels(standard_name: str, terms: dict):
+    """(vcoord, a, b, ptop, nk) of the source vertical coordinate: pressure levels a = p; hybrid a = ap, b; sigma b = sigma, ptop"""
+    t = {k: v for k, v in terms.items() if k != "ps"}
+    if standard_name == PRESSURE:
+        p = f64(t["p"]).ravel()
+        return VCOORD_PRESSURE, p, None, 0.0, p.size
+    if standard_name == HYBRID:
+        if "ap" in t:
+            ap = f64(t["ap"]).ravel()
+        elif "a" in t and "p0" in t:
+            ap = f64(t["a"]).ravel() * float(np.asarray(t["p0"], dtype=np.float64).reshape(-1)[0])  # ap_k = a_k * p0, fp64
         else:
-            raise FimexB200Error(f"vertical coordinate '{standard_name}' is not supported (one of {PRESSURE}, {HYBRID}, {SIGMA})")
-        check(rc, "VerticalInterpolator")
+            raise FimexB200Error(f"{HYBRID} needs the terms ap, b or a, p0, b; got {sorted(terms)}")
+        b = f64(t["b"]).ravel()
+        if b.size != ap.size:
+            raise FimexB200Error(f"{HYBRID}: {ap.size} values of ap but {b.size} of b")
+        return VCOORD_HYBRID, ap, b, 0.0, ap.size
+    if standard_name == SIGMA:
+        sigma = f64(t["sigma"]).ravel()
+        return VCOORD_SIGMA, None, sigma, float(np.asarray(t["ptop"], dtype=np.float64).reshape(-1)[0]), sigma.size
+    raise FimexB200Error(f"vertical coordinate '{standard_name}' is not supported (one of {PRESSURE}, {HYBRID}, {SIGMA})")
+
+
+class _VerticalHandle:
+    """Lifetime of an fb200_vinterp handle and the shape checks of its calls."""
+
+    nk = 0
+    needs_ps = False
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
@@ -93,6 +92,25 @@ class VerticalInterpolator:
         if self.needs_ps and (ps is None or int(np.prod(ps.shape, dtype=np.int64)) != nt * nxy):
             raise FimexB200Error(f"ps must hold nt * nxy = {nt * nxy} values")
         return nt, nxy, (nt, self.levels.size) + tuple(field.shape[2:])
+
+
+class VerticalInterpolator(_VerticalHandle):
+    """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on the target pressure levels."""
+
+    def __init__(self, standard_name: str, terms: dict, method: str, levels, ps_scale: float = 1.0, extrapolate: bool = True):
+        self.method = vertical_method(method)
+        self.levels = f64(levels).ravel()
+        self._h = C.c_void_p()
+        lib = load()
+        vcoord, a, b, ptop, self.nk = _source_levels(standard_name, terms)
+        self.needs_ps = vcoord != VCOORD_PRESSURE
+        if vcoord == VCOORD_SIGMA:
+            rc = lib.fb200_vinterp_create_sigma(self.method, ptr(b), self.nk, ptop, float(ps_scale), ptr(self.levels), self.levels.size,
+                                                int(bool(extrapolate)), C.byref(self._h))
+        else:
+            rc = lib.fb200_vinterp_create_hybrid(self.method, ptr(a), ptr(b), self.nk, float(ps_scale), ptr(self.levels), self.levels.size,
+                                                 int(bool(extrapolate)), C.byref(self._h))
+        check(rc, "VerticalInterpolator")
 
     def interpolateValues(self, field, ps=None, stream=None):
         """float32 [nt][nk][...] with NaN for undefined values -> float32 [nt][np][...] (numpy or CUDA tensors)"""
@@ -143,4 +161,123 @@ class VerticalInterpolator:
         out = np.empty(shape, dtype=odt)
         check(lib.fb200_vinterp_get_data_slice(self._h, int(capi.cdm_type(a.dtype)), ptr(a), ptr(p), nxy, nt, bad, int(capi.cdm_type(odt)),
                                                ptr(out)), "getDataSlice")
+        return out
+
+
+class _Columns(C.Structure):
+    """fb200_vcolumns"""
+    _fields_ = [("ps", C.c_void_p), ("t", C.c_void_p), ("q", C.c_void_p), ("z", C.c_void_p), ("zs", C.c_void_p)]
+
+
+class HeightInterpolator(_VerticalHandle):
+    """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on target levels in metres: above the
+    ground (``type="height"``) or above sea level (``type="altitude"``).  The altitude of every source level comes from
+    ``converter``:
+
+    * ``"hypsometric"``: integrated upward from the surface over the air temperature ``t`` [K] and, when given, the specific
+      humidity ``q`` [kg/kg]; hybrid or sigma source levels only;
+    * ``"standard"``: the standard-atmosphere altitude of each level's pressure [hPa after ``ps_scale``];
+    * ``"field"``: ``z_scale * z`` for a per-level field ``z`` (geopotential: ``z_scale = 1 / 9.80665``); the terms only give nk.
+
+    ``zs`` [...] is the surface altitude (times ``zs_scale``; surface geopotential: ``1 / 9.80665``): height targets of the standard
+    and field converters and altitude targets of the hypsometric one need it.  ``ps`` [nt][...], ``t``, ``q``, ``z`` [nt][nk][...]
+    are float32.  Methods: ``linear`` and ``nearestneighbor`` (``log`` and ``loglog`` are defined on ln p)."""
+
+    def __init__(self, standard_name: str, terms: dict, method: str, levels, type: str = "height", converter: str = "hypsometric",
+                 ps_scale: float = 1.0, z_scale: float = 1.0, zs_scale: float = 1.0, extrapolate: bool = True):
+        self.method = vertical_method(method)
+        if self.method not in (METHODS["linear"], METHODS["nearestneighbor"]):
+            raise FimexB200Error(f"height levels take the methods linear and nearestneighbor only (log and loglog are defined on ln p), "
+                                 f"got '{method}'")
+        if type not in TARGETS:
+            raise FimexB200Error(f"unknown height target type: '{type}' (one of {', '.join(TARGETS)})")
+        if converter not in CONVERTERS:
+            raise FimexB200Error(f"unknown height converter: '{converter}' (one of {', '.join(CONVERTERS)})")
+        self.levels = f64(levels).ravel()
+        self._h = C.c_void_p()
+        vcoord, a, b, ptop, self.nk = _source_levels(standard_name, terms)
+        if converter == "hypsometric" and vcoord == VCOORD_PRESSURE:
+            raise FimexB200Error("the hypsometric converter needs a surface pressure: hybrid or sigma source levels, not pressure levels")
+        self.needs_ps = converter == "hypsometric" or (converter == "standard" and vcoord != VCOORD_PRESSURE)
+        self.needs_t = converter == "hypsometric"
+        self.needs_z = converter == "field"
+        self.needs_zs = (type == "height") != (converter == "hypsometric")
+        lib = load()
+        rc = lib.fb200_vinterp_create_height(self.method, CONVERTERS[converter], TARGETS[type], vcoord, ptr(a), ptr(b), self.nk, ptop,
+                                             float(ps_scale), float(z_scale), float(zs_scale), ptr(self.levels), self.levels.size,
+                                             int(bool(extrapolate)), C.byref(self._h))
+        check(rc, "HeightInterpolator")
+
+    def _columns(self, nt, nxy, device, ps, t, q, z, zs):
+        """the fb200_vcolumns of a call, and the arrays it points into (kept alive by the caller)"""
+        level, column = nt * nxy, nt * self.nk * nxy
+        given = {"ps": (ps, self.needs_ps, level, "the surface pressure ps"),
+                 "t": (t, self.needs_t, column, "the air temperature t"),
+                 "q": (q, self.needs_t, column, "the specific humidity q"),
+                 "z": (z, self.needs_z, column, "the altitude field z"),
+                 "zs": (zs, self.needs_zs, nxy, "the surface altitude zs")}
+        cols, keep = _Columns(), []
+        for name, (a, used, n, what) in given.items():
+            if a is None or not used:
+                if used and name != "q":
+                    raise FimexB200Error(f"this converter and target need {what}")
+                continue
+            if device:
+                import torch
+                if not _is_torch(a) or not a.is_cuda or a.dtype != torch.float32:
+                    raise FimexB200Error(f"{name} must be a float32 CUDA tensor on the device path")
+                a = a.contiguous()
+            else:
+                a = capi.f32(a)
+            if int(np.prod(a.shape, dtype=np.int64)) != n:
+                raise FimexB200Error(f"{name} must hold {n} values, got shape {tuple(a.shape)}")
+            keep.append(a)
+            setattr(cols, name, ptr(a).value)
+        return cols, keep
+
+    def interpolateValues(self, field, ps=None, t=None, q=None, z=None, zs=None, stream=None):
+        """float32 [nt][nk][...] with NaN for undefined values -> float32 [nt][np][...] (numpy or CUDA tensors)"""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
+            nt, nxy, shape = self._shape(field, ps)
+            cols, keep = self._columns(nt, nxy, True, ps, t, q, z, zs)
+            out = torch.empty(shape, dtype=torch.float32, device=field.device)
+            check(lib.fb200_vinterp_interpolate_values_columns_device(self._h, ptr(field), C.byref(cols), nxy, nt, ptr(out), _stream_ptr(stream)),
+                  "interpolateValues")
+            return out
+        a = capi.f32(field)
+        nt, nxy, shape = self._shape(a, ps)
+        cols, keep = self._columns(nt, nxy, False, ps, t, q, z, zs)
+        out = np.empty(shape, dtype=np.float32)
+        check(lib.fb200_vinterp_interpolate_values_columns(self._h, ptr(a), C.byref(cols), nxy, nt, ptr(out)), "interpolateValues")
+        return out
+
+    def getDataSlice(self, field, ps=None, t=None, q=None, z=None, zs=None, bad_value=None, out_dtype=None, stream=None):
+        """The per-slice body of the vertical getDataSlice: `field` [nt][nk][...] of any CDM numeric type (numpy array, or CUDA tensor
+        for the device-resident path), fill -> NaN, interpolate, NaN -> fill and cast to `out_dtype` (default: the input's type).
+        `bad_value` = CDM::getFillValue of the variable (default: the type's default fill value)."""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous CUDA tensor")
+            odt = out_dtype if out_dtype is not None else field.dtype
+            bad = capi.default_fill_value(field.dtype) if bad_value is None else float(bad_value)
+            nt, nxy, shape = self._shape(field, ps)
+            cols, keep = self._columns(nt, nxy, True, ps, t, q, z, zs)
+            out = torch.empty(shape, dtype=odt, device=field.device)
+            check(lib.fb200_vinterp_get_data_slice_columns_device(self._h, int(capi.cdm_type(field.dtype)), ptr(field), C.byref(cols), nxy, nt,
+                                                                  bad, int(capi.cdm_type(odt)), ptr(out), _stream_ptr(stream)), "getDataSlice")
+            return out
+        a = np.ascontiguousarray(field)
+        odt = np.dtype(out_dtype) if out_dtype is not None else a.dtype
+        bad = capi.default_fill_value(a.dtype) if bad_value is None else float(bad_value)
+        nt, nxy, shape = self._shape(a, ps)
+        cols, keep = self._columns(nt, nxy, False, ps, t, q, z, zs)
+        out = np.empty(shape, dtype=odt)
+        check(lib.fb200_vinterp_get_data_slice_columns(self._h, int(capi.cdm_type(a.dtype)), ptr(a), C.byref(cols), nxy, nt, bad,
+                                                       int(capi.cdm_type(odt)), ptr(out)), "getDataSlice")
         return out

@@ -324,6 +324,54 @@ int fb200_vinterp_get_data_slice_device(const fb200_vinterp* handle, int inType,
                                         double badValue, int outType, void* d_out, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * (1e) vertical interpolation to height and altitude levels: the height branch of CDMVerticalInterpolator
+ *      (--verticalInterpolate.type=height / altitude; DESIGN.md section 2 states the arithmetic)
+ *
+ * Targets in metres: FB200_VZ_ALTITUDE above sea level, FB200_VZ_HEIGHT above the ground.  The altitude z_k of every source level
+ * comes from a converter:
+ *   FB200_VZ_STANDARD     the standard-atmosphere altitude (US Standard Atmosphere 1976 / ICAO) of the column pressure p_k [hPa];
+ *   FB200_VZ_HYPSOMETRIC  integrated upward from the surface over the air temperature t [K] and, when given, the specific humidity
+ *                         q [kg/kg] (virtual temperature); hybrid or sigma source levels only;
+ *   FB200_VZ_FIELD        z_k = z_scale * z, a per-level field (geopotential: z_scale = 1 / 9.80665; altitude: 1); the formula
+ *                         terms are not used and may be NULL.
+ * vcoord and a, b, ptop, ps_scale give the column pressures as for the pressure handles: FB200_VCOORD_PRESSURE (a = the levels),
+ * _HYBRID (a = ap, b) or _SIGMA (b = sigma, ptop).  The surface altitude is zs * zs_scale (surface geopotential: zs_scale =
+ * 1 / 9.80665); height targets of the standard and field converters and altitude targets of the hypsometric one need it.
+ * method: MIFI_VINT_METHOD_LIN or _NN only (log and loglog are defined on ln p).  Other rules as for the pressure handles.
+ * ---------------------------------------------------------------------------------------------- */
+#define FB200_VCOORD_PRESSURE 0
+#define FB200_VCOORD_HYBRID 1
+#define FB200_VCOORD_SIGMA 2
+#define FB200_VZ_STANDARD 0
+#define FB200_VZ_HYPSOMETRIC 1
+#define FB200_VZ_FIELD 2
+#define FB200_VZ_ALTITUDE 0
+#define FB200_VZ_HEIGHT 1
+/* the per-column inputs of a call, float32, NULL = not given: ps [nt][nxy], t, q, z [nt][nk][nxy], zs [nxy] (no time axis) */
+typedef struct fb200_vcolumns {
+    const float* ps;
+    const float* t;
+    const float* q;
+    const float* z;
+    const float* zs;
+} fb200_vcolumns;
+
+int fb200_vinterp_create_height(int method, int converter, int target, int vcoord, const double* a, const double* b, int nk, double ptop,
+                                double ps_scale, double z_scale, double zs_scale, const double* levels, int np, int extrapolate,
+                                fb200_vinterp** handle);
+/* The calls above with every per-column input: they take pressure handles too (only ps is read).  A height handle on the calls
+ * above, which pass ps alone, fails when it needs t, z or zs.  `cols` holds host pointers, `d_cols` (itself a host struct) device
+ * pointers. */
+int fb200_vinterp_interpolate_values_columns(const fb200_vinterp* handle, const float* in, const fb200_vcolumns* cols, size_t nxy, size_t nt,
+                                             float* out);
+int fb200_vinterp_interpolate_values_columns_device(const fb200_vinterp* handle, const float* d_in, const fb200_vcolumns* d_cols, size_t nxy,
+                                                    size_t nt, float* d_out, void* cuda_stream);
+int fb200_vinterp_get_data_slice_columns(const fb200_vinterp* handle, int inType, const void* in, const fb200_vcolumns* cols, size_t nxy,
+                                         size_t nt, double badValue, int outType, void* out);
+int fb200_vinterp_get_data_slice_columns_device(const fb200_vinterp* handle, int inType, const void* d_in, const fb200_vcolumns* d_cols,
+                                                size_t nxy, size_t nt, double badValue, int outType, void* d_out, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
  * ---------------------------------------------------------------------------------------------- */
 int mifi_string_to_interpolation_method(const char* stringMethod); /* :44 */
