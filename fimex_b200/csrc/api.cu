@@ -2070,15 +2070,18 @@ int fb200_vector_get_slice(const fb200_vector* v, int inType, const void* uIn, c
 } // extern "C"
 
 // ======================================================================================================
-// vertical interpolation to pressure levels (the pressure branch of CDMVerticalInterpolator) and to height and altitude levels
-// (its height branch)
+// vertical interpolation to pressure levels (the pressure branch of CDMVerticalInterpolator), to height and altitude levels
+// (its height branch) and to depth levels (its depth branch)
 // ======================================================================================================
+// Depth handles reuse two slots of fb200_vcolumns: ps carries the sea surface height eta, zs the sea-floor depth.
 struct fb200_vinterp {
     int device = 0;
-    bool has_ps = false;   // the column pressures depend on the surface pressure (hybrid or sigma levels), and the converter uses them
+    bool has_ps = false;   // the column pressures depend on the surface pressure (hybrid or sigma levels), and the converter uses them;
+                           // depth handles of the ocean coordinates: eta is read when given (it is optional: NULL means 0)
     bool needs_t = false;  // height handles: the hypsometric converter integrates the air temperature (and q, when given)
     bool needs_z = false;  // the field converter reads the altitude field z
-    bool needs_zs = false; // the surface altitude: height targets of the standard and field converters, altitude targets of the hypsometric one
+    bool needs_zs = false; // the surface altitude: height targets of the standard and field converters, altitude targets of the hypsometric one;
+                           // depth handles of the ocean coordinates: they need the sea-floor depth
     fb::VertTable vt;
     ~fb200_vinterp()
     {
@@ -2241,15 +2244,65 @@ int vinterp_create_height(int method, int converter, int target, int vcoord, con
     return FB_OK;
 }
 
+// ocean_sigma_coordinate, ocean_s_coordinate_g1 / _g2 or depth levels: x_k = -z_k from the terms s (sigma_k, s_k or the levels), C and
+// depth_c; the table holds s (depth levels, sigma) or dcs_k = depth_c * s_k (g1, g2), and C
+int vinterp_create_depth(int method, int vcoord, const double* s, const double* Ck, int nk, double depth_c, const double* levels, int np, int extrapolate,
+                         fb200_vinterp** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(method == FB_VINT_LIN || method == FB_VINT_NN,
+               "depth levels take the methods linear and nearestneighbor only (log and loglog are defined on ln p), got " + std::to_string(method));
+    FB_REQUIRE(vcoord >= FB_VD_DEPTH && vcoord <= FB_VD_OCEAN_S_G2, "unknown depth source vertical coordinate " + std::to_string(vcoord));
+    const bool g = vcoord == FB_VD_OCEAN_S_G1 || vcoord == FB_VD_OCEAN_S_G2;
+    FB_REQUIRE(nk >= 2 && nk <= kMaxVertLevels, "number of source levels must be in [2, 1024], got " + std::to_string(nk));
+    FB_REQUIRE(np >= 1 && np <= kMaxVertLevels, "number of target levels must be in [1, 1024], got " + std::to_string(np));
+    FB_REQUIRE(levels != nullptr, "null target levels");
+    FB_REQUIRE(all_finite(levels, np), "target levels must be finite");
+    FB_REQUIRE(s != nullptr, vcoord == FB_VD_DEPTH ? "null depth levels" : vcoord == FB_VD_OCEAN_SIGMA ? "null sigma" : "null s");
+    FB_REQUIRE(!g || Ck != nullptr, "null C: ocean_s_coordinate_g1 and _g2 need the stretching function C");
+    FB_REQUIRE(all_finite(s, nk) && (!g || all_finite(Ck, nk)), "vertical coordinate values must be finite");
+    FB_REQUIRE(std::isfinite(depth_c) && depth_c >= 0.0, "depth_c must be finite and >= 0");
+    if (use_device(default_device()) != FB_OK)
+        return FB_ERROR;
+    std::unique_ptr<fb200_vinterp> h(new fb200_vinterp());
+    h->device = default_device();
+    h->has_ps = vcoord != FB_VD_DEPTH;
+    h->needs_zs = vcoord != FB_VD_DEPTH;
+    VertTable& vt = h->vt;
+    vt.method = method;
+    vt.nk = nk;
+    vt.np = np;
+    vt.extrapolate = extrapolate != 0;
+    vt.depth_vcoord = vcoord;
+    vt.depth_c = depth_c;
+    std::vector<double> tab(2 * (size_t)nk + 2 * (size_t)np, 0.0);
+    for (int k = 0; k < nk; ++k) {
+        tab[k] = g ? depth_c * s[k] : s[k];
+        tab[nk + k] = g ? Ck[k] : 0.0;
+    }
+    double* lev = tab.data() + 2 * nk;
+    sort_targets(levels, np, lev, lev + np);
+    cudaStream_t st = cudaStreamPerThread;
+    if (upload_table(vt, tab, st) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    *handle = h.release();
+    return FB_OK;
+}
+
 int check_vinterp_call(const fb200_vinterp* h, const void* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, const void* out)
 {
     FB_REQUIRE(h != nullptr, "null vertical interpolation handle");
     FB_REQUIRE(nxy * nt == 0 || (in && out), "null data pointer");
     if (nxy * nt != 0) {
-        FB_REQUIRE(!h->has_ps || cols.ps, "this vertical coordinate needs the surface pressure ps");
+        const bool depth = h->vt.depth_vcoord != FB_VD_NONE;
+        FB_REQUIRE(!h->has_ps || cols.ps || depth, "this vertical coordinate needs the surface pressure ps"); // eta is optional
         FB_REQUIRE(!h->needs_t || cols.t, "the hypsometric converter needs the air temperature t");
         FB_REQUIRE(!h->needs_z || cols.z, "the field converter needs the altitude field z");
-        FB_REQUIRE(!h->needs_zs || cols.zs, "this converter and target need the surface altitude zs");
+        FB_REQUIRE(!h->needs_zs || cols.zs,
+                   depth ? "ocean s- and sigma coordinates need the sea-floor depth (the zs slot of fb200_vcolumns; the calls without _columns cannot pass it)"
+                         : "this converter and target need the surface altitude zs");
     }
     return use_device(h->device);
 }
@@ -2282,10 +2335,12 @@ int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* 
     if (typed && out_type != FB_T_FLOAT && tmp.get(&fout, out_n) != FB_OK)
         return FB_ERROR;
     const float* ps = h->has_ps ? cols.ps : nullptr;
-    const int rc = h->vt.converter == FB_VZ_NONE
+    const float* zs = h->needs_zs ? cols.zs : nullptr;
+    const int rc = h->vt.depth_vcoord != FB_VD_NONE ? launch_vertical_depth(h->vt, fin, ps, zs, (long long)nxy, (long long)nt, fout, st)
+                   : h->vt.converter == FB_VZ_NONE
                        ? launch_vertical(h->vt, fin, ps, (long long)nxy, (long long)nt, fout, st)
                        : launch_vertical_height(h->vt, fin, ps, h->needs_t ? cols.t : nullptr, h->needs_t ? cols.q : nullptr,
-                                                h->needs_z ? cols.z : nullptr, h->needs_zs ? cols.zs : nullptr, (long long)nxy, (long long)nt, fout, st);
+                                                h->needs_z ? cols.z : nullptr, zs, (long long)nxy, (long long)nt, fout, st);
     if (rc != FB_OK)
         return FB_ERROR;
     if (typed)
@@ -2294,7 +2349,7 @@ int vinterp_device(const fb200_vinterp* h, bool typed, int in_type, const void* 
 }
 
 // host arrays: time steps are the units of the staging pipeline of the horizontal calls; the field and up to three per-step inputs
-// (ps, t, q or z) go through it, zs (no time axis) is uploaded once per call
+// (ps, t, q or z) go through it, zs (no time axis) is uploaded once per call; for depth handles these are eta and the sea-floor depth
 int vinterp_host(const fb200_vinterp* h, bool typed, int in_type, const void* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, double bad,
                  int out_type, void* out)
 {
@@ -2364,6 +2419,12 @@ int fb200_vinterp_create_height(int method, int converter, int target, int vcoor
                    FB_OK
                ? MIFI_OK
                : MIFI_ERROR;
+}
+
+int fb200_vinterp_create_depth(int method, int vcoord, const double* s, const double* C, int nk, double depth_c, const double* levels, int np,
+                               int extrapolate, fb200_vinterp** handle)
+{
+    return vinterp_create_depth(method, vcoord, s, C, nk, depth_c, levels, np, extrapolate, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
 }
 
 void fb200_vinterp_destroy(fb200_vinterp* h)

@@ -136,12 +136,14 @@ int forward_build_plan(const int* d_cell, long long n_in, long long n_cells, For
 void forward_free_plan(ForwardPlan* plan);
 int launch_forward(int method, const ForwardPlan& plan, const float* d_in, float* d_out, long long nz, cudaStream_t st);
 
-// ---- vertical_kernels.cu (vertical interpolation to pressure, height and altitude levels) -------------------------------
+// ---- vertical_kernels.cu (vertical interpolation to pressure, height, altitude and depth levels) ------------------------
 // methods, numbered as the reference's MIFI_VINT_METHOD_* (include/fimex/mifi_constants.h)
 enum { FB_VINT_LIN = 0, FB_VINT_LOG = 1, FB_VINT_LOGLOG = 2, FB_VINT_NN = 3 };
-// height converters (FB_VZ_NONE: a pressure handle) and targets, numbered as FB200_VZ_* (include/fimex_b200.h)
+// height converters (FB_VZ_NONE: a pressure or depth handle) and targets, numbered as FB200_VZ_* (include/fimex_b200.h)
 enum { FB_VZ_NONE = -1, FB_VZ_STANDARD = 0, FB_VZ_HYPSOMETRIC = 1, FB_VZ_FIELD = 2 };
 enum { FB_VZ_ALTITUDE = 0, FB_VZ_HEIGHT = 1 };
+// source coordinates of the depth handles (FB_VD_NONE: a pressure or height handle), numbered as FB200_VCOORD_* (include/fimex_b200.h)
+enum { FB_VD_NONE = -1, FB_VD_DEPTH = 3, FB_VD_OCEAN_SIGMA = 4, FB_VD_OCEAN_S_G1 = 5, FB_VD_OCEAN_S_G2 = 6 };
 constexpr int kStdLayers = 7; // geopotential layers of the US Standard Atmosphere 1976
 struct VertTable {
     int method = 0, nk = 0, np = 0;
@@ -149,10 +151,13 @@ struct VertTable {
     double ps_scale = 1.0, shift = 0.0; // p_k = a_k + b_k * (ps * ps_scale - shift)
     // pressure handles: a[nk] | b[nk] | sorted targets[np] | their coordinates[np] | output row of each[np]
     // height handles:   a[nk] | b[nk] | standard-atmosphere layers h_b, p_b, c_b, e_b [4][kStdLayers] | sorted targets[np] | output row of each[np]
+    // depth handles:    levels, sigma_k or depth_c * s_k [nk] | C_k (0 for depth and sigma) [nk] | sorted targets[np] | output row of each[np]
     double* d_tab = nullptr;
     int converter = FB_VZ_NONE, target = FB_VZ_ALTITUDE;
     double z_scale = 1.0, zs_scale = 1.0; // z = z_scale * Z (field converter); z_s = zs_scale * zs
     double H = 0.0, cq = 0.0;             // R* / (M g0) [m/K]; M / M_w - 1 (virtual temperature)
+    int depth_vcoord = FB_VD_NONE;
+    double depth_c = 0.0; // ocean_s_coordinate_g1 / _g2
 };
 // the coordinate of each target the weights are linear in (p, ln p or ln ln p), computed with the kernel's own ln()
 int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st);
@@ -161,5 +166,8 @@ int launch_vertical(const VertTable& vt, const float* d_in, const float* d_ps, l
 // height handles: in, t, q, z [nt][nk][nxy], ps [nt][nxy], zs [nxy] (null where the converter and target do not use them), out [nt][np][nxy]
 int launch_vertical_height(const VertTable& vt, const float* d_in, const float* d_ps, const float* d_t, const float* d_q, const float* d_z,
                            const float* d_zs, long long nxy, long long nt, float* d_out, cudaStream_t st);
+// depth handles: in [nt][nk][nxy], eta [nt][nxy] (null: 0), depth [nxy] (null for depth levels), out [nt][np][nxy]
+int launch_vertical_depth(const VertTable& vt, const float* d_in, const float* d_eta, const float* d_depth, long long nxy, long long nt, float* d_out,
+                          cudaStream_t st);
 
 } // namespace fb

@@ -16,6 +16,10 @@
 // altitude z_k, which it computes level by level as the walk goes up from the surface (standard atmosphere of p_k, the
 // hypsometric sum over T and q, or a z field) and never stores.  The walk ends at the bracket of the highest target, so a column
 // is read only up to there (DESIGN.md sections 2 and 4).
+//
+// k_vertical_depth is the depth branch (targets in metres below the sea surface datum, from depth levels or the CF ocean sigma and
+// s-coordinates): the same walk, down from the surface end, in x_k = -z_k, which it computes from the terms in shared memory and the
+// column's sea-floor depth and sea surface height as it goes and never stores.  Land columns read no field value.
 #include "kernels.h"
 
 namespace fb {
@@ -341,6 +345,99 @@ __global__ void __launch_bounds__(kThreads, 3)
     }
 }
 
+// in [nt][nk][nxy]; eta [nt][nxy] (null: 0); depth [nxy] (null for depth levels); out [nt][np][nxy]; blockIdx.y = time step.
+// tab: levels, sigma_k or depth_c * s_k [nk] | C_k [nk] | sorted target depths[np] | output row of each sorted target[np]
+template <int VC, int M>
+__global__ void __launch_bounds__(kThreads, 3)
+    k_vertical_depth(const float* __restrict__ in, const float* __restrict__ eta, const float* __restrict__ depth, float* __restrict__ out,
+                     const double* __restrict__ tab, int nk, int np, int extrapolate, double depth_c, long long nxy, long long t0)
+{
+    extern __shared__ double s_tab[];
+    const int ntab = 2 * nk + 2 * np;
+    for (int i = threadIdx.x; i < ntab; i += blockDim.x)
+        s_tab[i] = tab[i];
+    __syncthreads();
+    const double* s_a = s_tab;
+    const double* s_c = s_tab + nk;
+    const double* s_lev = s_tab + 2 * nk;
+    const double* s_row = s_lev + np;
+
+    const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (c >= nxy)
+        return;
+    const long long t = t0 + blockIdx.y;
+    const float* col = in + t * nk * nxy + c;
+    float* ocol = out + t * np * nxy + c;
+    // the sea-floor depth h and the sea surface height e: land (h NaN or <= 0) and a NaN eta give a NaN column, which reads no field value
+    double h = 0.0, e = 0.0;
+    bool flat = false;
+    if (VC != FB_VD_DEPTH) {
+        h = (double)__ldg(depth + c);
+        flat = !(h > 0.0);
+        if (!flat && eta) {
+            e = (double)__ldg(eta + t * nxy + c);
+            flat = isnan(e);
+        }
+    }
+    const double eh = e + h;                                                // sigma, g2
+    const double hd = VC == FB_VD_OCEAN_S_G1 ? h - depth_c : depth_c + h; // g1: h - depth_c; g2: depth_c + h
+    // x_k = -z_k, the depth of level k below the datum of eta (DESIGN.md section 2)
+    auto level_x = [&](int k) -> double {
+        if (VC == FB_VD_DEPTH)
+            return s_a[k];
+        if (VC == FB_VD_OCEAN_SIGMA)
+            return -(e + __dmul_rn(s_a[k], eh));
+        if (VC == FB_VD_OCEAN_S_G1) {
+            const double S = s_a[k] + __dmul_rn(hd, s_c[k]);
+            return -(S + __dmul_rn(e, 1.0 + S / h));
+        }
+        const double S = (s_a[k] + __dmul_rn(h, s_c[k])) / hd;
+        return -(e + __dmul_rn(eh, S));
+    };
+    // The walk: level m counted from the surface end (the smaller x); xj = the coordinate of level j, xjm = that of level j - 1.
+    bool up = true;
+    double x0 = 0.0, xjm = 0.0, xj = 0.0;
+    if (!flat) {
+        const double xf = level_x(0), xl = level_x(nk - 1);
+        up = xf < xl;
+        flat = !(xf < xl) && !(xf > xl);
+        x0 = up ? xf : xl;
+        xj = up ? level_x(1) : level_x(nk - 2);
+        xjm = x0;
+    }
+    int j = 1, kc = -2;
+    float va = 0.f, vb = 0.f;
+    for (int i = 0; i < np; ++i) {
+        const double D = s_lev[i];
+        float r = undef_f();
+        if (!flat) {
+            while (j < nk - 1 && xj < D) { // NaN stops the walk: every target below it gets NaN
+                xjm = xj;
+                ++j;
+                xj = level_x(up ? j : nk - 1 - j);
+            }
+            if (extrapolate || (D >= x0 && !(j == nk - 1 && xj < D))) {
+                const int k = j - 1;
+                const int ka = up ? k : nk - 1 - k, kb = up ? k + 1 : nk - 2 - k;
+                if (k != kc) {
+                    va = k == kc + 1 ? vb : __ldg(col + (long long)ka * nxy); // the upper level of this bracket is the lower one of the last
+                    vb = __ldg(col + (long long)kb * nxy);
+                    kc = k;
+                }
+                if (isnan(xjm) || isnan(xj)) {
+                    r = undef_f();
+                } else if (M == FB_VINT_NN) {
+                    r = fabs(D - xj) < fabs(D - xjm) ? vb : va;
+                } else {
+                    const double w = xjm == xj ? 0.0 : (D - xjm) / (xj - xjm);
+                    r = (float)((double)va + __dmul_rn(w, (double)vb - (double)va));
+                }
+            }
+        }
+        __stcs(ocol + (long long)s_row[i] * nxy, r);
+    }
+}
+
 } // namespace
 
 int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st)
@@ -407,6 +504,42 @@ int launch_vertical_height(const VertTable& vt, const float* d_in, const float* 
 #undef FB_CASE
         default:
             FB_REQUIRE(false, "unknown height converter / method " + std::to_string(vt.converter) + " / " + std::to_string(vt.method));
+        }
+        count_launch();
+        FB_CUDA_CHECK(cudaGetLastError());
+    }
+    return FB_OK;
+}
+
+int launch_vertical_depth(const VertTable& vt, const float* d_in, const float* d_eta, const float* d_depth, long long nxy, long long nt, float* d_out,
+                          cudaStream_t st)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    FB_REQUIRE(vt.depth_vcoord == FB_VD_DEPTH || d_depth != nullptr, "ocean s- and sigma coordinates need the sea-floor depth");
+    const size_t smem = sizeof(double) * (size_t)(2 * vt.nk + 2 * vt.np);
+    const long long bx = (nxy + kThreads - 1) / kThreads;
+    FB_REQUIRE(bx < 2147483647LL, "too many columns for one call");
+    const int key = vt.depth_vcoord * 8 + vt.method;
+    for (long long t0 = 0; t0 < nt; t0 += 65535) {
+        const dim3 grid((unsigned)bx, (unsigned)std::min<long long>(nt - t0, 65535));
+        switch (key) {
+#define FB_CASE(V, M)                                                                                                                      \
+    case V * 8 + M:                                                                                                                        \
+        k_vertical_depth<V, M><<<grid, kThreads, smem, st>>>(d_in, d_eta, d_depth, d_out, vt.d_tab, vt.nk, vt.np, vt.extrapolate ? 1 : 0,  \
+                                                             vt.depth_c, nxy, t0);                                                         \
+        break;
+            FB_CASE(FB_VD_DEPTH, FB_VINT_LIN)
+            FB_CASE(FB_VD_DEPTH, FB_VINT_NN)
+            FB_CASE(FB_VD_OCEAN_SIGMA, FB_VINT_LIN)
+            FB_CASE(FB_VD_OCEAN_SIGMA, FB_VINT_NN)
+            FB_CASE(FB_VD_OCEAN_S_G1, FB_VINT_LIN)
+            FB_CASE(FB_VD_OCEAN_S_G1, FB_VINT_NN)
+            FB_CASE(FB_VD_OCEAN_S_G2, FB_VINT_LIN)
+            FB_CASE(FB_VD_OCEAN_S_G2, FB_VINT_NN)
+#undef FB_CASE
+        default:
+            FB_REQUIRE(false, "unknown depth coordinate / method " + std::to_string(vt.depth_vcoord) + " / " + std::to_string(vt.method));
         }
         count_launch();
         FB_CUDA_CHECK(cudaGetLastError());

@@ -1,5 +1,5 @@
-"""Host-side mirror of the pressure and height branches of the reference's CDMVerticalInterpolator
-(``--verticalInterpolate.type=pressure|height|altitude --verticalInterpolate.method=... --verticalInterpolate.level1=...``).
+"""Host-side mirror of the pressure, height and depth branches of the reference's CDMVerticalInterpolator
+(``--verticalInterpolate.type=pressure|height|altitude|depth --verticalInterpolate.method=... --verticalInterpolate.level1=...``).
 
 The source vertical coordinate is given by its CF standard name and formula terms, as the reference reads them from the CDM:
 
@@ -9,7 +9,8 @@ The source vertical coordinate is given by its CF standard name and formula term
 
 The surface pressure ``ps`` is not a term here: it is a field, passed with every slice.  All pressures are in the unit of the
 target levels (hPa, as the reference's level1 option); ``ps_scale`` converts the ``ps`` field to it (0.01 for Pa).  Height and
-altitude levels are in metres (:class:`HeightInterpolator`).  The arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md
+altitude levels are in metres (:class:`HeightInterpolator`), as are depth levels below the sea surface (:class:`DepthInterpolator`, from
+depth levels or the CF ocean sigma and s-coordinates).  The arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md
 section 2 states it).
 """
 from __future__ import annotations
@@ -34,6 +35,12 @@ VCOORD_PRESSURE, VCOORD_HYBRID, VCOORD_SIGMA = 0, 1, 2  # FB200_VCOORD_*
 TARGETS = {"altitude": 0, "height": 1}
 #: the ways to the altitude of every source level -> FB200_VZ_*
 CONVERTERS = {"standard": 0, "hypsometric": 1, "field": 2}
+
+DEPTH = "depth"
+OCEAN_SIGMA = "ocean_sigma_coordinate"
+OCEAN_S_G1 = "ocean_s_coordinate_g1"
+OCEAN_S_G2 = "ocean_s_coordinate_g2"
+VCOORD_DEPTH, VCOORD_OCEAN_SIGMA, VCOORD_OCEAN_S_G1, VCOORD_OCEAN_S_G2 = 3, 4, 5, 6  # FB200_VCOORD_*
 
 
 def vertical_method(name: str) -> int:
@@ -92,6 +99,51 @@ class _VerticalHandle:
         if self.needs_ps and (ps is None or int(np.prod(ps.shape, dtype=np.int64)) != nt * nxy):
             raise FimexB200Error(f"ps must hold nt * nxy = {nt * nxy} values")
         return nt, nxy, (nt, self.levels.size) + tuple(field.shape[2:])
+
+    def _values_columns(self, field, ps, columns, stream):
+        """interpolateValues through the _columns calls; columns(nt, nxy, device) -> (fb200_vcolumns, arrays to keep alive)"""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
+            nt, nxy, shape = self._shape(field, ps)
+            cols, keep = columns(nt, nxy, True)
+            out = torch.empty(shape, dtype=torch.float32, device=field.device)
+            check(lib.fb200_vinterp_interpolate_values_columns_device(self._h, ptr(field), C.byref(cols), nxy, nt, ptr(out), _stream_ptr(stream)),
+                  "interpolateValues")
+            return out
+        a = capi.f32(field)
+        nt, nxy, shape = self._shape(a, ps)
+        cols, keep = columns(nt, nxy, False)
+        out = np.empty(shape, dtype=np.float32)
+        check(lib.fb200_vinterp_interpolate_values_columns(self._h, ptr(a), C.byref(cols), nxy, nt, ptr(out)), "interpolateValues")
+        return out
+
+    def _slice_columns(self, field, ps, columns, bad_value, out_dtype, stream):
+        """getDataSlice through the _columns calls, as _values_columns"""
+        lib = load()
+        if _is_torch(field):
+            import torch
+            if not field.is_cuda or not field.is_contiguous():
+                raise FimexB200Error("device path needs a contiguous CUDA tensor")
+            odt = out_dtype if out_dtype is not None else field.dtype
+            bad = capi.default_fill_value(field.dtype) if bad_value is None else float(bad_value)
+            nt, nxy, shape = self._shape(field, ps)
+            cols, keep = columns(nt, nxy, True)
+            out = torch.empty(shape, dtype=odt, device=field.device)
+            check(lib.fb200_vinterp_get_data_slice_columns_device(self._h, int(capi.cdm_type(field.dtype)), ptr(field), C.byref(cols), nxy, nt,
+                                                                  bad, int(capi.cdm_type(odt)), ptr(out), _stream_ptr(stream)), "getDataSlice")
+            return out
+        a = np.ascontiguousarray(field)
+        odt = np.dtype(out_dtype) if out_dtype is not None else a.dtype
+        bad = capi.default_fill_value(a.dtype) if bad_value is None else float(bad_value)
+        nt, nxy, shape = self._shape(a, ps)
+        cols, keep = columns(nt, nxy, False)
+        out = np.empty(shape, dtype=odt)
+        check(lib.fb200_vinterp_get_data_slice_columns(self._h, int(capi.cdm_type(a.dtype)), ptr(a), C.byref(cols), nxy, nt, bad,
+                                                       int(capi.cdm_type(odt)), ptr(out)), "getDataSlice")
+        return out
 
 
 class VerticalInterpolator(_VerticalHandle):
@@ -169,6 +221,25 @@ class _Columns(C.Structure):
     _fields_ = [("ps", C.c_void_p), ("t", C.c_void_p), ("q", C.c_void_p), ("z", C.c_void_p), ("zs", C.c_void_p)]
 
 
+def _fill_columns(slots, device):
+    """{slot of fb200_vcolumns: (argument name, array, number of values)} -> (the fb200_vcolumns, the arrays it points into, kept alive
+    by the caller): float32, CUDA tensors on the device path"""
+    cols, keep = _Columns(), []
+    for slot, (name, a, n) in slots.items():
+        if device:
+            import torch
+            if not _is_torch(a) or not a.is_cuda or a.dtype != torch.float32:
+                raise FimexB200Error(f"{name} must be a float32 CUDA tensor on the device path")
+            a = a.contiguous()
+        else:
+            a = capi.f32(a)
+        if int(np.prod(a.shape, dtype=np.int64)) != n:
+            raise FimexB200Error(f"{name} must hold {n} values, got shape {tuple(a.shape)}")
+        keep.append(a)
+        setattr(cols, slot, ptr(a).value)
+    return cols, keep
+
+
 class HeightInterpolator(_VerticalHandle):
     """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on target levels in metres: above the
     ground (``type="height"``) or above sea level (``type="altitude"``).  The altitude of every source level comes from
@@ -216,68 +287,96 @@ class HeightInterpolator(_VerticalHandle):
                  "q": (q, self.needs_t, column, "the specific humidity q"),
                  "z": (z, self.needs_z, column, "the altitude field z"),
                  "zs": (zs, self.needs_zs, nxy, "the surface altitude zs")}
-        cols, keep = _Columns(), []
+        slots = {}
         for name, (a, used, n, what) in given.items():
             if a is None or not used:
                 if used and name != "q":
                     raise FimexB200Error(f"this converter and target need {what}")
                 continue
-            if device:
-                import torch
-                if not _is_torch(a) or not a.is_cuda or a.dtype != torch.float32:
-                    raise FimexB200Error(f"{name} must be a float32 CUDA tensor on the device path")
-                a = a.contiguous()
-            else:
-                a = capi.f32(a)
-            if int(np.prod(a.shape, dtype=np.int64)) != n:
-                raise FimexB200Error(f"{name} must hold {n} values, got shape {tuple(a.shape)}")
-            keep.append(a)
-            setattr(cols, name, ptr(a).value)
-        return cols, keep
+            slots[name] = (name, a, n)
+        return _fill_columns(slots, device)
 
     def interpolateValues(self, field, ps=None, t=None, q=None, z=None, zs=None, stream=None):
         """float32 [nt][nk][...] with NaN for undefined values -> float32 [nt][np][...] (numpy or CUDA tensors)"""
-        lib = load()
-        if _is_torch(field):
-            import torch
-            if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
-                raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
-            nt, nxy, shape = self._shape(field, ps)
-            cols, keep = self._columns(nt, nxy, True, ps, t, q, z, zs)
-            out = torch.empty(shape, dtype=torch.float32, device=field.device)
-            check(lib.fb200_vinterp_interpolate_values_columns_device(self._h, ptr(field), C.byref(cols), nxy, nt, ptr(out), _stream_ptr(stream)),
-                  "interpolateValues")
-            return out
-        a = capi.f32(field)
-        nt, nxy, shape = self._shape(a, ps)
-        cols, keep = self._columns(nt, nxy, False, ps, t, q, z, zs)
-        out = np.empty(shape, dtype=np.float32)
-        check(lib.fb200_vinterp_interpolate_values_columns(self._h, ptr(a), C.byref(cols), nxy, nt, ptr(out)), "interpolateValues")
-        return out
+        return self._values_columns(field, ps, lambda nt, nxy, device: self._columns(nt, nxy, device, ps, t, q, z, zs), stream)
 
     def getDataSlice(self, field, ps=None, t=None, q=None, z=None, zs=None, bad_value=None, out_dtype=None, stream=None):
         """The per-slice body of the vertical getDataSlice: `field` [nt][nk][...] of any CDM numeric type (numpy array, or CUDA tensor
         for the device-resident path), fill -> NaN, interpolate, NaN -> fill and cast to `out_dtype` (default: the input's type).
         `bad_value` = CDM::getFillValue of the variable (default: the type's default fill value)."""
-        lib = load()
-        if _is_torch(field):
-            import torch
-            if not field.is_cuda or not field.is_contiguous():
-                raise FimexB200Error("device path needs a contiguous CUDA tensor")
-            odt = out_dtype if out_dtype is not None else field.dtype
-            bad = capi.default_fill_value(field.dtype) if bad_value is None else float(bad_value)
-            nt, nxy, shape = self._shape(field, ps)
-            cols, keep = self._columns(nt, nxy, True, ps, t, q, z, zs)
-            out = torch.empty(shape, dtype=odt, device=field.device)
-            check(lib.fb200_vinterp_get_data_slice_columns_device(self._h, int(capi.cdm_type(field.dtype)), ptr(field), C.byref(cols), nxy, nt,
-                                                                  bad, int(capi.cdm_type(odt)), ptr(out), _stream_ptr(stream)), "getDataSlice")
-            return out
-        a = np.ascontiguousarray(field)
-        odt = np.dtype(out_dtype) if out_dtype is not None else a.dtype
-        bad = capi.default_fill_value(a.dtype) if bad_value is None else float(bad_value)
-        nt, nxy, shape = self._shape(a, ps)
-        cols, keep = self._columns(nt, nxy, False, ps, t, q, z, zs)
-        out = np.empty(shape, dtype=odt)
-        check(lib.fb200_vinterp_get_data_slice_columns(self._h, int(capi.cdm_type(a.dtype)), ptr(a), C.byref(cols), nxy, nt, bad,
-                                                       int(capi.cdm_type(odt)), ptr(out)), "getDataSlice")
-        return out
+        return self._slice_columns(field, ps, lambda nt, nxy, device: self._columns(nt, nxy, device, ps, t, q, z, zs), bad_value, out_dtype,
+                                   stream)
+
+
+def _depth_source(standard_name: str, terms: dict):
+    """(vcoord, s, C, depth_c) of the source vertical coordinate of a depth handle: depth levels s = the levels; ocean sigma s = sigma;
+    g1, g2 s, C, depth_c.  The fields eta and depth of the ocean coordinates are not terms here."""
+    def need(t, *names):
+        missing = [n for n in names if n not in t]
+        if missing:
+            raise FimexB200Error(f"{standard_name} needs the terms {', '.join(names)}; got {sorted(terms)}")
+    if standard_name == DEPTH:
+        need(terms, "depth")
+        return VCOORD_DEPTH, f64(terms["depth"]).ravel(), None, 0.0
+    t = {k: v for k, v in terms.items() if k not in ("eta", "depth")}
+    if standard_name == OCEAN_SIGMA:
+        need(t, "sigma")
+        return VCOORD_OCEAN_SIGMA, f64(t["sigma"]).ravel(), None, 0.0
+    if standard_name in (OCEAN_S_G1, OCEAN_S_G2):
+        need(t, "s", "C", "depth_c")
+        s, Ck = f64(t["s"]).ravel(), f64(t["C"]).ravel()
+        if s.size != Ck.size:
+            raise FimexB200Error(f"{standard_name}: {s.size} values of s but {Ck.size} of C")
+        vcoord = VCOORD_OCEAN_S_G1 if standard_name == OCEAN_S_G1 else VCOORD_OCEAN_S_G2
+        return vcoord, s, Ck, float(np.asarray(t["depth_c"], dtype=np.float64).reshape(-1)[0])
+    raise FimexB200Error(f"vertical coordinate '{standard_name}' is not supported for depth levels "
+                         f"(one of {DEPTH}, {OCEAN_SIGMA}, {OCEAN_S_G1}, {OCEAN_S_G2})")
+
+
+class DepthInterpolator(_VerticalHandle):
+    """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on target depths in metres below the sea
+    surface datum, positive down (``--verticalInterpolate.type=depth``).  Source coordinates and their terms:
+
+    * ``depth``: depth levels, positive down, ``{"depth": levels}``;
+    * ``ocean_sigma_coordinate``: ``{"sigma": sigma}``;
+    * ``ocean_s_coordinate_g1`` and ``_g2``: ``{"s": s, "C": C, "depth_c": depth_c}``.
+
+    The ocean coordinates read two fields with every slice: ``depth`` [...], the sea-floor depth h [m, positive down], which they
+    need, and ``eta`` [nt][...], the sea surface height [m] (None: 0), both float32.  A column with h NaN or <= 0 (land) or a NaN eta
+    gives NaN.  Methods: ``linear`` and ``nearestneighbor``."""
+
+    def __init__(self, standard_name: str, terms: dict, method: str, levels, extrapolate: bool = True):
+        self.method = vertical_method(method)
+        if self.method not in (METHODS["linear"], METHODS["nearestneighbor"]):
+            raise FimexB200Error(f"depth levels take the methods linear and nearestneighbor only (log and loglog are defined on ln p), "
+                                 f"got '{method}'")
+        self.levels = f64(levels).ravel()
+        self._h = C.c_void_p()
+        vcoord, s, Ck, depth_c = _depth_source(standard_name, terms)
+        self.nk = s.size
+        self.needs_depth = vcoord != VCOORD_DEPTH
+        rc = load().fb200_vinterp_create_depth(self.method, vcoord, ptr(s), ptr(Ck), self.nk, depth_c, ptr(self.levels), self.levels.size,
+                                               int(bool(extrapolate)), C.byref(self._h))
+        check(rc, "DepthInterpolator")
+
+    def _columns(self, nt, nxy, device, eta, depth):
+        """the fb200_vcolumns of a call (eta in the ps slot, the sea-floor depth in the zs slot), and the arrays it points into"""
+        slots = {}
+        if self.needs_depth:
+            if depth is None:
+                raise FimexB200Error("ocean s- and sigma coordinates need the sea-floor depth")
+            slots["zs"] = ("depth", depth, nxy)
+            if eta is not None:
+                slots["ps"] = ("eta", eta, nt * nxy)
+        return _fill_columns(slots, device)
+
+    def interpolateValues(self, field, eta=None, depth=None, stream=None):
+        """float32 [nt][nk][...] with NaN for undefined values -> float32 [nt][np][...] (numpy or CUDA tensors)"""
+        return self._values_columns(field, None, lambda nt, nxy, device: self._columns(nt, nxy, device, eta, depth), stream)
+
+    def getDataSlice(self, field, eta=None, depth=None, bad_value=None, out_dtype=None, stream=None):
+        """The per-slice body of the vertical getDataSlice: `field` [nt][nk][...] of any CDM numeric type (numpy array, or CUDA tensor
+        for the device-resident path), fill -> NaN, interpolate, NaN -> fill and cast to `out_dtype` (default: the input's type).
+        `bad_value` = CDM::getFillValue of the variable (default: the type's default fill value)."""
+        return self._slice_columns(field, None, lambda nt, nxy, device: self._columns(nt, nxy, device, eta, depth), bad_value, out_dtype,
+                                   stream)

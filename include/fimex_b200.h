@@ -347,7 +347,9 @@ int fb200_vinterp_get_data_slice_device(const fb200_vinterp* handle, int inType,
 #define FB200_VZ_FIELD 2
 #define FB200_VZ_ALTITUDE 0
 #define FB200_VZ_HEIGHT 1
-/* the per-column inputs of a call, float32, NULL = not given: ps [nt][nxy], t, q, z [nt][nk][nxy], zs [nxy] (no time axis) */
+/* the per-column inputs of a call, float32, NULL = not given: ps [nt][nxy], t, q, z [nt][nk][nxy], zs [nxy] (no time axis).
+ * Depth handles (1f) read two slots: ps carries the sea surface height eta [m] (NULL: 0) and zs the sea-floor depth h [m, positive
+ * down]; t, q and z are not read. */
 typedef struct fb200_vcolumns {
     const float* ps;
     const float* t;
@@ -370,6 +372,30 @@ int fb200_vinterp_get_data_slice_columns(const fb200_vinterp* handle, int inType
                                          size_t nt, double badValue, int outType, void* out);
 int fb200_vinterp_get_data_slice_columns_device(const fb200_vinterp* handle, int inType, const void* d_in, const fb200_vcolumns* d_cols,
                                                 size_t nxy, size_t nt, double badValue, int outType, void* d_out, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * (1f) vertical interpolation to depth levels: the depth branch of CDMVerticalInterpolator
+ *      (--verticalInterpolate.type=depth; DESIGN.md section 2 states the arithmetic)
+ *
+ * Targets in metres below the datum of eta, positive down.  Source vertical coordinates (CF standard names), with z_k the
+ * altitude of level k (negative below the datum) and x_k = -z_k:
+ *   FB200_VCOORD_DEPTH           depth levels, positive down: x_k = s_k (C, depth_c not used)
+ *   FB200_VCOORD_OCEAN_SIGMA     ocean_sigma_coordinate: z = eta + sigma_k * (h + eta), sigma_k = s_k
+ *   FB200_VCOORD_OCEAN_S_G1      ocean_s_coordinate_g1: S = depth_c * s_k + (h - depth_c) * C_k, z = S + eta * (1 + S / h)
+ *   FB200_VCOORD_OCEAN_S_G2      ocean_s_coordinate_g2: S = (depth_c * s_k + h * C_k) / (depth_c + h), z = eta + (eta + h) * S
+ * eta [nt][nxy] is the sea surface height (the ps slot of fb200_vcolumns, or the ps argument of the calls without _columns; NULL
+ * means 0), h [nxy] the sea-floor depth (the zs slot, no time axis).  The ocean coordinates need h, so the calls without _columns
+ * refuse them; depth-level handles read neither and work on every call.  A column with h NaN or <= 0 (land), a NaN eta, or equal
+ * ends of x gives NaN and reads no field value.  method: MIFI_VINT_METHOD_LIN or _NN only.  C != NULL for g1 and g2;
+ * 0 <= depth_c < inf; 2 <= nk <= 1024, 1 <= np <= 1024, all values finite.  Other rules as for the height handles.
+ * ---------------------------------------------------------------------------------------------- */
+#define FB200_VCOORD_DEPTH 3
+#define FB200_VCOORD_OCEAN_SIGMA 4
+#define FB200_VCOORD_OCEAN_S_G1 5
+#define FB200_VCOORD_OCEAN_S_G2 6
+
+int fb200_vinterp_create_depth(int method, int vcoord, const double* s, const double* C, int nk, double depth_c, const double* levels, int np,
+                               int extrapolate, fb200_vinterp** handle);
 
 /* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
