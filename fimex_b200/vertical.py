@@ -146,6 +146,14 @@ class _VerticalHandle:
         return out
 
 
+def _device_ps(ps):
+    """ps of a device-path call, as the C ABI reads it: float32 on the device (the shape is checked by _shape); anything else raises"""
+    import torch
+    if not _is_torch(ps) or not ps.is_cuda or ps.dtype != torch.float32:
+        raise FimexB200Error("ps must be a float32 CUDA tensor on the device path")
+    return ps.contiguous()
+
+
 class VerticalInterpolator(_VerticalHandle):
     """Interpolates [nt][nk][...] fields on the source vertical coordinate to [nt][np][...] on the target pressure levels."""
 
@@ -172,7 +180,7 @@ class VerticalInterpolator(_VerticalHandle):
             if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
                 raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
             nt, nxy, shape = self._shape(field, ps)
-            psd = ps.contiguous() if ps is not None and self.needs_ps else None
+            psd = _device_ps(ps) if self.needs_ps else None
             out = torch.empty(shape, dtype=torch.float32, device=field.device)
             check(lib.fb200_vinterp_interpolate_values_device(self._h, ptr(field), ptr(psd), nxy, nt, ptr(out), _stream_ptr(stream)),
                   "interpolateValues")
@@ -196,11 +204,7 @@ class VerticalInterpolator(_VerticalHandle):
             odt = out_dtype if out_dtype is not None else field.dtype
             bad = capi.default_fill_value(field.dtype) if bad_value is None else float(bad_value)
             nt, nxy, shape = self._shape(field, ps)
-            psd = None
-            if ps is not None and self.needs_ps:
-                if not ps.is_cuda or ps.dtype != torch.float32:
-                    raise FimexB200Error("ps must be a float32 CUDA tensor on the device path")
-                psd = ps.contiguous()
+            psd = _device_ps(ps) if self.needs_ps else None
             out = torch.empty(shape, dtype=odt, device=field.device)
             check(lib.fb200_vinterp_get_data_slice_device(self._h, int(capi.cdm_type(field.dtype)), ptr(field), ptr(psd), nxy, nt, bad,
                                                           int(capi.cdm_type(odt)), ptr(out), _stream_ptr(stream)), "getDataSlice")
