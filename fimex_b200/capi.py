@@ -185,6 +185,10 @@ def _declare(lib):
         "fb200_vinterp_get_data_slice_columns": (i, [_vp, i, _vp, _vp, sz, sz, C.c_double, i, _vp]),
         "fb200_vinterp_get_data_slice_columns_device": (i, [_vp, i, _vp, _vp, sz, sz, C.c_double, i, _vp, _vp]),
         "fb200_vinterp_create_depth": (i, [i, i, _vp, _vp, i, C.c_double, _vp, i, i, P(_vp)]),
+        "fb200_vconvert_create": (i, [i, i, _vp, _vp, i, C.c_double, C.c_double, P(_vp)]),
+        "fb200_vconvert_destroy": (None, [_vp]),
+        "fb200_vconvert_values": (i, [_vp, _vp, _vp, sz, sz, _vp]),
+        "fb200_vconvert_values_device": (i, [_vp, _vp, _vp, sz, sz, _vp, _vp]),
         "mifi_string_to_interpolation_method": (i, [C.c_char_p]),
         "mifi_interpolate_f": (i, [i, C.c_char_p, _vp, _vp, _vp, i, i, i, i, i, C.c_char_p, _vp, _vp, _vp, i, i, i, i]),
         "mifi_vector_reproject_values_f": (i, [i, C.c_char_p, C.c_char_p, _vp, _vp, _vp, _vp, i, i, i, i, i]),

@@ -2176,6 +2176,17 @@ constexpr double kStdL[kStdLayers] = {-6.5e-3, 0.0, 1e-3, 2.8e-3, 0.0, -2.8e-3, 
 constexpr double kStdP[kStdLayers] = {1013.25, 226.3206, 54.74889, 8.680187, 1.109063, 0.6693887, 0.03956420};
 constexpr double kRstar = 8.31432, kMair = 0.0289644, kMwater = 0.01801528, kG0 = 9.80665;
 
+// the a | b terms of p_k = a_k + b_k * (ps * ps_scale - shift) from the formula terms of FB200_VCOORD_PRESSURE (a = the levels),
+// _HYBRID (a = ap, b) or _SIGMA (b = sigma; a_k = shift = ptop) into tab[0 .. 2 nk)
+void pressure_terms(int vcoord, const double* a, const double* b, int nk, double ptop, double* tab)
+{
+    const bool sigma = vcoord == FB200_VCOORD_SIGMA, hybrid = vcoord == FB200_VCOORD_HYBRID;
+    for (int k = 0; k < nk; ++k) {
+        tab[k] = sigma ? ptop : a[k];
+        tab[nk + k] = (sigma || hybrid) ? b[k] : 0.0;
+    }
+}
+
 int vinterp_create_height(int method, int converter, int target, int vcoord, const double* a, const double* b, int nk, double ptop,
                           double ps_scale, double z_scale, double zs_scale, const double* levels, int np, int extrapolate, fb200_vinterp** handle)
 {
@@ -2223,10 +2234,8 @@ int vinterp_create_height(int method, int converter, int target, int vcoord, con
     vt.H = kRstar / (kMair * kG0);
     vt.cq = kMair / kMwater - 1.0;
     std::vector<double> tab(2 * (size_t)nk + 4 * kStdLayers + 2 * (size_t)np, 0.0);
-    for (int k = 0; k < nk && !field; ++k) {
-        tab[k] = sigma ? ptop : a[k];
-        tab[nk + k] = (sigma || hybrid) ? b[k] : 0.0;
-    }
+    if (!field)
+        pressure_terms(vcoord, a, b, nk, ptop, tab.data());
     double* layers = tab.data() + 2 * nk; // h_b | p_b | c_b | e_b
     for (int l = 0; l < kStdLayers; ++l) {
         layers[l] = kStdH[l];
@@ -2397,6 +2406,103 @@ const fb200_vcolumns& or_none(const fb200_vcolumns* cols)
 
 } // namespace
 
+// ======================================================================================================
+// the data conversions of the vertical interpolator (CDMPressureConversions: theta2T, omega2vwind, add4Dpressure), on the model levels
+// ======================================================================================================
+struct fb200_vconvert {
+    int device = 0;
+    int op = 0, vcoord = 0;
+    bool has_ps = false; // hybrid or sigma levels
+    double kappa = 0.0;  // R_d / c_pd of theta2T
+    fb::VertTable vt;    // a | b, ps_scale, shift and H (omega2vwind) as for the pressure and height handles; np = 0
+    ~fb200_vconvert()
+    {
+        fb::DeviceGuard on(device);
+        if (vt.d_tab)
+            cudaFree(vt.d_tab);
+    }
+};
+
+namespace {
+
+int vconvert_create(int op, int vcoord, const double* a, const double* b, int nk, double ptop, double ps_scale, fb200_vconvert** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(op >= FB_VCONV_THETA2T && op <= FB_VCONV_PRESSURE, "unknown data conversion " + std::to_string(op));
+    FB_REQUIRE(vcoord >= FB200_VCOORD_PRESSURE && vcoord <= FB200_VCOORD_SIGMA, "unknown source vertical coordinate " + std::to_string(vcoord));
+    FB_REQUIRE(nk >= 1 && nk <= kMaxVertLevels, "number of levels must be in [1, 1024], got " + std::to_string(nk));
+    const bool sigma = vcoord == FB200_VCOORD_SIGMA, hybrid = vcoord == FB200_VCOORD_HYBRID;
+    FB_REQUIRE(sigma || a != nullptr, "null ap (or pressure levels)");
+    FB_REQUIRE(!(sigma || hybrid) || b != nullptr, sigma ? "null sigma" : "null b");
+    FB_REQUIRE((sigma || all_finite(a, nk)) && (!(sigma || hybrid) || all_finite(b, nk)), "vertical coordinate values must be finite");
+    FB_REQUIRE(std::isfinite(ps_scale) && std::isfinite(ptop), "ps_scale and ptop must be finite");
+    if (use_device(default_device()) != FB_OK)
+        return FB_ERROR;
+    std::unique_ptr<fb200_vconvert> h(new fb200_vconvert());
+    h->device = default_device();
+    h->op = op;
+    h->vcoord = vcoord;
+    h->has_ps = sigma || hybrid;
+    h->kappa = 2.0 / 7.0; // R_d / c_pd of an ideal diatomic gas, c_pd = 3.5 R_d
+    VertTable& vt = h->vt;
+    vt.nk = nk;
+    vt.ps_scale = ps_scale;
+    vt.shift = sigma ? ptop : 0.0;
+    vt.H = kRstar / (kMair * kG0); // H g0 = R* / M = R_d
+    std::vector<double> tab(2 * (size_t)nk, 0.0);
+    pressure_terms(vcoord, a, b, nk, ptop, tab.data());
+    cudaStream_t st = cudaStreamPerThread;
+    if (upload_table(vt, tab, st) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    *handle = h.release();
+    return FB_OK;
+}
+
+int check_vconvert_call(const fb200_vconvert* h, const void* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, const void* out)
+{
+    FB_REQUIRE(h != nullptr, "null data conversion handle");
+    if (nxy * nt != 0) {
+        FB_REQUIRE(out && (in || h->op == FB_VCONV_PRESSURE), "null data pointer");
+        FB_REQUIRE(!h->has_ps || cols.ps, "this vertical coordinate needs the surface pressure ps");
+        FB_REQUIRE(h->op != FB_VCONV_OMEGA2VWIND || cols.t, "omega2vwind needs the air temperature t");
+    }
+    return use_device(h->device);
+}
+
+int vconvert_device(const fb200_vconvert* h, const float* d_in, const fb200_vcolumns& cols, size_t nxy, size_t nt, float* d_out, cudaStream_t st)
+{
+    return launch_vconvert(h->op, h->vcoord, h->vt, h->kappa, h->op == FB_VCONV_PRESSURE ? nullptr : d_in, h->has_ps ? cols.ps : nullptr,
+                           h->op == FB_VCONV_OMEGA2VWIND ? cols.t : nullptr, (long long)nxy, (long long)nt, d_out, st);
+}
+
+// host arrays: time steps are the units of the staging pipeline; the field, ps and t are its inputs where the conversion reads them
+int vconvert_host(const fb200_vconvert* h, const float* in, const fb200_vcolumns& cols, size_t nxy, size_t nt, float* out)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    const size_t level = nxy * sizeof(float), column = level * (size_t)h->vt.nk;
+    const float* steps[3] = {h->op == FB_VCONV_PRESSURE ? nullptr : in, h->has_ps ? cols.ps : nullptr, h->op == FB_VCONV_OMEGA2VWIND ? cols.t : nullptr};
+    const size_t unit[3] = {column, level, column};
+    HostArrays arrays;
+    arrays.device = h->device;
+    for (int i = 0; i < 3; ++i) {
+        arrays.in[i] = steps[i];
+        arrays.in_unit[i] = steps[i] ? unit[i] : 0;
+    }
+    arrays.out[0] = out;
+    arrays.out_unit[0] = column;
+    return stage_host(arrays, nt, [&](const void* const* d_in, size_t n, void* const* d_out, cudaStream_t s) {
+        fb200_vcolumns dc = {};
+        dc.ps = static_cast<const float*>(d_in[1]);
+        dc.t = static_cast<const float*>(d_in[2]);
+        return vconvert_device(h, static_cast<const float*>(d_in[0]), dc, nxy, n, static_cast<float*>(d_out[0]), s);
+    });
+}
+
+} // namespace
+
 extern "C" {
 
 int fb200_vinterp_create_hybrid(int method, const double* ap, const double* b, int nk, double ps_scale, const double* levels, int np,
@@ -2490,6 +2596,31 @@ int fb200_vinterp_get_data_slice_columns_device(const fb200_vinterp* h, int inTy
         return MIFI_ERROR;
     return vinterp_device(h, true, inType, d_in, or_none(d_cols), nxy, nt, badValue, outType, d_out, as_stream(stream)) == FB_OK ? MIFI_OK
                                                                                                                                   : MIFI_ERROR;
+}
+
+int fb200_vconvert_create(int op, int vcoord, const double* a, const double* b, int nk, double ptop, double ps_scale, fb200_vconvert** handle)
+{
+    return vconvert_create(op, vcoord, a, b, nk, ptop, ps_scale, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+void fb200_vconvert_destroy(fb200_vconvert* h)
+{
+    delete h;
+}
+
+int fb200_vconvert_values(const fb200_vconvert* h, const float* in, const fb200_vcolumns* cols, size_t nxy, size_t nt, float* out)
+{
+    if (check_vconvert_call(h, in, or_none(cols), nxy, nt, out) != FB_OK)
+        return MIFI_ERROR;
+    return vconvert_host(h, in, or_none(cols), nxy, nt, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_vconvert_values_device(const fb200_vconvert* h, const float* d_in, const fb200_vcolumns* d_cols, size_t nxy, size_t nt, float* d_out,
+                                 void* stream)
+{
+    if (check_vconvert_call(h, d_in, or_none(d_cols), nxy, nt, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return vconvert_device(h, d_in, or_none(d_cols), nxy, nt, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
 }
 
 // ---------------------------------------------------------------------------------------- mifi_* drop-ins

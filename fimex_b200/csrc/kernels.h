@@ -169,5 +169,12 @@ int launch_vertical_height(const VertTable& vt, const float* d_in, const float* 
 // depth handles: in [nt][nk][nxy], eta [nt][nxy] (null: 0), depth [nxy] (null for depth levels), out [nt][np][nxy]
 int launch_vertical_depth(const VertTable& vt, const float* d_in, const float* d_eta, const float* d_depth, long long nxy, long long nt, float* d_out,
                           cudaStream_t st);
+// data conversions, numbered as FB200_VCONV_* (include/fimex_b200.h); source coordinates FB200_VCOORD_PRESSURE, _HYBRID, _SIGMA
+enum { FB_VCONV_THETA2T = 0, FB_VCONV_OMEGA2VWIND = 1, FB_VCONV_PRESSURE = 2 };
+enum { FB_VCOORD_PRESSURE = 0, FB_VCOORD_HYBRID = 1, FB_VCOORD_SIGMA = 2 };
+// vt: a[nk] | b[nk], ps_scale, shift and H of a pressure or height handle (np = 0).  in [nt][nk][nxy] (theta or omega; null for
+// FB_VCONV_PRESSURE), ps [nt][nxy] (null for pressure levels), t [nt][nk][nxy] (omega2vwind), out [nt][nk][nxy]; d_out == d_in is allowed
+int launch_vconvert(int op, int vcoord, const VertTable& vt, double kappa, const float* d_in, const float* d_ps, const float* d_t, long long nxy,
+                    long long nt, float* d_out, cudaStream_t st);
 
 } // namespace fb

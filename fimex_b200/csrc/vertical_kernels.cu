@@ -438,6 +438,52 @@ __global__ void __launch_bounds__(kThreads, 3)
     }
 }
 
+// The data conversions of the vertical interpolator (CDMPressureConversions: theta2T, omega2vwind, add4Dpressure) on [nt][nk][nxy]
+// fields, one thread per column and time step, level by level: every level row is a coalesced load and store.  p_k as the pressure
+// handles form it (a, b and the shift of a VertTable), evaluated where it is needed and never stored except as add4Dpressure's output.
+// in [nt][nk][nxy] (theta or omega; unused for FB_VCONV_PRESSURE), ps [nt][nxy] (null for pressure levels), tt [nt][nk][nxy]
+// (omega2vwind), out [nt][nk][nxy].  in and out may be the same array, so neither is __restrict__ nor read through the texture path.
+// tab: a[nk] | b[nk]; pressure levels: the factor (p_k / p0)^kappa of every level is formed once per block in s_tab[nk .. 2 nk)
+template <int OP, int VC>
+__global__ void __launch_bounds__(kThreads)
+    k_vconvert(const float* in, const float* __restrict__ ps, const float* tt, float* out, const double* __restrict__ tab, int nk,
+               double ps_scale, double shift, double kappa, double H, long long nxy, long long t0)
+{
+    extern __shared__ double s_tab[];
+    for (int i = threadIdx.x; i < 2 * nk; i += blockDim.x)
+        s_tab[i] = tab[i];
+    __syncthreads();
+    const double* s_a = s_tab;
+    const double* s_b = s_tab + nk;
+    if (OP == FB_VCONV_THETA2T && VC == FB_VCOORD_PRESSURE) {
+        for (int k = threadIdx.x; k < nk; k += blockDim.x)
+            s_tab[nk + k] = vexp(__dmul_rn(kappa, vlog(s_a[k] / 1000.0)));
+        __syncthreads();
+    }
+
+    const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (c >= nxy)
+        return;
+    const long long t = t0 + blockIdx.y;
+    const long long base = t * nk * nxy + c;
+    const double q = VC == FB_VCOORD_PRESSURE ? 0.0 : __dmul_rn((double)__ldg(ps + t * nxy + c), ps_scale) - shift;
+#pragma unroll 4
+    for (int k = 0; k < nk; ++k) {
+        const long long i = base + (long long)k * nxy;
+        const double p = VC == FB_VCOORD_PRESSURE ? s_a[k] : s_a[k] + __dmul_rn(s_b[k], q);
+        double r;
+        if (OP == FB_VCONV_THETA2T) {
+            const double f = VC == FB_VCOORD_PRESSURE ? s_b[k] : vexp(__dmul_rn(kappa, vlog(p / 1000.0)));
+            r = __dmul_rn((double)in[i], f);
+        } else if (OP == FB_VCONV_OMEGA2VWIND) {
+            r = -__dmul_rn((double)in[i], __dmul_rn(H, (double)tt[i])) / __dmul_rn(100.0, p);
+        } else {
+            r = p;
+        }
+        __stcs(out + i, (float)r);
+    }
+}
+
 } // namespace
 
 int launch_vert_coords(int method, const double* d_lev, double* d_x, int np, cudaStream_t st)
@@ -540,6 +586,41 @@ int launch_vertical_depth(const VertTable& vt, const float* d_in, const float* d
 #undef FB_CASE
         default:
             FB_REQUIRE(false, "unknown depth coordinate / method " + std::to_string(vt.depth_vcoord) + " / " + std::to_string(vt.method));
+        }
+        count_launch();
+        FB_CUDA_CHECK(cudaGetLastError());
+    }
+    return FB_OK;
+}
+
+int launch_vconvert(int op, int vcoord, const VertTable& vt, double kappa, const float* d_in, const float* d_ps, const float* d_t, long long nxy,
+                    long long nt, float* d_out, cudaStream_t st)
+{
+    if (nxy == 0 || nt == 0)
+        return FB_OK;
+    const size_t smem = sizeof(double) * (size_t)(2 * vt.nk);
+    const long long bx = (nxy + kThreads - 1) / kThreads;
+    FB_REQUIRE(bx < 2147483647LL, "too many columns for one call");
+    const int key = op * 8 + vcoord;
+    for (long long t0 = 0; t0 < nt; t0 += 65535) {
+        const dim3 grid((unsigned)bx, (unsigned)std::min<long long>(nt - t0, 65535));
+        switch (key) {
+#define FB_CASE(O, V)                                                                                                                      \
+    case O * 8 + V:                                                                                                                        \
+        k_vconvert<O, V><<<grid, kThreads, smem, st>>>(d_in, d_ps, d_t, d_out, vt.d_tab, vt.nk, vt.ps_scale, vt.shift, kappa, vt.H, nxy, t0); \
+        break;
+            FB_CASE(FB_VCONV_THETA2T, FB_VCOORD_PRESSURE)
+            FB_CASE(FB_VCONV_THETA2T, FB_VCOORD_HYBRID)
+            FB_CASE(FB_VCONV_THETA2T, FB_VCOORD_SIGMA)
+            FB_CASE(FB_VCONV_OMEGA2VWIND, FB_VCOORD_PRESSURE)
+            FB_CASE(FB_VCONV_OMEGA2VWIND, FB_VCOORD_HYBRID)
+            FB_CASE(FB_VCONV_OMEGA2VWIND, FB_VCOORD_SIGMA)
+            FB_CASE(FB_VCONV_PRESSURE, FB_VCOORD_PRESSURE)
+            FB_CASE(FB_VCONV_PRESSURE, FB_VCOORD_HYBRID)
+            FB_CASE(FB_VCONV_PRESSURE, FB_VCOORD_SIGMA)
+#undef FB_CASE
+        default:
+            FB_REQUIRE(false, "unknown data conversion / source coordinate " + std::to_string(op) + " / " + std::to_string(vcoord));
         }
         count_launch();
         FB_CUDA_CHECK(cudaGetLastError());

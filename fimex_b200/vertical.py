@@ -10,7 +10,8 @@ The source vertical coordinate is given by its CF standard name and formula term
 The surface pressure ``ps`` is not a term here: it is a field, passed with every slice.  All pressures are in the unit of the
 target levels (hPa, as the reference's level1 option); ``ps_scale`` converts the ``ps`` field to it (0.01 for Pa).  Height and
 altitude levels are in metres (:class:`HeightInterpolator`), as are depth levels below the sea surface (:class:`DepthInterpolator`, from
-depth levels or the CF ocean sigma and s-coordinates).  The arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md
+depth levels or the CF ocean sigma and s-coordinates).  :class:`PressureConversion` runs the data conversions on the model
+levels (theta2T, omega2vwind, add4Dpressure) on the same column pressures.  The arithmetic runs in libfimex_b200.so on the GPU (DESIGN.md
 section 2 states it).
 """
 from __future__ import annotations
@@ -75,14 +76,15 @@ def _source_levels(standard_name: str, terms: dict):
 
 
 class _VerticalHandle:
-    """Lifetime of an fb200_vinterp handle and the shape checks of its calls."""
+    """Lifetime of an fb200_vinterp (or fb200_vconvert) handle and the shape checks of its calls."""
 
     nk = 0
     needs_ps = False
+    _destroy = "fb200_vinterp_destroy"
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h:
-            load().fb200_vinterp_destroy(self._h)
+            getattr(load(), self._destroy)(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):
@@ -384,3 +386,81 @@ class DepthInterpolator(_VerticalHandle):
         `bad_value` = CDM::getFillValue of the variable (default: the type's default fill value)."""
         return self._slice_columns(field, None, lambda nt, nxy, device: self._columns(nt, nxy, device, eta, depth), bad_value, out_dtype,
                                    stream)
+
+
+#: --verticalInterpolate.dataConversion values -> FB200_VCONV_*
+CONVERSIONS = {"theta2T": 0, "omega2vwind": 1, "add4Dpressure": 2}
+
+
+class PressureConversion(_VerticalHandle):
+    """The data conversions of the vertical interpolator on the model levels (``--verticalInterpolate.dataConversion``, the
+    reference's CDMPressureConversions), each on the column pressure p_k [hPa] of the source vertical coordinate (terms as for
+    :class:`VerticalInterpolator`; ``ps_scale`` converts ``ps`` to hPa):
+
+    * ``"theta2T"``: air potential temperature -> air temperature, ``T = theta (p_k / 1000)^(2/7)`` [K];
+    * ``"omega2vwind"``: omega [Pa/s] and the air temperature ``t`` [K] -> upward air velocity ``w = -omega R_d T / (g0 p_k)`` [m/s];
+    * ``"add4Dpressure"``: the pressure field p_k itself [hPa], [nt][nk][...]; there is no input field.
+
+    Float32 in, float32 out; numpy arrays (host buffers) or CUDA tensors (device-resident, on ``stream``)."""
+
+    _destroy = "fb200_vconvert_destroy"
+
+    def __init__(self, standard_name: str, terms: dict, operation: str, ps_scale: float = 1.0):
+        if operation not in CONVERSIONS:
+            raise FimexB200Error(f"unknown data conversion: '{operation}' (one of {', '.join(CONVERSIONS)})")
+        self.operation = operation
+        self._h = C.c_void_p()
+        vcoord, a, b, ptop, self.nk = _source_levels(standard_name, terms)
+        self.needs_ps = vcoord != VCOORD_PRESSURE
+        self.needs_t = operation == "omega2vwind"
+        check(load().fb200_vconvert_create(CONVERSIONS[operation], vcoord, ptr(a), ptr(b), self.nk, ptop, float(ps_scale), C.byref(self._h)),
+              "PressureConversion")
+
+    def convert(self, field=None, ps=None, t=None, nt=None, stream=None):
+        """``field`` [nt][nk][...] (theta or omega; None for add4Dpressure), ``ps`` [nt][...] (hybrid and sigma levels), ``t``
+        [nt][nk][...] (omega2vwind) -> float32 [nt][nk][...].  add4Dpressure takes its shape from ``ps``, or on pressure levels from
+        ``nt``: [nt][nk]."""
+        pressure = self.operation == "add4Dpressure"
+        if pressure:
+            if ps is not None:
+                nt_, nxy, rest = int(ps.shape[0]), int(np.prod(ps.shape[1:], dtype=np.int64)), tuple(ps.shape[1:])
+            elif self.needs_ps:
+                raise FimexB200Error("this vertical coordinate needs the surface pressure ps")
+            elif nt is None:
+                raise FimexB200Error("add4Dpressure on pressure levels needs nt")
+            else:
+                nt_, nxy, rest = int(nt), 1, ()
+            device = _is_torch(ps)
+        else:
+            if field is None:
+                raise FimexB200Error(f"{self.operation} needs the field")
+            device = _is_torch(field)
+            if field.ndim < 2 or field.shape[1] != self.nk:
+                raise FimexB200Error(f"field must be [nt][{self.nk}][...], got shape {tuple(field.shape)}")
+            nt_, nxy, rest = int(field.shape[0]), int(np.prod(field.shape[2:], dtype=np.int64)), tuple(field.shape[2:])
+        slots = {}
+        if self.needs_ps:
+            if ps is None:
+                raise FimexB200Error("this vertical coordinate needs the surface pressure ps")
+            slots["ps"] = ("ps", ps, nt_ * nxy)
+        if self.needs_t:
+            if t is None:
+                raise FimexB200Error("omega2vwind needs the air temperature t")
+            slots["t"] = ("t", t, nt_ * self.nk * nxy)
+        cols, keep = _fill_columns(slots, device)
+        shape = (nt_, self.nk) + rest
+        lib = load()
+        if device:
+            import torch
+            d_in = None
+            if not pressure:
+                if not field.is_cuda or field.dtype != torch.float32 or not field.is_contiguous():
+                    raise FimexB200Error("device path needs a contiguous float32 CUDA tensor")
+                d_in = field
+            out = torch.empty(shape, dtype=torch.float32, device=ps.device if pressure else field.device)
+            check(lib.fb200_vconvert_values_device(self._h, ptr(d_in), C.byref(cols), nxy, nt_, ptr(out), _stream_ptr(stream)), "convert")
+            return out
+        a = None if pressure else capi.f32(field)
+        out = np.empty(shape, dtype=np.float32)
+        check(lib.fb200_vconvert_values(self._h, ptr(a), C.byref(cols), nxy, nt_, ptr(out)), "convert")
+        return out

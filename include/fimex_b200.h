@@ -398,6 +398,32 @@ int fb200_vinterp_create_depth(int method, int vcoord, const double* s, const do
                                int extrapolate, fb200_vinterp** handle);
 
 /* ------------------------------------------------------------------------------------------------
+ * (1g) the data conversions of the vertical interpolator on the model levels (--verticalInterpolate.dataConversion, the reference's
+ *      CDMPressureConversions; DESIGN.md section 2 states the arithmetic)
+ *
+ *   FB200_VCONV_THETA2T      air_potential_temperature theta [K] -> air_temperature T = theta * (p_k / 1000 hPa)^(2/7) [K]
+ *   FB200_VCONV_OMEGA2VWIND  lagrangian_tendency_of_air_pressure omega [Pa/s] and air_temperature T [K] -> upward_air_velocity
+ *                            w = -omega R_d T / (g0 p_k) [m/s], R_d = R* / M
+ *   FB200_VCONV_PRESSURE     add4Dpressure: the column pressure p_k itself [hPa], an [nt][nk][nxy] field; no input field
+ * vcoord, a, b, ptop and ps_scale give p_k [hPa] as for fb200_vinterp_create_height: FB200_VCOORD_PRESSURE (a = the levels), _HYBRID
+ * (a = ap, b) or _SIGMA (b = sigma, ptop).  1 <= nk <= 1024, all values finite.  Float in, float out; NaN in the field, t or ps gives
+ * NaN for the values it enters.  The handle is immutable and every call re-entrant, as for the other handles.
+ * ---------------------------------------------------------------------------------------------- */
+#define FB200_VCONV_THETA2T 0
+#define FB200_VCONV_OMEGA2VWIND 1
+#define FB200_VCONV_PRESSURE 2
+typedef struct fb200_vconvert fb200_vconvert; /* opaque */
+
+int fb200_vconvert_create(int op, int vcoord, const double* a, const double* b, int nk, double ptop, double ps_scale, fb200_vconvert** handle);
+void fb200_vconvert_destroy(fb200_vconvert* handle);
+/* in: [nt][nk][nxy] float (theta or omega; NULL for FB200_VCONV_PRESSURE); cols->ps [nt][nxy] (hybrid and sigma levels), cols->t
+ * [nt][nk][nxy] (omega2vwind); the other slots are not read.  out: [nt][nk][nxy] float.  Host buffers (copies pipelined over the time
+ * steps) or, for _device, device pointers on `cuda_stream` without synchronisation.  The _device form may run in place (d_out == d_in). */
+int fb200_vconvert_values(const fb200_vconvert* handle, const float* in, const fb200_vcolumns* cols, size_t nxy, size_t nt, float* out);
+int fb200_vconvert_values_device(const fb200_vconvert* handle, const float* d_in, const fb200_vcolumns* d_cols, size_t nxy, size_t nt,
+                                 float* d_out, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
  * ---------------------------------------------------------------------------------------------- */
 int mifi_string_to_interpolation_method(const char* stringMethod); /* :44 */
