@@ -55,9 +55,155 @@ constexpr int kCells = FB_FWD_CELLS; // target cells per thread: their first gat
                           // a second table with the first input index of every cell, read next to the offsets, shortens the chain to
                           // two loads but adds 72 MB of table traffic per slice: 0.093 ms instead of 0.081 (mean), 0.090 / 0.078 (max)
 
-// one target cell: aggregate its CSR segment [beg, end) in ascending input order; v0 = value of the first entry (prefetched)
+// std::nth_element(first, first + nth, first + n) with operator<, restated from libstdc++ (bits/stl_algo.h __introselect and its
+// helpers, bits/stl_heap.h); the same comparisons and moves as oracle/mifi_oracle.c's orc_nth_element.  Only segments whose result
+// depends on the algorithm come here (NaN, or both signs of zero): one thread works through its own copy of the segment.
+namespace nth {
+__device__ __forceinline__ void swapf(float* a, float* b)
+{
+    const float t = *a;
+    *a = *b;
+    *b = t;
+}
+
+__device__ void push_heap(float* v, long long hole, long long top, float value)
+{
+    long long parent = (hole - 1) / 2;
+    while (hole > top && v[parent] < value) {
+        v[hole] = v[parent];
+        hole = parent;
+        parent = (hole - 1) / 2;
+    }
+    v[hole] = value;
+}
+
+__device__ void adjust_heap(float* v, long long hole, long long len, float value)
+{
+    const long long top = hole;
+    long long child = hole;
+    while (child < (len - 1) / 2) {
+        child = 2 * (child + 1);
+        if (v[child] < v[child - 1])
+            child--;
+        v[hole] = v[child];
+        hole = child;
+    }
+    if ((len & 1) == 0 && child == (len - 2) / 2) {
+        child = 2 * (child + 1);
+        v[hole] = v[child - 1];
+        hole = child - 1;
+    }
+    push_heap(v, hole, top, value);
+}
+
+__device__ void heap_select(float* first, float* middle, float* last)
+{
+    const long long len = middle - first;
+    if (len >= 2) {
+        for (long long parent = (len - 2) / 2;; parent--) {
+            adjust_heap(first, parent, len, first[parent]);
+            if (parent == 0)
+                break;
+        }
+    }
+    for (float* i = middle; i < last; ++i)
+        if (*i < *first) {
+            const float value = *i;
+            *i = *first;
+            adjust_heap(first, 0, len, value);
+        }
+}
+
+__device__ void insertion_sort(float* first, float* last)
+{
+    if (first == last)
+        return;
+    for (float* i = first + 1; i != last; ++i) {
+        const float val = *i;
+        if (val < *first) {
+            for (float* p = i; p != first; --p)
+                *p = *(p - 1);
+            *first = val;
+        } else {
+            float* hole = i;
+            float* next = i - 1;
+            while (val < *next) {
+                *hole = *next;
+                hole = next;
+                --next;
+            }
+            *hole = val;
+        }
+    }
+}
+
+__device__ void move_median_to_first(float* result, float* a, float* b, float* c)
+{
+    if (*a < *b) {
+        if (*b < *c)
+            swapf(result, b);
+        else if (*a < *c)
+            swapf(result, c);
+        else
+            swapf(result, a);
+    } else if (*a < *c)
+        swapf(result, a);
+    else if (*b < *c)
+        swapf(result, c);
+    else
+        swapf(result, b);
+}
+
+__device__ float* unguarded_partition_pivot(float* first, float* last)
+{
+    float* mid = first + (last - first) / 2;
+    move_median_to_first(first, first + 1, mid, last - 1);
+    float* lo = first + 1;
+    float* hi = last;
+    for (;;) {
+        while (*lo < *first)
+            ++lo;
+        --hi;
+        while (*first < *hi)
+            --hi;
+        if (!(lo < hi))
+            return lo;
+        swapf(lo, hi);
+        ++lo;
+    }
+}
+
+__device__ void nth_element(float* first, long long nth_index, long long n)
+{
+    float* last = first + n;
+    float* nth = first + nth_index;
+    if (first == last || nth == last)
+        return;
+    int depth_limit = 0; // std::__lg(n) * 2
+    for (long long m = n; m > 1; m >>= 1)
+        depth_limit += 2;
+    while (last - first > 3) {
+        if (depth_limit == 0) {
+            heap_select(first, nth + 1, last);
+            swapf(first, nth);
+            return;
+        }
+        --depth_limit;
+        float* cut = unguarded_partition_pivot(first, last);
+        if (cut <= nth)
+            first = cut;
+        else
+            last = cut;
+    }
+    insertion_sort(first, last);
+}
+} // namespace nth
+
+// one target cell: aggregate its CSR segment [beg, end) in ascending input order; v0 = value of the first entry (prefetched).
+// scr (median only): this level's scratch, one float per mapped point; the cell may use scr[beg, end).
 template <int AGG, bool UNDEF>
-__device__ __forceinline__ float aggregate_cell(const float* __restrict__ lv, const int* __restrict__ perm, int beg, int end, float v0)
+__device__ __forceinline__ float aggregate_cell(const float* __restrict__ lv, const int* __restrict__ perm, int beg, int end, float v0,
+                                                float* __restrict__ scr)
 {
     float res = undef_f();
     if (beg >= end)
@@ -98,14 +244,28 @@ __device__ __forceinline__ float aggregate_cell(const float* __restrict__ lv, co
         }
         if (have)
             res = best;
-    } else { // median = sorted[n/2] (nth_element, :49-53); rank selection, O(n^2) but segments are short
+    } else { // median = v[n/2] after nth_element(v.begin(), v.begin() + n/2, v.end()) (:49-53)
         long long cnt = 0;
+        bool has_nan = false, has_pz = false, has_nz = false;
         for (int k = beg; k < end; ++k) {
             const float v = __ldg(lv + __ldg(perm + k));
-            if (UNDEF || !isnan(v))
+            if (UNDEF || !isnan(v)) {
                 ++cnt;
+                has_nan |= isnan(v);
+                has_pz |= (v == 0.f && !signbit(v));
+                has_nz |= (v == 0.f && signbit(v));
+            }
         }
-        if (cnt > 0) {
+        if (has_nan || (has_pz && has_nz)) { // < is no strict weak order here, or equal elements differ in their bits
+            long long m = 0;
+            for (int k = beg; k < end; ++k) {
+                const float v = __ldg(lv + __ldg(perm + k));
+                if (UNDEF || !isnan(v))
+                    scr[beg + m++] = v;
+            }
+            nth::nth_element(scr + beg, cnt / 2, cnt);
+            res = scr[beg + cnt / 2];
+        } else if (cnt > 0) { // every element equal to the median has the same bits: rank selection, O(n^2) but segments are short
             const long long want = cnt / 2;
             for (int k = beg; k < end; ++k) {
                 const float v = __ldg(lv + __ldg(perm + k));
@@ -190,7 +350,8 @@ __device__ __forceinline__ void aggregate_cell_levels(const float* __restrict__ 
 template <int AGG, bool UNDEF, int ZL>
 __global__ void __launch_bounds__(kThreads) k_forward(const int* __restrict__ perm, const int* __restrict__ offsets,
                                                     const float* __restrict__ in, float* __restrict__ out, long long n_in,
-                                                    long long n_cells, long long nz, int vec_ok)
+                                                    long long n_cells, long long nz, int vec_ok, float* __restrict__ scratch,
+                                                    long long scratch_stride)
 {
     const long long c0 = (blockIdx.x * (long long)kThreads + threadIdx.x) * kCells;
     if (c0 >= n_cells)
@@ -211,6 +372,8 @@ __global__ void __launch_bounds__(kThreads) k_forward(const int* __restrict__ pe
 #pragma unroll
     for (int j = 0; j < kCells; ++j)
         first[j] = off[j] < off[j + 1] ? __ldg(perm + off[j]) : -1; // the same for every level
+    // the median's scratch: one slot of n_mapped floats per blockIdx.y, which works through its levels one after another
+    float* scr = AGG == AG_MEDIAN ? scratch + (long long)blockIdx.y * scratch_stride : nullptr;
     const long long valid = n_cells - c0;
     auto store = [&](long long z, const float (&res)[kCells]) {
         float* o = out + z * n_cells + c0;
@@ -256,11 +419,14 @@ __global__ void __launch_bounds__(kThreads) k_forward(const int* __restrict__ pe
                 v0[j] = first[j] >= 0 ? __ldg(lv + first[j]) : 0.f; // kCells independent gathers in flight
 #pragma unroll
             for (int j = 0; j < kCells; ++j)
-                res[j] = aggregate_cell<AGG, UNDEF>(lv, perm, off[j], off[j + 1], v0[j]);
+                res[j] = aggregate_cell<AGG, UNDEF>(lv, perm, off[j], off[j + 1], v0[j], scr);
             store(zz, res);
         }
     }
 }
+
+// the median's scratch is at most this many bytes: config 5 (10 M points) would need 2.5 GB for 64 levels at once
+constexpr size_t kMedianScratchBytes = 256u << 20;
 
 template <int AGG>
 int launch_agg(bool undef, int gx, cudaStream_t st, const ForwardPlan& p, const float* in, float* out, long long nz)
@@ -270,15 +436,28 @@ int launch_agg(bool undef, int gx, cudaStream_t st, const ForwardPlan& p, const 
         const long long passes = (nz + 3) / 4;
         dim3 grid(gx, (unsigned)(passes < 64 ? passes : 64));
         if (undef)
-            k_forward<AGG, true, 4><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok);
+            k_forward<AGG, true, 4><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok, nullptr, 0);
         else
-            k_forward<AGG, false, 4><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok);
+            k_forward<AGG, false, 4><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok, nullptr, 0);
     } else {
-        dim3 grid(gx, (unsigned)(nz < 64 ? nz : 64));
+        long long gy = nz < 64 ? nz : 64;
+        float* scratch = nullptr;
+        const long long stride = p.n_mapped > 0 ? p.n_mapped : 1;
+        if (AGG == AG_MEDIAN) { // one scratch slot per blockIdx.y: fewer levels at once when the slots would not fit
+            const long long fit = (long long)(kMedianScratchBytes / (sizeof(float) * (size_t)stride));
+            gy = gy < fit ? gy : (fit > 1 ? fit : 1);
+            FB_CUDA_CHECK(cudaMallocAsync(&scratch, sizeof(float) * (size_t)(stride * gy), st));
+        }
+        dim3 grid(gx, (unsigned)gy);
         if (undef)
-            k_forward<AGG, true, 1><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok);
+            k_forward<AGG, true, 1><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok, scratch, stride);
         else
-            k_forward<AGG, false, 1><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok);
+            k_forward<AGG, false, 1><<<grid, kThreads, 0, st>>>(p.d_perm, p.d_offsets, in, out, p.n_in, p.n_cells, nz, vec_ok, scratch, stride);
+        if (scratch) {
+            const cudaError_t e = cudaGetLastError();
+            cudaFreeAsync(scratch, st);
+            FB_CUDA_CHECK(e);
+        }
     }
     count_launch();
     FB_CUDA_CHECK(cudaGetLastError());

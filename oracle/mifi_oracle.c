@@ -19,6 +19,7 @@
  */
 #include "shim/proj_api.h"
 
+#include <stddef.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -705,10 +706,148 @@ void orc_round_and_clamp(const double* pos, size_t n, int maxi, int* idx)
     }
 }
 
-static int orc_cmp_float(const void* a, const void* b)
+/* std::nth_element(first, nth, last) on floats with operator<, restated from libstdc++'s bits/stl_algo.h (__introselect,
+ * __unguarded_partition_pivot, __move_median_to_first, __insertion_sort, __heap_select) and bits/stl_heap.h (__make_heap,
+ * __adjust_heap, __push_heap, __pop_heap).  The C++ standard leaves the result undefined when the range holds NaN (< is then
+ * no strict weak order) and does not say which of several equal elements lands at nth (+0 == -0); this restatement makes
+ * the same comparisons and moves in the same order as that library, so it picks the same element bit for bit. */
+static void orc_swapf(float* a, float* b)
 {
-    const float x = *(const float*)a, y = *(const float*)b;
-    return (x > y) - (x < y);
+    const float t = *a;
+    *a = *b;
+    *b = t;
+}
+
+static void orc_push_heap(float* v, ptrdiff_t hole, ptrdiff_t top, float value)
+{
+    ptrdiff_t parent = (hole - 1) / 2;
+    while (hole > top && v[parent] < value) {
+        v[hole] = v[parent];
+        hole = parent;
+        parent = (hole - 1) / 2;
+    }
+    v[hole] = value;
+}
+
+static void orc_adjust_heap(float* v, ptrdiff_t hole, ptrdiff_t len, float value)
+{
+    const ptrdiff_t top = hole;
+    ptrdiff_t child = hole;
+    while (child < (len - 1) / 2) {
+        child = 2 * (child + 1);
+        if (v[child] < v[child - 1])
+            child--;
+        v[hole] = v[child];
+        hole = child;
+    }
+    if ((len & 1) == 0 && child == (len - 2) / 2) {
+        child = 2 * (child + 1);
+        v[hole] = v[child - 1];
+        hole = child - 1;
+    }
+    orc_push_heap(v, hole, top, value);
+}
+
+static void orc_heap_select(float* first, float* middle, float* last)
+{
+    const ptrdiff_t len = middle - first;
+    if (len >= 2) { /* __make_heap */
+        for (ptrdiff_t parent = (len - 2) / 2;; parent--) {
+            orc_adjust_heap(first, parent, len, first[parent]);
+            if (parent == 0)
+                break;
+        }
+    }
+    for (float* i = middle; i < last; ++i)
+        if (*i < *first) { /* __pop_heap(first, middle, i) */
+            const float value = *i;
+            *i = *first;
+            orc_adjust_heap(first, 0, len, value);
+        }
+}
+
+static void orc_insertion_sort(float* first, float* last)
+{
+    if (first == last)
+        return;
+    for (float* i = first + 1; i != last; ++i) {
+        const float val = *i;
+        if (val < *first) {
+            memmove(first + 1, first, sizeof(float) * (size_t)(i - first));
+            *first = val;
+        } else { /* __unguarded_linear_insert */
+            float* hole = i;
+            float* next = i - 1;
+            while (val < *next) {
+                *hole = *next;
+                hole = next;
+                --next;
+            }
+            *hole = val;
+        }
+    }
+}
+
+static void orc_move_median_to_first(float* result, float* a, float* b, float* c)
+{
+    if (*a < *b) {
+        if (*b < *c)
+            orc_swapf(result, b);
+        else if (*a < *c)
+            orc_swapf(result, c);
+        else
+            orc_swapf(result, a);
+    } else if (*a < *c)
+        orc_swapf(result, a);
+    else if (*b < *c)
+        orc_swapf(result, c);
+    else
+        orc_swapf(result, b);
+}
+
+static float* orc_unguarded_partition_pivot(float* first, float* last)
+{
+    float* mid = first + (last - first) / 2;
+    orc_move_median_to_first(first, first + 1, mid, last - 1);
+    float* lo = first + 1;
+    float* hi = last;
+    const float* pivot = first;
+    for (;;) {
+        while (*lo < *pivot)
+            ++lo;
+        --hi;
+        while (*pivot < *hi)
+            --hi;
+        if (!(lo < hi))
+            return lo;
+        orc_swapf(lo, hi);
+        ++lo;
+    }
+}
+
+void orc_nth_element(float* first, size_t nth_index, size_t n)
+{
+    float* last = first + n;
+    float* nth = first + nth_index;
+    if (first == last || nth == last)
+        return;
+    int depth_limit = 0; /* std::__lg(n) * 2 */
+    for (size_t m = n; m > 1; m >>= 1)
+        depth_limit += 2;
+    while (last - first > 3) {
+        if (depth_limit == 0) {
+            orc_heap_select(first, nth + 1, last);
+            orc_swapf(first, nth);
+            return;
+        }
+        --depth_limit;
+        float* cut = orc_unguarded_partition_pivot(first, last);
+        if (cut <= nth)
+            first = cut;
+        else
+            last = cut;
+    }
+    orc_insertion_sort(first, last);
 }
 
 static float orc_aggregate(int method, float* v, size_t n)
@@ -727,7 +866,7 @@ static float orc_aggregate(int method, float* v, size_t n)
     }
     case ORC_FWD_MEDIAN:
     case ORC_FWD_UNDEF_MEDIAN:
-        qsort(v, n, sizeof(float), orc_cmp_float); /* nth_element(...)[n/2] == sorted[n/2] (:49-53) */
+        orc_nth_element(v, n / 2, n); /* nth_element(v.begin(), v.begin() + n/2, v.end()); v[n/2] (:49-53) */
         return v[n / 2];
     case ORC_FWD_MAX:
     case ORC_FWD_UNDEF_MAX: {

@@ -274,6 +274,16 @@ class Oracle(_Base):
             raise RuntimeError("orc_forward_interpolate failed")
         return out.reshape(inZ, outY, outX)
 
+    def nth_element(self, values, nth):
+        """the restated std::nth_element(v, v + nth, v + n) of the forward median on a float32 copy; returns the copy"""
+        a, ap = _f(np.array(values, dtype=np.float32, copy=True))
+        f = self.lib.orc_nth_element
+        f.restype = None
+        f.argtypes = [_fp, C.c_size_t, C.c_size_t]
+        if a.size:
+            f(ap, int(nth), a.size)
+        return a
+
     def bad2nan(self, data, bad):
         a, ap = _f(np.array(data, dtype=np.float32, copy=True))
         f = self.lib.orc_bad2nan

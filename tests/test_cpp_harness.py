@@ -4,6 +4,7 @@ test/testInterpolation.cc cases restated.  Compiling and linking against libfime
 needs a GPU."""
 import os
 import subprocess
+import tempfile
 
 import pytest
 
@@ -11,7 +12,8 @@ from fimex_b200 import capi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "tests", "cpp", "testInterpolation_b200.cc")
-EXE = os.path.join(ROOT, "tests", "cpp", "testInterpolation_b200")
+# built outside the repository tree, which may be read-only where the suite runs
+EXE = os.path.join(tempfile.gettempdir(), f"fimex_b200_testInterpolation_b200_{os.getuid()}_{os.getpid()}")
 
 
 def _build():

@@ -387,3 +387,19 @@ def test_fill2d_and_creepfill2d_against_reference(oracle, reference, shape):
     assert np.array_equal(oracle.fill2d(full, 0.01, 1.6, 100)[0], full)
     allnan = np.full(shape, np.nan, dtype=np.float32)
     assert np.isnan(oracle.creepfill2d(allnan, 20, 2)[0]).all()
+
+
+@pytest.mark.parametrize("nx,ny", [(799, 799), (800, 800), (1600, 1599), (1000, 1000), (1200, 900), (900, 1200), (2000, 2000), (30, 700),
+                                   (700, 30)])
+def test_fill2d_and_creepfill2d_against_reference_at_kernel_switch_shapes(oracle, reference, nx, ny):
+    """the shapes at which tests/test_gpu_forward_fill_fuzz.py compares the device kernels with the restatement: the restatement
+    against the compiled reference there too, one parameter set per process (a negative char weight for creepfillval2d)"""
+    rng = np.random.default_rng(nx * 3 + ny)
+    f = _holey_field(rng, (1, ny, nx), 0.1)
+    got, n1 = oracle.fill2d(f, 0.01, 1.6, 100)
+    want, n2 = oracle.fill2d(f, 0.01, 1.6, 100, lib=reference.lib, name="mifi_fill2d_f")
+    assert n1 == n2 and np.array_equal(got.view(np.uint32), want.view(np.uint32))
+    for repeat, weight, dv in ((20, 2, None), (5, 200, -3.5)):
+        got, n1 = oracle.creepfill2d(f, repeat, weight, dv)
+        want, n2 = oracle.creepfill2d(f, repeat, weight, dv, lib=reference.lib, prefix="ref")
+        assert n1 == n2 and np.array_equal(got.view(np.uint32), want.view(np.uint32)), (repeat, weight, dv)
