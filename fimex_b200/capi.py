@@ -189,6 +189,12 @@ def _declare(lib):
         "fb200_vconvert_destroy": (None, [_vp]),
         "fb200_vconvert_values": (i, [_vp, _vp, _vp, sz, sz, _vp]),
         "fb200_vconvert_values_device": (i, [_vp, _vp, _vp, sz, sz, _vp, _vp]),
+        "fb200_tinterp_create": (i, [_vp, i, _vp, i, i, P(_vp)]),
+        "fb200_tinterp_destroy": (None, [_vp]),
+        "fb200_tinterp_source_steps": (i, [_vp, i, P(i), P(i), P(C.c_double)]),
+        "fb200_tinterp_get_step": (i, [_vp, i, i, _vp, _vp, sz, C.c_double, i, _vp]),
+        "fb200_tinterp_get_step_device": (i, [_vp, i, i, _vp, _vp, sz, C.c_double, i, _vp, _vp]),
+        "fb200_tinterp_get_data_slice_device": (i, [_vp, i, _vp, sz, C.c_double, i, _vp, _vp]),
         "mifi_string_to_interpolation_method": (i, [C.c_char_p]),
         "mifi_interpolate_f": (i, [i, C.c_char_p, _vp, _vp, _vp, i, i, i, i, i, C.c_char_p, _vp, _vp, _vp, i, i, i, i]),
         "mifi_vector_reproject_values_f": (i, [i, C.c_char_p, C.c_char_p, _vp, _vp, _vp, _vp, i, i, i, i, i]),

@@ -2503,6 +2503,111 @@ int vconvert_host(const fb200_vconvert* h, const float* in, const fb200_vcolumns
 
 } // namespace
 
+// ======================================================================================================
+// time interpolation (CDMTimeInterpolator's linear change of the time axis)
+// ======================================================================================================
+struct fb200_tinterp {
+    int device = 0;
+    int nt = 0, nj = 0;
+    std::vector<TimeStep> map;    // [nj] in target order: lower source step ia (-1: no bracket), weight w
+    TimeStep* d_sorted = nullptr; // [nj] the targets by ia, those without a bracket last: the table of the stack call
+    TimeStep* d_single = nullptr; // [nj] {0 (-1: no bracket), row 0, w_j}: the one-target tables of the step calls
+    ~fb200_tinterp()
+    {
+        fb::DeviceGuard on(device);
+        if (d_sorted)
+            cudaFree(d_sorted);
+        if (d_single)
+            cudaFree(d_single);
+    }
+};
+
+namespace {
+
+constexpr int kMaxTimeTargets = 1 << 20;
+
+int tinterp_create(const double* times, int nt, const double* new_times, int nj, int extrapolate, fb200_tinterp** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(nt >= 2, "number of source times must be at least 2, got " + std::to_string(nt));
+    FB_REQUIRE(nj >= 1 && nj <= kMaxTimeTargets, "number of target times must be in [1, 1048576], got " + std::to_string(nj));
+    FB_REQUIRE(times != nullptr && new_times != nullptr, "null time axis");
+    FB_REQUIRE(all_finite(times, nt) && all_finite(new_times, nj), "times must be finite");
+    for (int k = 0; k + 1 < nt; ++k)
+        FB_REQUIRE(times[k] < times[k + 1], "source times must be strictly increasing");
+    if (use_device(default_device()) != FB_OK)
+        return FB_ERROR;
+    std::unique_ptr<fb200_tinterp> h(new fb200_tinterp());
+    h->device = default_device();
+    h->nt = nt;
+    h->nj = nj;
+    h->map.resize(nj);
+    std::vector<TimeStep> single(nj);
+    for (int j = 0; j < nj; ++j) {
+        const double tau = new_times[j];
+        int k = -1;
+        if (tau < times[0] || tau > times[nt - 1]) {
+            if (extrapolate)
+                k = tau < times[0] ? 0 : nt - 2; // the end pair on that side
+        } else { // the smallest k with t_k <= tau <= t_k+1
+            k = (int)(std::lower_bound(times, times + nt, tau) - times) - 1;
+            k = k < 0 ? 0 : k;
+        }
+        const double w = k < 0 ? 0.0 : (tau - times[k]) / (times[k + 1] - times[k]);
+        h->map[j] = TimeStep{k, j, w};
+        single[j] = TimeStep{k < 0 ? -1 : 0, 0, w};
+    }
+    std::vector<TimeStep> sorted(h->map);
+    std::stable_sort(sorted.begin(), sorted.end(), [](const TimeStep& x, const TimeStep& y) { return (unsigned)x.ia < (unsigned)y.ia; });
+    cudaStream_t st = cudaStreamPerThread;
+    if (dev_alloc(&h->d_sorted, nj) != FB_OK || dev_alloc(&h->d_single, nj) != FB_OK)
+        return FB_ERROR;
+    FB_CUDA_CHECK(cudaMemcpyAsync(h->d_sorted, sorted.data(), sizeof(TimeStep) * nj, cudaMemcpyHostToDevice, st));
+    FB_CUDA_CHECK(cudaMemcpyAsync(h->d_single, single.data(), sizeof(TimeStep) * nj, cudaMemcpyHostToDevice, st));
+    FB_CUDA_CHECK(cudaStreamSynchronize(st));
+    *handle = h.release();
+    return FB_OK;
+}
+
+// stack: the whole-stack call (j is not used); otherwise the step call of target j
+int check_tinterp_call(const fb200_tinterp* h, bool stack, int j, int in_type, int out_type, size_t n, const void* a, const void* b, const void* out)
+{
+    FB_REQUIRE(h != nullptr, "null time interpolation handle");
+    if (check_slice_types(in_type, out_type) != FB_OK)
+        return FB_ERROR;
+    FB_REQUIRE(stack || (j >= 0 && j < h->nj), "target step " + std::to_string(j) + " out of range [0, " + std::to_string(h->nj) + ")");
+    const bool reads = stack || h->map[j].ia >= 0; // a target without a bracket reads no source step
+    FB_REQUIRE(n == 0 || (out && (!reads || (a && b))), "null data pointer");
+    return use_device(h->device);
+}
+
+bool has_bad_value(double bad)
+{
+    return !std::isnan((float)bad); // mifi_bad2nanf takes a float
+}
+
+// host buffers: elements are the units of the staging pipeline; a and b are its inputs (absent for a target without a bracket)
+int tinterp_get_step_host(const fb200_tinterp* h, int j, int in_type, const void* a, const void* b, size_t n, double bad, int out_type, void* out)
+{
+    if (n == 0)
+        return FB_OK;
+    HostArrays arrays;
+    arrays.device = h->device;
+    if (h->map[j].ia >= 0) {
+        arrays.in[0] = a;
+        arrays.in[1] = b;
+        arrays.in_unit[0] = arrays.in_unit[1] = type_size(in_type);
+    }
+    arrays.out[0] = out;
+    arrays.out_unit[0] = type_size(out_type);
+    return stage_host(arrays, n, [&](const void* const* d_in, size_t cnt, void* const* d_out, cudaStream_t s) {
+        return launch_tinterp(in_type, d_in[0], d_in[1], (long long)cnt, has_bad_value(bad), (float)bad, h->d_single + j, 1, out_type, bad, d_out[0], s);
+    });
+}
+
+} // namespace
+
 extern "C" {
 
 int fb200_vinterp_create_hybrid(int method, const double* ap, const double* b, int nk, double ps_scale, const double* levels, int np,
@@ -2621,6 +2726,57 @@ int fb200_vconvert_values_device(const fb200_vconvert* h, const float* d_in, con
     if (check_vconvert_call(h, d_in, or_none(d_cols), nxy, nt, d_out) != FB_OK)
         return MIFI_ERROR;
     return vconvert_device(h, d_in, or_none(d_cols), nxy, nt, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_tinterp_create(const double* times, int nt, const double* new_times, int nt_new, int extrapolate, fb200_tinterp** handle)
+{
+    return tinterp_create(times, nt, new_times, nt_new, extrapolate, handle) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+void fb200_tinterp_destroy(fb200_tinterp* h)
+{
+    delete h;
+}
+
+int fb200_tinterp_source_steps(const fb200_tinterp* h, int j, int* ia, int* ib, double* w)
+{
+    FB_REQUIRE(h != nullptr, "null time interpolation handle");
+    FB_REQUIRE(j >= 0 && j < h->nj, "target step " + std::to_string(j) + " out of range [0, " + std::to_string(h->nj) + ")");
+    FB_REQUIRE(ia && ib && w, "null output pointer");
+    const TimeStep& m = h->map[j];
+    *ia = m.ia;
+    *ib = m.ia < 0 ? -1 : m.ia + 1;
+    *w = m.w;
+    return MIFI_OK;
+}
+
+int fb200_tinterp_get_step(const fb200_tinterp* h, int j, int inType, const void* a, const void* b, size_t n, double badValue, int outType, void* out)
+{
+    if (check_tinterp_call(h, false, j, inType, outType, n, a, b, out) != FB_OK)
+        return MIFI_ERROR;
+    return tinterp_get_step_host(h, j, inType, a, b, n, badValue, outType, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_tinterp_get_step_device(const fb200_tinterp* h, int j, int inType, const void* d_a, const void* d_b, size_t n, double badValue, int outType,
+                                  void* d_out, void* stream)
+{
+    if (check_tinterp_call(h, false, j, inType, outType, n, d_a, d_b, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return launch_tinterp(inType, d_a, d_b, (long long)n, has_bad_value(badValue), (float)badValue, h->d_single + j, 1, outType, badValue, d_out,
+                          as_stream(stream)) == FB_OK
+               ? MIFI_OK
+               : MIFI_ERROR;
+}
+
+int fb200_tinterp_get_data_slice_device(const fb200_tinterp* h, int inType, const void* d_in, size_t n, double badValue, int outType, void* d_out,
+                                        void* stream)
+{
+    if (check_tinterp_call(h, true, 0, inType, outType, n, d_in, d_in, d_out) != FB_OK)
+        return MIFI_ERROR;
+    return launch_tinterp(inType, d_in, nullptr, (long long)n, has_bad_value(badValue), (float)badValue, h->d_sorted, h->nj, outType, badValue, d_out,
+                          as_stream(stream)) == FB_OK
+               ? MIFI_OK
+               : MIFI_ERROR;
 }
 
 // ---------------------------------------------------------------------------------------- mifi_* drop-ins

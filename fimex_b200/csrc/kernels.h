@@ -177,4 +177,15 @@ enum { FB_VCOORD_PRESSURE = 0, FB_VCOORD_HYBRID = 1, FB_VCOORD_SIGMA = 2 };
 int launch_vconvert(int op, int vcoord, const VertTable& vt, double kappa, const float* d_in, const float* d_ps, const float* d_t, long long nxy,
                     long long nt, float* d_out, cudaStream_t st);
 
+// ---- time_kernels.cu (time interpolation: CDMTimeInterpolator's linear change of the time axis) ------------------------
+// one target step: output row `row` = step ia + w * (step ia+1 - step ia); ia = -1: no bracket (NaN, stored as the fill value)
+struct alignas(16) TimeStep {
+    int ia, row;
+    double w;
+};
+// d_tab [nj]: the targets in non-decreasing ia, those with ia = -1 last.  in [.][n] of in_type (step k at d_in + k n; d_in_b != null:
+// a two-step call with step 1 at d_in_b), badValue -> NaN while loading when has_bad; out [.][n] of out_type, NaN -> fill + cast
+int launch_tinterp(int in_type, const void* d_in, const void* d_in_b, long long n, bool has_bad, float bad, const TimeStep* d_tab, int nj, int out_type,
+                   double fill, void* d_out, cudaStream_t st);
+
 } // namespace fb

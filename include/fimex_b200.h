@@ -424,6 +424,34 @@ int fb200_vconvert_values_device(const fb200_vconvert* handle, const float* d_in
                                  float* d_out, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * (1h) time interpolation: the linear change of the time axis of CDMTimeInterpolator (--timeInterpolate.timeSpec; DESIGN.md
+ *      section 2 states the arithmetic)
+ *
+ * times [nt]: the source times, strictly increasing, 2 <= nt; new_times [nt_new]: the target times in any order, repeats allowed,
+ * 1 <= nt_new <= 1048576; all finite and in ONE unit.  Target j takes the smallest bracket k with t_k <= tau_j <= t_k+1 and
+ * w = (tau_j - t_k) / (t_k+1 - t_k) in fp64; outside [t_0, t_nt-1] the end pair on that side when extrapolate != 0, else no bracket
+ * (the step is NaN, stored as badValue).  Every value: r = (float)((double)A + w * ((double)B - (double)A)), no FMA.  The slices are
+ * typed as in (1c): inType in with badValue -> NaN, NaN -> badValue and round + cast to outType out (float: inType = outType =
+ * FB200_FLOAT, badValue = NaN); no scale or offset is applied.  The handle is immutable and every call re-entrant.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct fb200_tinterp fb200_tinterp; /* opaque */
+
+int fb200_tinterp_create(const double* times, int nt, const double* new_times, int nt_new, int extrapolate, fb200_tinterp** handle);
+void fb200_tinterp_destroy(fb200_tinterp* handle);
+/* the time-change map of target step j: source steps ia < ib and weight w; ia = ib = -1 where no bracket applies */
+int fb200_tinterp_source_steps(const fb200_tinterp* handle, int j, int* ia, int* ib, double* w);
+/* one target step from the two source slices the map names (n elements each; NULL allowed where no bracket applies): the shape of
+ * the reference's getDataSlice(var, unLimDimPos).  Host buffers (copies pipelined over element chunks) or, for _device, device
+ * pointers on `cuda_stream` without synchronisation. */
+int fb200_tinterp_get_step(const fb200_tinterp* handle, int j, int inType, const void* a, const void* b, size_t n, double badValue, int outType,
+                           void* out);
+int fb200_tinterp_get_step_device(const fb200_tinterp* handle, int j, int inType, const void* d_a, const void* d_b, size_t n, double badValue,
+                                  int outType, void* d_out, void* cuda_stream);
+/* the whole stack on the device: d_in [nt][n] -> d_out [nt_new][n], every source step the targets need read once */
+int fb200_tinterp_get_data_slice_device(const fb200_tinterp* handle, int inType, const void* d_in, size_t n, double badValue, int outType,
+                                        void* d_out, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
  * ---------------------------------------------------------------------------------------------- */
 int mifi_string_to_interpolation_method(const char* stringMethod); /* :44 */
