@@ -47,7 +47,8 @@ __global__ void k_nn_keys(const double* __restrict__ lon, const double* __restri
         const int ix = (int)(s / ny), iy = (int)(s % ny);
         const long long pos = ix + (long long)iy * nx;
         const bool bad = isnan(lon[pos]) || isnan(lat[pos]);
-        keys[s] = bad ? 0xffffffffffffffffull : orderable(lat[pos]); // invalid points sort last and are cut off
+        // invalid points sort last and are cut off; -0 + 0 is +0, so -0 and +0 are one key and keep insertion order
+        keys[s] = bad ? 0xffffffffffffffffull : orderable(lat[pos] + 0.);
         vals[s] = (int)s;
     }
 }
@@ -263,10 +264,16 @@ __global__ void __launch_bounds__(kThreads) k_kd_search(double* __restrict__ px,
         sincos(plat, &sla, &cla);
         sincos(plon, &slo, &clo);
         const double qx = __dmul_rn(cla, clo), qy = __dmul_rn(cla, slo), qz = sla; // :1045-1047
+        // the window is centred on the latitude of the point q, which a target beyond a pole (|plat| > pi/2) is not
+        double wlat = remainder(plat, 2. * FB_PI);
+        if (wlat > 0.5 * FB_PI)
+            wlat = FB_PI - wlat;
+        else if (wlat < -0.5 * FB_PI)
+            wlat = -FB_PI - wlat;
         long long a, b;
         {
             long long lo = 0, hi = m;
-            const double lowlat = plat - window;
+            const double lowlat = wlat - window;
             while (lo < hi) {
                 const long long mid = (lo + hi) >> 1;
                 if (sorted_lat[mid] < lowlat)
@@ -276,7 +283,7 @@ __global__ void __launch_bounds__(kThreads) k_kd_search(double* __restrict__ px,
             }
             a = lo;
             hi = m;
-            const double highlat = plat + window;
+            const double highlat = wlat + window;
             while (lo < hi) {
                 const long long mid = (lo + hi) >> 1;
                 if (sorted_lat[mid] <= highlat)
@@ -368,15 +375,10 @@ int coordnn_search(double* d_px, double* d_py, long long n, const double* h_lon,
     FB_CUDA_CHECK(cudaMemcpyAsync(h_best.data(), d_best, sizeof(double) * steps, cudaMemcpyDeviceToHost, st));
     FB_CUDA_CHECK(cudaStreamSynchronize(st));
     double worst = 2.;
-    bool have = false;
-    for (double b : h_best) {
-        if (b > 2.5)
-            continue; // skipped sample
-        if (!have || b < worst)
+    for (double b : h_best)
+        if (b < worst) // a skipped sample is 3
             worst = b;
-        have = true;
-    }
-    FB_REQUIRE(have, "coord_nearestneighbor: no valid sample point in the source coordinates");
+    // no valid sample leaves worst = 2 and, as in the reference, roi = acos(2) = NaN: every target gets (-1, -1)
     double roi = std::acos(worst);
     roi *= 1.414;
     if (roi > FB_PI)
