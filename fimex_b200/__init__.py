@@ -14,7 +14,8 @@ The product is ``fimex_b200/lib/libfimex_b200.so`` (hand-written sm_100a CUDA be
 * :mod:`fimex_b200.vertical` -- the pressure, height and depth branches of ``CDMVerticalInterpolator`` (model levels -> pressure, height,
   altitude or depth levels) and its data conversions (``PressureConversion``: theta2T, omega2vwind, add4Dpressure) on the GPU;
 * :mod:`fimex_b200.timeinterp` -- the linear change of the time axis of ``CDMTimeInterpolator`` (``TimeInterpolator``) on the GPU;
-* :mod:`fimex_b200.merger` -- ``CDMMerger`` (inner grid merged into an outer one with border smoothing) on the same interpolations;
+* :mod:`fimex_b200.merger` -- ``CDMMerger`` (inner grid merged into an outer one with linear border smoothing): the three gathers, the
+  blend and the overlay of a merged slice in one call on the GPU;
 * :mod:`fimex_b200.slab`    -- one-process-per-GPU slab partition of the (time x level) stack with a single
   NCCL broadcast of the cached tables.
 """
@@ -28,7 +29,7 @@ from .capi import (DataType, cdm_type, default_fill_value, LATITUDE, LONGITUDE, 
 from .cached import CachedForwardInterpolation, CachedInterpolation, CachedVectorReprojection
 from .interpolator import Interpolator, axis_spec_requires_start_end, spatial_axis_spec, tokenize_dotted
 from .processor import Processor
-from .merger import Merger, extend_inner_axis, linear_border_smoothing
+from .merger import Merger, extend_inner_axis, linear_border_smoothing, parse_smoothing
 from .timeinterp import TimeInterpolator
 from .vertical import DepthInterpolator, HeightInterpolator, PressureConversion, VerticalInterpolator, vertical_method
 
@@ -37,7 +38,7 @@ from .vertical import DepthInterpolator, HeightInterpolator, PressureConversion,
 BICUBIC_FP32_AVAILABLE = True
 
 __all__ = [
-    "CachedInterpolation", "CachedForwardInterpolation", "CachedVectorReprojection", "Interpolator", "Processor", "Merger", "VerticalInterpolator", "HeightInterpolator", "DepthInterpolator", "PressureConversion", "TimeInterpolator", "vertical_method", "extend_inner_axis", "linear_border_smoothing", "spatial_axis_spec", "axis_spec_requires_start_end", "tokenize_dotted", "Method", "DataType", "cdm_type", "default_fill_value", "FimexB200Error",
+    "CachedInterpolation", "CachedForwardInterpolation", "CachedVectorReprojection", "Interpolator", "Processor", "Merger", "VerticalInterpolator", "HeightInterpolator", "DepthInterpolator", "PressureConversion", "TimeInterpolator", "vertical_method", "extend_inner_axis", "linear_border_smoothing", "parse_smoothing", "spatial_axis_spec", "axis_spec_requires_start_end", "tokenize_dotted", "Method", "DataType", "cdm_type", "default_fill_value", "FimexB200Error",
     "MIFI_OK", "MIFI_ERROR", "PROJ_AXIS", "LONGITUDE", "LATITUDE", "MIFI_VECTOR_KEEP_SIZE", "load", "lib_path", "version", "last_error",
     "set_device", "kernel_launches", "mifi_interpolate_f", "mifi_points2position", "mifi_project_axes", "mifi_project_values",
     "mifi_get_vector_reproject_matrix", "mifi_get_vector_reproject_matrix_field", "mifi_get_vector_reproject_matrix_points",

@@ -19,7 +19,7 @@ LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libfimex_b200.so")
 
 SOURCES = ["api.cu", "setup_kernels.cu", "gather_kernels.cu", "forward_kernels.cu", "coordnn_kernels.cu", "adapter_kernels.cu", "staged_kernels.cu", "bicubic_staged.cu", "fill_kernels.cu",
-           "vertical_kernels.cu", "time_kernels.cu", "proj_parse.cpp"]
+           "vertical_kernels.cu", "time_kernels.cu", "merge_kernels.cu", "proj_parse.cpp"]
 HEADERS = ["common.cuh", "proj.cuh", "kernels.h", "tables.cuh", "interp_math.cuh", "convert.cuh", os.path.join("..", "..", "include", "fimex_b200.h")]
 
 NVCC_FLAGS = [

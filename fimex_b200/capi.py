@@ -195,6 +195,10 @@ def _declare(lib):
         "fb200_tinterp_get_step": (i, [_vp, i, i, _vp, _vp, sz, C.c_double, i, _vp]),
         "fb200_tinterp_get_step_device": (i, [_vp, i, i, _vp, _vp, sz, C.c_double, i, _vp, _vp]),
         "fb200_tinterp_get_data_slice_device": (i, [_vp, i, _vp, sz, C.c_double, i, _vp, _vp]),
+        "fb200_merge_create": (i, [_vp, _vp, _vp, sz, sz, sz, sz, i, i, i, P(_vp)]),
+        "fb200_merge_destroy": (None, [_vp]),
+        "fb200_merge_get_data_slice": (i, [_vp, i, _vp, sz, C.c_double, _vp, sz, C.c_double, i, C.c_double, _vp, P(sz)]),
+        "fb200_merge_get_data_slice_device": (i, [_vp, i, _vp, sz, C.c_double, _vp, sz, C.c_double, i, C.c_double, _vp, P(sz), _vp]),
         "mifi_string_to_interpolation_method": (i, [C.c_char_p]),
         "mifi_interpolate_f": (i, [i, C.c_char_p, _vp, _vp, _vp, i, i, i, i, i, C.c_char_p, _vp, _vp, _vp, i, i, i, i]),
         "mifi_vector_reproject_values_f": (i, [i, C.c_char_p, C.c_char_p, _vp, _vp, _vp, _vp, i, i, i, i, i]),

@@ -232,6 +232,7 @@ struct fb200_interp {
     bool forward = false;
     int device = 0;
     size_t inX = 0, inY = 0, outX = 0, outY = 0;
+    size_t srcX = 0, srcY = 0; // the source grid as created: inX, inY before createReducedDomain cropped them
     size_t npts = 0; // outX*outY (backward) or inX*inY (forward)
     double* d_px = nullptr;
     double* d_py = nullptr;
@@ -371,6 +372,8 @@ int new_interp(int funcType, bool forward, size_t inX, size_t inY, size_t outX, 
     h->device = default_device();
     h->inX = inX;
     h->inY = inY;
+    h->srcX = inX;
+    h->srcY = inY;
     h->outX = outX;
     h->outY = outY;
     h->npts = forward ? inX * inY : outX * outY;
@@ -2608,6 +2611,164 @@ int tinterp_get_step_host(const fb200_tinterp* h, int j, int in_type, const void
 
 } // namespace
 
+// ======================================================================================================
+// merger (CDMMerger: the inner grid blended into the outer one at its border, then laid over the outer one on a target grid)
+// ======================================================================================================
+struct fb200_merge {
+    const fb200_interp* o2i = nullptr; // outer -> inner grid; all three are borrowed: the caller keeps them alive
+    const fb200_interp* i2t = nullptr; // inner -> target grid
+    const fb200_interp* o2t = nullptr; // outer -> target grid
+    int device = 0;
+    size_t innerX = 0, innerY = 0, outerX = 0, outerY = 0;
+    int t = 0, b = 0; // transition and border width of CDMBorderSmoothing_Linear
+    bool use_outer = true;
+};
+
+namespace {
+
+// The device chain works through the levels in chunks whose float intermediates (the outer slab cropped to one handle's domain,
+// the outer field on the inner grid, the smoothed window, the top and base fields on the target grid) take at most this many bytes,
+// or one level where a single level is larger: a whole stack never needs a second copy of itself in scratch.
+constexpr size_t kMergeScratchBytes = 256ull << 20;
+
+std::string grid_str(size_t x, size_t y)
+{
+    return std::to_string(x) + " x " + std::to_string(y);
+}
+
+int check_merge_handle(const fb200_interp* h, const char* which, size_t srcX, size_t srcY, const char* src_name)
+{
+    FB_REQUIRE(h != nullptr, std::string("null ") + which + " interpolation handle");
+    FB_REQUIRE(!h->forward && (h->method == FB_NN || h->method == FB_BILINEAR || h->method == FB_BICUBIC),
+               std::string("the ") + which + " handle must interpolate with nearest neighbour, bilinear or bicubic (method " + std::to_string(h->method) + ")");
+    FB_REQUIRE(h->srcX == srcX && h->srcY == srcY,
+               std::string("the ") + which + " handle reads a " + grid_str(h->srcX, h->srcY) + " grid, the " + src_name + " grid is " + grid_str(srcX, srcY));
+    return FB_OK;
+}
+
+int merge_create(const fb200_interp* o2i, const fb200_interp* i2t, const fb200_interp* o2t, size_t innerX, size_t innerY, size_t outerX, size_t outerY,
+                 int t, int b, int use_outer, fb200_merge** handle)
+{
+    FB_REQUIRE(handle != nullptr, "null handle pointer");
+    *handle = nullptr;
+    FB_REQUIRE(t >= 1, "transition width must be at least 1 (the linear border smoothing divides by it), got " + std::to_string(t));
+    FB_REQUIRE(b >= 0, "border width must not be negative, got " + std::to_string(b));
+    FB_REQUIRE(innerX > 0 && innerY > 0 && outerX > 0 && outerY > 0, "empty inner or outer grid");
+    if (check_merge_handle(o2i, "outer -> inner", outerX, outerY, "outer") != FB_OK || check_merge_handle(i2t, "inner -> target", innerX, innerY, "inner") != FB_OK ||
+        check_merge_handle(o2t, "outer -> target", outerX, outerY, "outer") != FB_OK)
+        return FB_ERROR;
+    FB_REQUIRE(o2i->outX == innerX && o2i->outY == innerY,
+               "the outer -> inner handle writes a " + grid_str(o2i->outX, o2i->outY) + " grid, the inner grid is " + grid_str(innerX, innerY));
+    FB_REQUIRE(i2t->outX == o2t->outX && i2t->outY == o2t->outY, "the inner -> target handle writes a " + grid_str(i2t->outX, i2t->outY) +
+                                                                      " grid, the outer -> target handle a " + grid_str(o2t->outX, o2t->outY) + " grid");
+    FB_REQUIRE(o2i->device == i2t->device && o2i->device == o2t->device, "the three interpolation handles live on different devices");
+    std::unique_ptr<fb200_merge> h(new fb200_merge());
+    h->o2i = o2i;
+    h->i2t = i2t;
+    h->o2t = o2t;
+    h->device = o2i->device;
+    h->innerX = innerX;
+    h->innerY = innerY;
+    h->outerX = outerX;
+    h->outerY = outerY;
+    h->t = t;
+    h->b = b;
+    h->use_outer = use_outer != 0;
+    *handle = h.release();
+    return FB_OK;
+}
+
+// both sizes must hold the same whole number of levels of their grid; *nz receives it
+int check_merge_call(const fb200_merge* h, int in_type, int out_type, size_t inner_size, size_t outer_size, const void* inner, const void* outer,
+                     const void* out, size_t* nz)
+{
+    FB_REQUIRE(h != nullptr, "null merge handle");
+    FB_REQUIRE(!h->o2i->invalid && !h->i2t->invalid && !h->o2t->invalid,
+               "an interpolation handle of the merger is unusable: createReducedDomain failed while rebuilding its tables");
+    if (check_slice_types(in_type, out_type) != FB_OK)
+        return FB_ERROR;
+    const size_t il = h->innerX * h->innerY, ol = h->outerX * h->outerY;
+    FB_REQUIRE(inner_size % il == 0, "inner size " + std::to_string(inner_size) + " is not a whole number of " + grid_str(h->innerX, h->innerY) + " levels");
+    FB_REQUIRE(outer_size % ol == 0, "outer size " + std::to_string(outer_size) + " is not a whole number of " + grid_str(h->outerX, h->outerY) + " levels");
+    *nz = inner_size / il;
+    FB_REQUIRE(outer_size / ol == *nz, "inner has " + std::to_string(*nz) + " levels, outer " + std::to_string(outer_size / ol));
+    FB_REQUIRE(*nz == 0 || (inner && outer && out), "null data pointer");
+    return use_device(h->device);
+}
+
+size_t merge_target_level(const fb200_merge* h)
+{
+    return h->i2t->outX * h->i2t->outY;
+}
+
+// crop + convert, outer -> inner gather, smoothing, inner -> target gather, crop + convert, outer -> target gather, overlay: all on st
+int merge_device(const fb200_merge* h, int in_type, const void* d_inner, double bad_inner, const void* d_outer, double bad_outer, size_t nz, int out_type,
+                 double out_fill, void* d_out, cudaStream_t st)
+{
+    const fb200_interp *o2i = h->o2i, *i2t = h->i2t, *o2t = h->o2t;
+    const size_t inner_lvl = h->innerX * h->innerY, outer_lvl = h->outerX * h->outerY, target_lvl = merge_target_level(h);
+    if (nz == 0 || target_lvl == 0)
+        return FB_OK;
+    const size_t crop_lvl = std::max(o2i->inX * o2i->inY, o2t->inX * o2t->inY); // one buffer: the two crops are used one after the other
+    const size_t smooth_lvl = i2t->inX * i2t->inY;
+    const size_t per_level = sizeof(float) * (crop_lvl + inner_lvl + smooth_lvl + 2 * target_lvl);
+    const size_t zc = std::min(nz, std::max<size_t>(1, kMergeScratchBytes / per_level));
+    Scratch tmp(st);
+    float *crop = nullptr, *on_inner = nullptr, *smooth = nullptr, *top = nullptr, *base = nullptr;
+    if (tmp.get(&crop, zc * crop_lvl) != FB_OK || tmp.get(&on_inner, zc * inner_lvl) != FB_OK || tmp.get(&smooth, zc * smooth_lvl) != FB_OK ||
+        tmp.get(&top, zc * target_lvl) != FB_OK || tmp.get(&base, zc * target_lvl) != FB_OK)
+        return FB_ERROR;
+    SliceIO io; // the gathers as getDataSlice on float with NaN = undefined both ways (pre/postprocesses of a handle apply)
+    io.typed = true;
+    io.bad[0] = std::numeric_limits<double>::quiet_NaN();
+    auto gather = [&](const fb200_interp* g, const float* in, size_t zn, float* out) {
+        const void* i[1] = {in};
+        void* o[1] = {out};
+        return run_slice_device(g, nullptr, 1, i, zn, o, io, st);
+    };
+    const bool outer_has_bad = has_bad_value(bad_outer), inner_has_bad = !std::isnan(bad_inner);
+    const size_t in_elem = type_size(in_type), out_elem = type_size(out_type);
+    for (size_t z0 = 0; z0 < nz; z0 += zc) {
+        const size_t zn = std::min(zc, nz - z0);
+        const char* inner = static_cast<const char*>(d_inner) + z0 * inner_lvl * in_elem;
+        const char* outer = static_cast<const char*>(d_outer) + z0 * outer_lvl * in_elem;
+        char* out = static_cast<char*>(d_out) + z0 * target_lvl * out_elem;
+        if (launch_crop_as_float(in_type, outer, h->outerX, h->outerY, o2i->xMin, o2i->yMin, o2i->inX, o2i->inY, zn, outer_has_bad, (float)bad_outer, crop,
+                                 st) != FB_OK ||
+            gather(o2i, crop, zn, on_inner) != FB_OK ||
+            launch_border_smooth_linear(in_type, inner, inner_has_bad, bad_inner, on_inner, h->innerX, h->innerY, h->t, h->b, h->use_outer, i2t->xMin,
+                                        i2t->yMin, i2t->inX, i2t->inY, zn, smooth, st) != FB_OK ||
+            gather(i2t, smooth, zn, top) != FB_OK ||
+            launch_crop_as_float(in_type, outer, h->outerX, h->outerY, o2t->xMin, o2t->yMin, o2t->inX, o2t->inY, zn, outer_has_bad, (float)bad_outer, crop,
+                                 st) != FB_OK ||
+            gather(o2t, crop, zn, base) != FB_OK || launch_merge_overlay(top, base, (long long)(zn * target_lvl), out_type, out_fill, out, st) != FB_OK)
+            return FB_ERROR;
+    }
+    return FB_OK;
+}
+
+// host buffers: inner and outer go up once and the merged slice comes down once, pipelined over level chunks
+int merge_host(const fb200_merge* h, int in_type, const void* inner, double bad_inner, const void* outer, double bad_outer, size_t nz, int out_type,
+               double out_fill, void* out)
+{
+    const size_t target_lvl = merge_target_level(h);
+    if (nz == 0 || target_lvl == 0)
+        return FB_OK;
+    HostArrays arrays;
+    arrays.device = h->device;
+    arrays.in[0] = inner;
+    arrays.in_unit[0] = h->innerX * h->innerY * type_size(in_type);
+    arrays.in[1] = outer;
+    arrays.in_unit[1] = h->outerX * h->outerY * type_size(in_type);
+    arrays.out[0] = out;
+    arrays.out_unit[0] = target_lvl * type_size(out_type);
+    return stage_host(arrays, nz, [&](const void* const* d_in, size_t zn, void* const* d_o, cudaStream_t s) {
+        return merge_device(h, in_type, d_in[0], bad_inner, d_in[1], bad_outer, zn, out_type, out_fill, d_o[0], s);
+    });
+}
+
+} // namespace
+
 extern "C" {
 
 int fb200_vinterp_create_hybrid(int method, const double* ap, const double* b, int nk, double ps_scale, const double* levels, int np,
@@ -2777,6 +2938,42 @@ int fb200_tinterp_get_data_slice_device(const fb200_tinterp* h, int inType, cons
                           as_stream(stream)) == FB_OK
                ? MIFI_OK
                : MIFI_ERROR;
+}
+
+int fb200_merge_create(const fb200_interp* outerToInner, const fb200_interp* innerToTarget, const fb200_interp* outerToTarget, size_t innerX, size_t innerY,
+                       size_t outerX, size_t outerY, int transitionWidth, int borderWidth, int useOuterIfInnerUndefined, fb200_merge** handle)
+{
+    return merge_create(outerToInner, innerToTarget, outerToTarget, innerX, innerY, outerX, outerY, transitionWidth, borderWidth, useOuterIfInnerUndefined,
+                        handle) == FB_OK
+               ? MIFI_OK
+               : MIFI_ERROR;
+}
+
+void fb200_merge_destroy(fb200_merge* h)
+{
+    delete h;
+}
+
+int fb200_merge_get_data_slice(const fb200_merge* h, int inType, const void* inner, size_t innerSize, double badInner, const void* outer, size_t outerSize,
+                               double badOuter, int outType, double outFill, void* out, size_t* newSize)
+{
+    size_t nz = 0;
+    if (check_merge_call(h, inType, outType, innerSize, outerSize, inner, outer, out, &nz) != FB_OK)
+        return MIFI_ERROR;
+    if (newSize)
+        *newSize = merge_target_level(h) * nz;
+    return merge_host(h, inType, inner, badInner, outer, badOuter, nz, outType, outFill, out) == FB_OK ? MIFI_OK : MIFI_ERROR;
+}
+
+int fb200_merge_get_data_slice_device(const fb200_merge* h, int inType, const void* d_inner, size_t innerSize, double badInner, const void* d_outer,
+                                      size_t outerSize, double badOuter, int outType, double outFill, void* d_out, size_t* newSize, void* stream)
+{
+    size_t nz = 0;
+    if (check_merge_call(h, inType, outType, innerSize, outerSize, d_inner, d_outer, d_out, &nz) != FB_OK)
+        return MIFI_ERROR;
+    if (newSize)
+        *newSize = merge_target_level(h) * nz;
+    return merge_device(h, inType, d_inner, badInner, d_outer, badOuter, nz, outType, outFill, d_out, as_stream(stream)) == FB_OK ? MIFI_OK : MIFI_ERROR;
 }
 
 // ---------------------------------------------------------------------------------------- mifi_* drop-ins

@@ -188,4 +188,16 @@ struct alignas(16) TimeStep {
 int launch_tinterp(int in_type, const void* d_in, const void* d_in_b, long long n, bool has_bad, float bad, const TimeStep* d_tab, int nj, int out_type,
                    double fill, void* d_out, cudaStream_t st);
 
+// ---- merge_kernels.cu (CDMMerger: crop, linear border smoothing, overlay) -------------------------------------------------
+// [nz][ny][nx] of in_type -> the window [x0, x0 + w) x [y0, y0 + h) of every level as float [nz][h][w], badValue -> NaN when has_bad
+// (the gather's own input adapter, mifi_bad2nanf)
+int launch_crop_as_float(int in_type, const void* d_in, long long nx, long long ny, long long x0, long long y0, long long w, long long h, long long nz,
+                         bool has_bad, float bad, float* d_out, cudaStream_t st);
+// the linear border smoothing (DESIGN.md section 2) of inner [nz][ny][nx] of in_type (values equal to (in_type)bad -> NaN when has_bad)
+// with outer [nz][ny][nx] float on the inner grid, in fp64; only the window [x0, x0 + w) x [y0, y0 + h) is written, as float [nz][h][w]
+int launch_border_smooth_linear(int in_type, const void* d_inner, bool has_bad, double bad, const float* d_outer, long long nx, long long ny, int t, int b,
+                                bool use_outer, long long x0, long long y0, long long w, long long h, long long nz, float* d_out, cudaStream_t st);
+// out[i] = top[i] where it is not NaN, else base[i]; NaN -> fill, round + cast to out_type
+int launch_merge_overlay(const float* d_top, const float* d_base, long long n, int out_type, double fill, void* d_out, cudaStream_t st);
+
 } // namespace fb

@@ -10,17 +10,38 @@ Reference (arebru/fimex 0.67.2):
   CDMOverlay::getDataSlice (top where defined, else base)               src/CDMOverlay.cc:63-92
   makeMergedCDM (outer interpolated to the inner grid)                  src/CDMMergeUtils.cc:214-246
 
-The three interpolations of one merged slice -- outer -> inner grid (for the border blend), blended inner -> target grid,
-outer -> target grid -- run on the GPU through `Interpolator`; the blend and the overlay are the reference's own per-value
-rules on the host (a few thousand values; they are not part of the gather path).  As in interpolator.py the CDM side (which
-variables, coordinate systems, units) stays with the host application: grids are described by proj4 string and axes.
+One merged slice is one call of fb200_merge_get_data_slice[_device] (include/fimex_b200.h, section 1i): the outer -> inner
+gather, the linear border blend on the inner grid, the blended inner -> target gather, the outer -> target gather and the overlay
+all run on the GPU, on the three `Interpolator` handles built by setTargetGrid.  `linear_border_smoothing` below restates the
+blend in numpy; it is the reference the tests hold the kernel to, not part of the slice path.  As in interpolator.py the CDM
+side (which variables, coordinate systems, units) stays with the host application: grids are described by proj4 string and
+axes.
 """
 from __future__ import annotations
 
+import ctypes as C
+import re
+
 import numpy as np
 
-from .capi import FimexB200Error, Method
+from . import capi
+from .cached import _is_torch, _stream_ptr
+from .capi import FimexB200Error, Method, check, load, ptr
 from .interpolator import Interpolator
+
+_LINEAR = re.compile(r"\s*LINEAR\s*\(\s*(\d+)\s*,\s*(\d+)\s*\)\s*")
+
+
+def parse_smoothing(spec):
+    """--merge.smoothing (CDMBorderSmoothing_LinearFactory): "LINEAR(transitionWidth,borderWidth)" -> (t, b), integers with t >= 1
+    (the blend divides by it) and b >= 0; anything else raises"""
+    m = _LINEAR.fullmatch(spec) if isinstance(spec, str) else None
+    if m is None:
+        raise FimexB200Error(f"cannot parse smoothing '{spec}': expected LINEAR(transitionWidth,borderWidth)")
+    t, b = int(m.group(1)), int(m.group(2))
+    if t < 1:
+        raise FimexB200Error(f"smoothing '{spec}': the transition width must be at least 1")
+    return t, b
 
 
 def extend_inner_axis(inner, outer):
@@ -77,42 +98,103 @@ def linear_border_smoothing(inner, outer, transition_width=5, border_width=2, us
     return np.where(np.isnan(vi), vo if use_outer_if_inner_undefined else np.nan, merged)
 
 
+class _MergeHandle:
+    """fb200_merge: borrows the three interpolation handles, so it keeps their owners alive"""
+
+    def __init__(self, o2i, i2t, o2t, inner_shape, outer_shape, t, b, use_outer):
+        self.keep = (o2i, i2t, o2t)
+        self.key = (t, b, bool(use_outer))
+        self._h = C.c_void_p()
+        (nyi, nxi), (nyo, nxo) = inner_shape, outer_shape
+        check(load().fb200_merge_create(o2i._h, i2t._h, o2t._h, nxi, nyi, nxo, nyo, int(t), int(b), int(bool(use_outer)), C.byref(self._h)),
+              "CDMMerger")
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h:
+            load().fb200_merge_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def _fill_for(dtype, value):
+    """the bad / fill value of a slice: as given, else NaN for floating types and defaultFillValue_ for integer types"""
+    if value is not None:
+        return float(value)
+    return float("nan") if np.dtype(str(dtype).replace("torch.", "")).kind == "f" else capi.default_fill_value(dtype)
+
+
 class Merger:
     """CDMMerger for one variable's horizontal coordinate systems: an inner (fine, small) grid merged into an outer (coarse,
     large) one on a target grid.
 
-    proj_inner / proj_outer : proj4 strings; x/y axes in the projection's unit, degrees when `is_degree`
+    proj_inner / proj_outer : proj4 strings; x/y axes in the projection's unit, degrees when `is_degree` (the inner grid's, and the
+    outer grid's too unless `outer_is_degree` says otherwise: a projected inner grid inside a lat/lon outer one)
     """
 
-    def __init__(self, proj_inner, x_inner, y_inner, proj_outer, x_outer, y_outer, is_degree):
+    def __init__(self, proj_inner, x_inner, y_inner, proj_outer, x_outer, y_outer, is_degree, outer_is_degree=None):
         self.proj_inner, self.proj_outer = proj_inner, proj_outer
         self.x_inner, self.y_inner = np.asarray(x_inner, dtype=np.float64), np.asarray(y_inner, dtype=np.float64)
         self.x_outer, self.y_outer = np.asarray(x_outer, dtype=np.float64), np.asarray(y_outer, dtype=np.float64)
         self.is_degree = bool(is_degree)
+        self.outer_is_degree = self.is_degree if outer_is_degree is None else bool(outer_is_degree)
         self.gridInterpolationMethod = Method.BILINEAR  # src/CDMMerger.cc:84
         self.transitionWidth, self.borderWidth = 5, 2   # CDMBorderSmoothing_LinearFactory defaults
         self.useOuterIfInnerUndefined = True
         self._outer_to_inner = None
         self._inner_to_target = None
         self._outer_to_target = None
+        self._merge = None
 
     def setGridInterpolationMethod(self, method):
+        """takes effect with the next setTargetGrid / setTargetGridFromInner, as in the reference"""
         self.gridInterpolationMethod = Method(int(method))
+
+    def setSmoothing(self, spec):
+        """CDMMerger::setSmoothing with the --merge.smoothing option string, e.g. "LINEAR(5,2)" """
+        self.transitionWidth, self.borderWidth = parse_smoothing(spec)
+        if self._outer_to_target is not None:
+            self._merge_handle()
+        return self
+
+    def setUseOuterIfInnerUndefined(self, flag):
+        """CDMBorderSmoothing::setUseOuterIfInnerUndefined"""
+        self.useOuterIfInnerUndefined = bool(flag)
+        return self
+
+    def _merge_handle(self):
+        """the fb200_merge handle of the current target grid and smoothing, rebuilt whenever one of them has changed"""
+        key = (self.transitionWidth, self.borderWidth, bool(self.useOuterIfInnerUndefined))
+        if self._merge is None or self._merge.key != key:
+            if not (int(self.transitionWidth) >= 1 and int(self.borderWidth) >= 0):
+                raise FimexB200Error(f"smoothing LINEAR({self.transitionWidth},{self.borderWidth}): the transition width must be at least 1 "
+                                     "and the border width at least 0")
+            self._merge = None
+            self._merge = _MergeHandle(self._outer_to_inner.cachedInterpolation, self._inner_to_target.cachedInterpolation,
+                                       self._outer_to_target.cachedInterpolation, (self.y_inner.size, self.x_inner.size),
+                                       (self.y_outer.size, self.x_outer.size), self.transitionWidth, self.borderWidth, self.useOuterIfInnerUndefined)
+        return self._merge
 
     def setTargetGrid(self, proj, tx, ty, tx_unit="m", ty_unit="m"):
         """CDMMerger::setTargetGrid -> makeCDM (:211-229)"""
         unit = "degree" if self.is_degree else "m"
         m = self.gridInterpolationMethod
+        self._merge = None
         # readerSmooth: outer interpolated onto the INNER grid (makeMergedCDM, CDMMergeUtils.cc:234-243)
-        self._outer_to_inner = Interpolator(self.proj_outer, self.x_outer, self.y_outer, self.is_degree)
+        self._outer_to_inner = Interpolator(self.proj_outer, self.x_outer, self.y_outer, self.outer_is_degree)
         self._outer_to_inner.changeProjection(m, self.proj_inner, self.x_inner, self.y_inner, unit, unit)
         # interpolatedST: the smoothed inner field onto the target grid
         self._inner_to_target = Interpolator(self.proj_inner, self.x_inner, self.y_inner, self.is_degree)
         self._inner_to_target.changeProjection(m, proj, tx, ty, tx_unit, ty_unit)
         # readerOverlay: the outer field onto the target grid, underneath
-        self._outer_to_target = Interpolator(self.proj_outer, self.x_outer, self.y_outer, self.is_degree)
+        self._outer_to_target = Interpolator(self.proj_outer, self.x_outer, self.y_outer, self.outer_is_degree)
         self._outer_to_target.changeProjection(m, proj, tx, ty, tx_unit, ty_unit)
         self.target_shape = (len(np.atleast_1d(ty)) if not isinstance(ty, str) else None, len(np.atleast_1d(tx)) if not isinstance(tx, str) else None)
+        self._merge_handle()
         return self
 
     def setTargetGridFromInner(self):
@@ -125,15 +207,56 @@ class Merger:
         self.target_x, self.target_y = vx, vy
         return self.setTargetGrid(self.proj_inner, vx, vy, unit, unit)
 
-    def getDataSlice(self, inner, outer):
-        """One merged slice: `inner` [.., nyI, nxI] and `outer` [.., nyO, nxO] as float64 with NaN = undefined (getScaledDataSlice);
-        returns [.., nyT, nxT] float64"""
+    def getDataSlice(self, inner, outer, inner_bad_value=None, outer_bad_value=None, out_dtype=None, out_fill=None, stream=None):
+        """One merged slice in one call (CDMMerger::getDataSlice): `inner` [.., nyI, nxI] and `outer` [.., nyO, nxO] with the same
+        leading dimensions, of one CDM type -- numpy arrays (host buffers) or contiguous CUDA tensors (the result is a CUDA tensor;
+        enqueued on `stream`, default the current torch stream, without synchronising).  Values equal to the bad values are
+        undefined (default: NaN for floating types, defaultFillValue_ for integer ones); the result [.., nyT, nxT] is of `out_dtype`
+        (default: the inner's type) with undefined cells set to `out_fill` (default: NaN for floating types, defaultFillValue_ for
+        integer ones)."""
         if self._outer_to_target is None:
             raise FimexB200Error("must call setTargetGrid or setTargetGridFromInner before getDataSlice")
-        nan = float("nan")
-        vi, vo = np.asarray(inner, dtype=np.float64), np.asarray(outer, dtype=np.float64)
-        outer_on_inner = self._outer_to_inner.getDataSlice(vo, bad_value=nan)
-        smooth = linear_border_smoothing(vi, outer_on_inner, self.transitionWidth, self.borderWidth, self.useOuterIfInnerUndefined)
-        top = self._inner_to_target.getDataSlice(smooth, bad_value=nan)
-        base = self._outer_to_target.getDataSlice(vo, bad_value=nan)
-        return np.where(np.isnan(top), base, top)  # CDMOverlay.cc:80-85
+        mh = self._merge_handle()
+        lib = load()
+        ci = self._inner_to_target.cachedInterpolation
+        ny_t, nx_t = ci.getOutY(), ci.getOutX()
+        on_device = _is_torch(inner)
+        if on_device:
+            import torch
+            if not _is_torch(outer) or not (inner.is_cuda and outer.is_cuda) or inner.device != outer.device:
+                raise FimexB200Error("inner and outer must both be CUDA tensors on one device")
+            if inner.dtype != outer.dtype:
+                raise FimexB200Error(f"inner and outer differ in type: {inner.dtype} and {outer.dtype}")
+            if not (inner.is_contiguous() and outer.is_contiguous()):
+                raise FimexB200Error("device path needs contiguous CUDA tensors")
+            dtype = inner.dtype
+            odt = out_dtype if out_dtype is not None else dtype
+        else:
+            vi, vo = np.asarray(inner), np.asarray(outer)
+            if vi.dtype != vo.dtype:  # one CDM type for both: the common type both convert to without loss where there is one
+                common = np.result_type(vi.dtype, vo.dtype)
+                vi, vo = vi.astype(common), vo.astype(common)
+            inner, outer = np.ascontiguousarray(vi), np.ascontiguousarray(vo)
+            dtype = inner.dtype
+            odt = np.dtype(out_dtype) if out_dtype is not None else dtype
+        if inner.ndim < 2 or outer.ndim < 2 or tuple(inner.shape[-2:]) != (self.y_inner.size, self.x_inner.size) or \
+                tuple(outer.shape[-2:]) != (self.y_outer.size, self.x_outer.size):
+            raise FimexB200Error(f"inner {tuple(inner.shape)} and outer {tuple(outer.shape)} do not end in the inner "
+                                 f"({self.y_inner.size}, {self.x_inner.size}) and outer ({self.y_outer.size}, {self.x_outer.size}) grids")
+        lead = tuple(inner.shape[:-2])
+        if tuple(outer.shape[:-2]) != lead:
+            raise FimexB200Error(f"inner and outer differ in their leading dimensions: {lead} and {tuple(outer.shape[:-2])}")
+        bad_i, bad_o, fill = _fill_for(dtype, inner_bad_value), _fill_for(dtype, outer_bad_value), _fill_for(odt, out_fill)
+        in_code, out_code = int(capi.cdm_type(dtype)), int(capi.cdm_type(odt))
+        nz = int(np.prod(lead, dtype=np.int64)) if lead else 1
+        new_size = C.c_size_t()
+        if on_device:
+            out = torch.empty(lead + (ny_t, nx_t), dtype=odt, device=inner.device)
+            check(lib.fb200_merge_get_data_slice_device(mh._h, in_code, ptr(inner), inner.numel(), bad_i, ptr(outer), outer.numel(), bad_o, out_code,
+                                                        fill, ptr(out), C.byref(new_size), _stream_ptr(stream)), "CDMMerger getDataSlice")
+        else:
+            out = np.empty(lead + (ny_t, nx_t), dtype=odt)
+            check(lib.fb200_merge_get_data_slice(mh._h, in_code, ptr(inner), inner.size, bad_i, ptr(outer), outer.size, bad_o, out_code, fill,
+                                                 ptr(out), C.byref(new_size)), "CDMMerger getDataSlice")
+        assert new_size.value == nz * ny_t * nx_t
+        return out

@@ -452,6 +452,38 @@ int fb200_tinterp_get_data_slice_device(const fb200_tinterp* handle, int inType,
                                         void* d_out, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * (1i) CDMMerger: an inner (fine, small) grid merged into an outer (coarse, large) one on a target grid, with the linear border
+ *      smoothing of CDMBorderSmoothing_Linear (--merge.smoothing=LINEAR(transitionWidth,borderWidth); DESIGN.md section 2 states
+ *      the arithmetic)
+ *
+ * The handle BORROWS three interpolation handles of (1a) -- the caller keeps them alive, as with fb200_vector in
+ * fb200_interp_get_vector_slice: outerToInner reads the outer grid and writes the inner grid, innerToTarget reads the inner grid,
+ * outerToTarget reads the outer grid, and both write the same target grid.  Each may carry a reduced domain (createReducedDomain);
+ * the slabs are cropped to it inside.  All three use nearest neighbour, bilinear or bicubic, on one device.  transitionWidth >= 1
+ * (the blend divides by it), borderWidth >= 0.  create refuses anything else with MIFI_ERROR and a message.
+ *
+ * One slice: outer -> inner grid, the border blend on the inner grid, blended inner -> target, outer -> target, and the overlay
+ * (the blended inner where defined, else the outer).  inner [nz][innerY][innerX] and outer [nz][outerY][outerX] (the full grids,
+ * same nz; innerSize and outerSize in values) are both of inType; the inner value equal to badInner cast to inType and the outer
+ * value whose float equals (float)badOuter (mifi_bad2nanf, as the gathers of (1c)) are undefined; NaN never matches.  out
+ * [nz][outY][outX] of outType, undefined -> outFill, rounded and cast as in (1c); *newSize receives its number of values.  No
+ * scale or offset is applied.  The host form uploads inner and outer once and downloads out once, pipelined over level chunks;
+ * _device takes device pointers and enqueues everything on cuda_stream without synchronising.  The device chain keeps at most
+ * 256 MB of float intermediates (or one level, where one level needs more).  The handle is immutable and every call re-entrant.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct fb200_merge fb200_merge; /* opaque */
+
+int fb200_merge_create(const fb200_interp* outerToInner, const fb200_interp* innerToTarget, const fb200_interp* outerToTarget, size_t innerX,
+                       size_t innerY, size_t outerX, size_t outerY, int transitionWidth, int borderWidth, int useOuterIfInnerUndefined,
+                       fb200_merge** handle);
+void fb200_merge_destroy(fb200_merge* handle);
+int fb200_merge_get_data_slice(const fb200_merge* handle, int inType, const void* inner, size_t innerSize, double badInner, const void* outer,
+                               size_t outerSize, double badOuter, int outType, double outFill, void* out, size_t* newSize);
+int fb200_merge_get_data_slice_device(const fb200_merge* handle, int inType, const void* d_inner, size_t innerSize, double badInner,
+                                      const void* d_outer, size_t outerSize, double badOuter, int outType, double outFill, void* d_out,
+                                      size_t* newSize, void* cuda_stream);
+
+/* ------------------------------------------------------------------------------------------------
  * (2) the reference's C symbols for this path -- include/fimex/interpolation.h (line of each prototype given)
  * ---------------------------------------------------------------------------------------------- */
 int mifi_string_to_interpolation_method(const char* stringMethod); /* :44 */
