@@ -194,7 +194,10 @@ int parse_proj(const char* definition, ProjDef* P, char* err, int errlen)
         return fail(err, errlen, -5, "unknown projection id '" + name + "' (supported: latlong, ob_tran, stere, lcc)");
 
     if (!kv.flag("no_defs")) { // proj_def.dat defaults
-        kv.add("ellps", "WGS84");
+        // pj_init does not default the ellipsoid when the string gives a datum or any earth figure: a
+        // default +rf would otherwise win over a user's +b, and +datum=NAD83 would lose its GRS80
+        if (!kv.has("datum") && !kv.has("ellps") && !kv.has("a") && !kv.has("b") && !kv.has("rf") && !kv.has("f"))
+            kv.add("ellps", "WGS84");
         if (P->kind == PK_LCC) {
             kv.add("lat_1", "33");
             kv.add("lat_2", "45");

@@ -26,9 +26,11 @@
  *     config 2;
  *   - the reference's own tests at the PROJ boundary (test/testInterpolation.cc:265-278, 280-393, 396-512, 515-654;
  *     test/testInterpolator.cc:398-472), re-run in tests/test_oracle_golden.py and tests/test_gpu_parity.py.
- *   What remains UNPINNED: datum shifts (+towgs84 with non-zero parameters, +nadgrids) and the last-ulp behaviour of libproj
- *   itself (libm differences) -- no configuration of BASELINE.json or of the reference's tests uses a datum shift
- *   (SURVEY.md 8c').
+ *   - 3- and 7-parameter datum shifts (+towgs84, +datum=WGS84|NAD83) against an independent geocentric reference
+ *     (tests/datum_reference.py: geodetic -> ECEF, position-vector Helmert, PROJ 4's R^T inverse, Heikkinen's closed form
+ *     polished by Newton in long double), <= 1e-11 degree of arc on random CRS pairs of all four families, plus the parser's
+ *     +ellps / +datum / +towgs84 precedence and the early exits (tests/test_datum_reference_host.py).
+ *   What remains UNPINNED: grid shifts (+nadgrids, refused) and the last-ulp behaviour of libproj itself (libm differences).
  *
  * Supported grammar (SURVEY.md 8a row P): +proj=latlong|longlat|latlon|lonlat, ob_tran (+o_proj one of
  * the four lat/long names, +o_lat_p, +o_lon_p), stere (+lat_0 +lon_0 +lat_ts | +k|+k_0), lcc (+lat_1
@@ -601,7 +603,10 @@ projPJ pj_init_plus(const char* definition)
     }
     /* defaults of proj_def.dat, appended at the end unless +no_defs (pj_init.c get_defaults) */
     if (!pl_bool(&pl, "no_defs")) {
-        pl_append(&pl, "ellps", "WGS84");
+        /* get_opt: "don't default ellipse if datum, ellps or any earth model information is set" */
+        if (!pl_has(&pl, "datum") && !pl_has(&pl, "ellps") && !pl_has(&pl, "a") && !pl_has(&pl, "b") && !pl_has(&pl, "rf") &&
+            !pl_has(&pl, "f"))
+            pl_append(&pl, "ellps", "WGS84");
         if (P->kind == KIND_LCC) {
             pl_append(&pl, "lat_1", "33");
             pl_append(&pl, "lat_2", "45");
